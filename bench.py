@@ -2,6 +2,7 @@
 """bench.py — uint16 voxel GB/s of the sqeazy volume pipeline (encode + decode) on B200.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload cfg2|cfg1|cfg3|cfg4|cfg5] [--no-per-config]
+                    [--dump-outputs DIR]
 
 A *step* = one encode + one decode of one volume through the pipeline (cfg4: one decode of a batch of reference blobs).
   value    raw volume bytes / (t_encode + t_decode), inputs resident in HBM (sqyx_* device API), summed over ranks
@@ -17,6 +18,10 @@ A *step* = one encode + one decode of one volume through the pipeline (cfg4: one
 N > 1 (torchrun): every rank encodes/decodes its own stack (stacks partitioned over GPUs; weak scaling; no data-path
 collective — cfg3's quantiser adds the NCCL histogram all-reduce); time = max over ranks.
 `--impl reference` times the reference's CPU implementation (rank 0 only) on bounded slabs of the same workload.
+`--dump-outputs DIR` writes what rank 0's timed steps returned in the last step (blobs and decoded stacks of the main
+workload) to DIR as .npy files; inputs are seeded, so two builds of the library can be compared output for output. cfg4
+times two framings one after the other and dumps the decoded stacks of the last (block-linked) one; without oracle/_ref
+it has no reference-made blobs, is skipped and writes nothing (said on stderr).
 """
 from __future__ import annotations
 
@@ -25,7 +30,9 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
+import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
@@ -41,6 +48,30 @@ WORKLOADS = {
 CFG4_PER_GPU = 8       # BASELINE cfg4: 64 blobs over 8 GPUs
 CFG5_PER_GPU = 32      # BASELINE cfg5: 1000 stacks, stack v -> GPU v mod G; a bounded sample per GPU
 METRIC = "uint16 voxel GB/s encode+decode"
+DUMP_SAMPLES = 1 << 23   # float32 values over all arrays of one --dump-outputs (32 MiB)
+DUMP_CHUNK = 1 << 22     # elements per chunk sum
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each tensor of `arrays` (name -> tensor of uint8 or 16-bit voxels) as DIR/<name>.npy: its elements
+    read as unsigned integers in float32 (exact), all of them or, when the array exceeds its share of DUMP_SAMPLES, a
+    sorted sample at positions drawn from a generator seeded by the name. DIR/<name>_chunk_sums.npy (float64, exact)
+    holds the sums over consecutive DUMP_CHUNK elements, so that every element counts in the comparison."""
+    import numpy as np
+    import torch
+
+    os.makedirs(dirname, exist_ok=True)
+    per_array = DUMP_SAMPLES // len(arrays)
+    for name, t in arrays.items():
+        flat = t.reshape(-1)
+        n = flat.numel()
+        mask = (1 << (8 * flat.element_size())) - 1
+        sums = [int((flat[s:s + DUMP_CHUNK].to(torch.int64) & mask).sum().item()) for s in range(0, n, DUMP_CHUNK)]
+        np.save(os.path.join(dirname, name + "_chunk_sums.npy"), np.array(sums, dtype=np.float64))
+        if n > per_array:
+            idx = np.sort(np.random.default_rng(zlib.crc32(name.encode())).integers(0, n, size=per_array))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        np.save(os.path.join(dirname, name + ".npy"), ((flat.to(torch.int64) & mask).cpu().numpy()).astype(np.float32))
 
 
 def measured_peak_hbm():
@@ -58,7 +89,7 @@ class ClockSampler:
     def __init__(self, gpu_index):
         self.proc = None
         self.gpu_index = gpu_index
-        self.path = f"/tmp/sqy_clocks_{os.getpid()}.csv"
+        self.path = os.path.join(tempfile.gettempdir(), f"sqy_clocks_{os.getpid()}.csv")
 
     def start(self):
         try:
@@ -262,7 +293,7 @@ def copy_ceiling(ctx, h_in, h_out, d_buf, reps=2):
             "what": "raw stack H2D then D2H by cudaMemcpyAsync from the same pinned buffers, all ranks at once"}
 
 
-def run_pipeline_workload(ctx, wname, steps, warmup, want_e2e=True, detail=True, sampler_cls=None):
+def run_pipeline_workload(ctx, wname, steps, warmup, want_e2e=True, detail=True, sampler_cls=None, dump_dir=None):
     """cfg1 / cfg2 / cfg3: one stack per rank through the whole pipeline, device-resident and through the host API"""
     import numpy as np
 
@@ -318,6 +349,8 @@ def run_pipeline_workload(ctx, wname, steps, warmup, want_e2e=True, detail=True,
     clocks = sampler.stop() if sampler else None
     launches = sq.kernel_launches() - launches0
     stats = sq.last_lz4_stats()
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(dump_dir, {"blob": blob, "decoded": out})
     t_enc_ms = ctx.max_over_ranks(t_enc_ms)
     t_dec_ms = ctx.max_over_ranks(t_dec_ms)
     total_s = (t_enc_ms + t_dec_ms) / 1e3
@@ -431,7 +464,7 @@ def run_pipeline_workload(ctx, wname, steps, warmup, want_e2e=True, detail=True,
     return res
 
 
-def run_cfg5(ctx, steps, warmup):
+def run_cfg5(ctx, steps, warmup, dump_dir=None):
     """time-lapse: stack v -> rank v mod G; the stacks of a rank as one batch (sqyx_*_batch_device_UI16)"""
     torch, sq = ctx.torch, ctx.sq
     from sqeazy_b200.synth import torch_volume
@@ -465,6 +498,8 @@ def run_cfg5(ctx, steps, warmup):
         td += ev[1].elapsed_time(ev[2])
     ctx.barrier()
     launches = sq.kernel_launches() - launches0
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(dump_dir, {**{f"blob_{i}": b for i, b in enumerate(blobs)}, **{f"decoded_{i}": o for i, o in enumerate(outs)}})
     te, td = ctx.max_over_ranks(te), ctx.max_over_ranks(td)
     tot = ctx.world * n * raw * steps
     res = {"workload": "cfg5", "pipeline": pipeline, "shape_zyx": list(shape), "stacks_per_gpu": n,
@@ -477,7 +512,7 @@ def run_cfg5(ctx, steps, warmup):
     return res
 
 
-def run_cfg4(ctx, steps, warmup):
+def run_cfg4(ctx, steps, warmup, dump_dir=None):
     """decode-only of REFERENCE-made bitswap1->lz4 blobs: CFG4_PER_GPU stacks per GPU (64 over 8 GPUs), both framings the
     reference produces — one frame per 256 KiB chunk (its multi-threaded mode) and one block-linked frame (its one-thread
     mode, the sqy CLI default). The blobs are made by oracle/_ref (the reference's own stage code + liblz4) before the
@@ -490,6 +525,8 @@ def run_cfg4(ctx, steps, warmup):
 
     ref = orc.ref()
     if not ref.available:
+        if dump_dir:
+            print("bench.py: cfg4 skipped without oracle/_ref: nothing dumped to " + dump_dir, file=sys.stderr)
         return {"workload": "cfg4", "skipped": "oracle/_ref (the compiled reference) is not present: no reference-made blobs"}
     shape, pipeline, preset, _ = WORKLOADS["cfg4"]
     name = "bitswap1(num_bits_per_plane=1)->lz4(accel=1,blocksize_kb=256,framestep_kb=256,n_chunks_of_input=0)"
@@ -538,6 +575,8 @@ def run_cfg4(ctx, steps, warmup):
         res[framing] = {"decode_gbs": ctx.world * B * raw * steps / (ms / 1e3) / 1e9, "ms_per_batch": ms / steps,
                         "blob_ratio": raw / int(blobs[0].numel()), "bit_exact": ok}
         del blobs, batch
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(dump_dir, {f"decoded_{i}": o for i, o in enumerate(outs)})
     res["value"] = res["frame_per_chunk"]["decode_gbs"]
     res["gpu_launches"] = int(total_launches)
     del vols, planes, outs
@@ -646,7 +685,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-per-config", action="store_true", help="only the main workload (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the main workload's outputs of the last timed step to DIR/<name>.npy (cfg4: of its last framing, "
+                         "and nothing when it is skipped; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
 
     shape, pipeline, preset, chain_id = WORKLOADS[args.workload]
     if args.preset:
@@ -695,11 +741,12 @@ def main():
 
     t_start = time.perf_counter()
     if args.workload in ("cfg1", "cfg2", "cfg3"):
-        main_res = run_pipeline_workload(ctx, args.workload, args.steps, warmup, want_e2e=not args.no_e2e, detail=True, sampler_cls=ClockSampler)
+        main_res = run_pipeline_workload(ctx, args.workload, args.steps, warmup, want_e2e=not args.no_e2e, detail=True, sampler_cls=ClockSampler,
+                                         dump_dir=args.dump_outputs)
     elif args.workload == "cfg4":
-        main_res = run_cfg4(ctx, args.steps, warmup)
+        main_res = run_cfg4(ctx, args.steps, warmup, dump_dir=args.dump_outputs)
     else:
-        main_res = run_cfg5(ctx, args.steps, warmup)
+        main_res = run_cfg5(ctx, args.steps, warmup, dump_dir=args.dump_outputs)
 
     # ---- the other BASELINE configurations, a few steps each ----
     per_config = None

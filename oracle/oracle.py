@@ -364,8 +364,215 @@ class Ref:
         return rc, out, secs.value
 
 
+class _LZ4FFrameInfo(ctypes.Structure):
+    _fields_ = [("blockSizeID", c_int), ("blockMode", c_int), ("contentChecksumFlag", c_int), ("frameType", c_int),
+                ("contentSize", ctypes.c_ulonglong), ("dictID", ctypes.c_uint), ("blockChecksumFlag", c_int)]
+
+
+class _LZ4FPreferences(ctypes.Structure):
+    _fields_ = [("frameInfo", _LZ4FFrameInfo), ("compressionLevel", c_int), ("autoFlush", ctypes.c_uint),
+                ("favorDecSpeed", ctypes.c_uint), ("reserved", ctypes.c_uint * 3)]
+
+
+class Standin:
+    """Stand-in for `Ref` where oracle/_ref cannot be built (the reference's sources are not in the repository), reached
+    through the `ref_or_standin` test fixture only. It is NOT the reference's code:
+      * LZ4 encode: the reference's lz4_scheme encode (SURVEY.md A.5) restated over liblz4, the library the reference
+        calls; byte-identical to the reference-made payloads of tests/golden (tests/test_oracle.py);
+      * LZ4 decode: the reference's decode loop (lz4.hpp:257-339) restated over liblz4's LZ4F_decompress; rc 0 only when
+        exactly the expected bytes come out;
+      * filters, diff, quantiser: the C port (oracle/sqy_oracle.c), pinned to the reference by the golden vectors;
+      * L2 size (rmestbkrd): the kernel's sysfs record of the host, independent of the library under test.
+    `available` is False without liblz4. Tests that pin the C port itself need the reference (`live_ref`)."""
+
+    LZ4_LIB = "liblz4.so.1"
+
+    def __init__(self):
+        self.port = port()
+        try:
+            self.lz4 = ctypes.CDLL(self.LZ4_LIB)
+            self.available = True
+        except OSError:
+            self.lz4, self.available = None, False
+            return
+        L = self.lz4
+        L.LZ4F_isError.argtypes = [ctypes.c_size_t]
+        for f in ("LZ4F_compressBound", "LZ4F_compressBegin", "LZ4F_compressUpdate", "LZ4F_compressEnd"):
+            getattr(L, f).restype = ctypes.c_size_t
+        L.LZ4F_compressBound.argtypes = [ctypes.c_size_t, c_void_p]
+        L.LZ4F_createCompressionContext.argtypes = [POINTER(c_void_p), ctypes.c_uint]
+        L.LZ4F_freeCompressionContext.argtypes = [c_void_p]
+        L.LZ4F_compressBegin.argtypes = [c_void_p, c_void_p, ctypes.c_size_t, c_void_p]
+        L.LZ4F_compressUpdate.argtypes = [c_void_p, c_void_p, ctypes.c_size_t, c_void_p, ctypes.c_size_t, c_void_p]
+        L.LZ4F_compressEnd.argtypes = [c_void_p, c_void_p, ctypes.c_size_t, c_void_p]
+        L.LZ4F_decompress.restype = ctypes.c_size_t
+        L.LZ4F_decompress.argtypes = [c_void_p, c_void_p, POINTER(ctypes.c_size_t), c_void_p, POINTER(ctypes.c_size_t), c_void_p]
+        L.LZ4F_createDecompressionContext.argtypes = [POINTER(c_void_p), ctypes.c_uint]
+        L.LZ4F_freeDecompressionContext.argtypes = [c_void_p]
+
+    # ---- lz4_scheme (encoders/lz4.hpp:58-274, lz4_utils.hpp:99-173 as summarised in SURVEY.md A.5) ----
+    def _lz4_args(self, config: bytes):
+        args = {"accel": 1, "blocksize_kb": 256, "framestep_kb": 256, "n_chunks_of_input": 0}
+        for k, v in minors(config.decode()).items():
+            if k in args:
+                args[k] = int(v)
+        bs = self.port.closest_blocksize_kb(args["blocksize_kb"])
+        fs = bs if args["framestep_kb"] < bs else bs * max(1, round(args["framestep_kb"] / bs))
+        if args["n_chunks_of_input"]:
+            fs = 0
+        return args["accel"], bs, fs, args["n_chunks_of_input"]
+
+    def _prefs(self, accel, bs_kb):
+        p = _LZ4FPreferences()
+        p.frameInfo.blockSizeID = {64: 4, 256: 5, 1024: 6, 4096: 7}[bs_kb]   # linked blocks, no checksums, no content size
+        p.compressionLevel = accel
+        return p
+
+    def _encode_serial(self, raw: np.ndarray, chunk: int, prefs) -> bytes:
+        """one frame: compressBegin, one compressUpdate per chunk, compressEnd"""
+        L = self.lz4
+        cap = L.LZ4F_compressBound(chunk, ctypes.byref(prefs)) + 64
+        buf = np.zeros(max(cap, 64), dtype=np.uint8)
+        ctx = c_void_p()
+        assert not L.LZ4F_isError(L.LZ4F_createCompressionContext(ctypes.byref(ctx), 100))
+        parts = []
+        try:
+            def put(n):
+                assert not L.LZ4F_isError(n), "liblz4 frame compression failed"
+                parts.append(buf[:n].tobytes())
+            put(L.LZ4F_compressBegin(ctx, _p(buf), buf.size, ctypes.byref(prefs)))
+            for s in range(0, raw.size, chunk):
+                piece = np.ascontiguousarray(raw[s:s + chunk])
+                put(L.LZ4F_compressUpdate(ctx, _p(buf), buf.size, _p(piece), piece.size, None))
+            put(L.LZ4F_compressEnd(ctx, _p(buf), buf.size, None))
+        finally:
+            L.LZ4F_freeCompressionContext(ctx)
+        return b"".join(parts)
+
+    def lz4_config(self, config=b"") -> str:
+        accel, bs, fs, n = self._lz4_args(config)
+        return f"accel={accel},blocksize_kb={bs},framestep_kb={fs},n_chunks_of_input={n}"
+
+    def lz4_encode(self, a, nthreads=1, config=b""):
+        """payload exactly as lz4_scheme<T>::encode writes it: one frame (nthreads = 1 or one chunk), else a frame per chunk"""
+        raw = np.ascontiguousarray(a).view(np.uint8).ravel()
+        accel, bs, fs, n = self._lz4_args(config)
+        chunk = min(raw.size // n if n else fs << 10, raw.size) or raw.size or 1
+        prefs = self._prefs(accel, bs)
+        if nthreads <= 1 or raw.size <= chunk:
+            out = self._encode_serial(raw, chunk, prefs)
+        else:
+            out = b"".join(self._encode_serial(raw[s:s + chunk], chunk, prefs) for s in range(0, raw.size, chunk))
+        return np.frombuffer(out, dtype=np.uint8).copy()
+
+    def _lz4_decode(self, payload, nbytes):
+        """frames one after the other (skippable ones skipped by liblz4) until the input is used up"""
+        L = self.lz4
+        src = np.ascontiguousarray(payload, dtype=np.uint8)
+        out = np.zeros(nbytes, dtype=np.uint8)
+        ctx = c_void_p()
+        assert not L.LZ4F_isError(L.LZ4F_createDecompressionContext(ctypes.byref(ctx), 100))
+        pos = got = hint = 0
+        try:
+            while pos < src.size:
+                dst_n, src_n = ctypes.c_size_t(nbytes - got), ctypes.c_size_t(src.size - pos)
+                hint = L.LZ4F_decompress(ctx, c_void_p(out.ctypes.data + got), ctypes.byref(dst_n),
+                                         c_void_p(src.ctypes.data + pos), ctypes.byref(src_n), None)
+                if L.LZ4F_isError(hint) or (src_n.value == 0 and dst_n.value == 0):
+                    return 1, out
+                pos += src_n.value
+                got += dst_n.value
+        finally:
+            L.LZ4F_freeDecompressionContext(ctx)
+        return (0 if hint == 0 and got == nbytes else 1), out
+
+    def lz4_decode_u16(self, payload, n_voxels):
+        rc, out = self._lz4_decode(payload, 2 * n_voxels)
+        return rc, out.view(np.uint16)
+
+    def lz4_decode_bytes(self, payload, nbytes):
+        return self._lz4_decode(payload, nbytes)
+
+    # ---- filters and quantiser: the C port ----
+    def l2_cache_bytes(self) -> int:
+        base = "/sys/devices/system/cpu/cpu0/cache"
+        for idx in sorted(os.listdir(base)):
+            with open(os.path.join(base, idx, "level")) as f:
+                if f.read().strip() != "2":
+                    continue
+            with open(os.path.join(base, idx, "size")) as f:
+                size = f.read().strip()
+            return int(size[:-1]) << {"K": 10, "M": 20}[size[-1]] if size[-1] in "KM" else int(size)
+        raise RuntimeError("no L2 cache record under " + base)
+
+    def bitswap_encode(self, w, a, nthreads=1, scalar=False):
+        return self.port.bitswap_encode(w, a)
+
+    def bitswap_decode(self, w, a):
+        return self.port.bitswap_decode(w, a)
+
+    def bitswap8_encode(self, w, a):
+        return self.port.bitswap8_encode(w, a)
+
+    def bitswap8_decode(self, w, a):
+        return self.port.bitswap8_decode(w, a)
+
+    def remove_background(self, a, threshold, nthreads=1):
+        return self.port.remove_background(a, threshold)
+
+    def remove_background8(self, a, threshold):
+        return self.port.remove_background8(a, threshold)
+
+    def rmestbkrd(self, vol, nthreads=1):
+        return self.port.rmestbkrd(vol, self.l2_cache_bytes())[0]
+
+    def diff(self, vol, decode=False, nthreads=1):
+        return self.port.diff(vol, decode=decode)
+
+    def quantiser_setup(self, a):
+        hist = self.port.histogram(np.ascontiguousarray(a, dtype=np.uint16))
+        enc, dec = self.port.quantiser_luts(hist)
+        return hist, enc, dec
+
+    def quantiser_encode(self, a):
+        _, enc, dec = self.quantiser_setup(a)
+        return self.port.lut_apply(a, enc), dec
+
+    def quantiser_lut_string(self, dec) -> str:
+        return lut_to_verbatim(dec)
+
+    # ---- stage chains of oracle/ref_harness.cpp ----
+    def pipeline_encode_stages(self, pipeline_id, vol, nthreads, w=1, threshold=0):
+        import time
+
+        vol = np.ascontiguousarray(vol, dtype=np.uint16)
+        t0 = time.perf_counter()
+        if pipeline_id == 0:
+            data = self.port.bitswap_encode(1, vol)
+        elif pipeline_id == 1:
+            data = self.port.bitswap_encode(1, self.rmestbkrd(vol))
+        elif pipeline_id == 2:
+            data = self.quantiser_encode(vol)[0]
+        elif pipeline_id == 3:
+            data = self.port.bitswap_encode(w, self.port.remove_background(vol, threshold))
+        else:
+            data = vol
+        payload = self.lz4_encode(data, nthreads=nthreads)
+        return payload, time.perf_counter() - t0
+
+    def pipeline_decode_stages(self, w, payload, n_voxels):
+        import time
+
+        t0 = time.perf_counter()
+        rc, out = self.lz4_decode_u16(payload, n_voxels)
+        if rc == 0 and w:
+            out = self.port.bitswap_decode(w, out)
+        return rc, out, time.perf_counter() - t0
+
+
 _port = None
 _ref = None
+_standin = None
 
 
 def port() -> Port:
@@ -380,6 +587,13 @@ def ref() -> Ref:
     if _ref is None:
         _ref = Ref()
     return _ref
+
+
+def standin() -> Standin:
+    global _standin
+    if _standin is None:
+        _standin = Standin()
+    return _standin
 
 
 # ------------------------------------------------------------------------------------------------

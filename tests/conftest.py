@@ -34,12 +34,37 @@ def port():
 
 @pytest.fixture(scope="session")
 def ref():
+    """the reference's own stage code, oracle/_ref: built only from the reference's sources, which are not part of this
+    repository; the tests that pin the oracle port itself need it and skip without it"""
     from oracle import oracle
 
     r = oracle.ref()
     if not r.available:
-        pytest.skip("oracle/_ref (compiled reference stages) not built")
+        pytest.skip("oracle/_ref (the reference's compiled stage code, built from sources outside this repository) not built")
     return r
+
+
+@pytest.fixture(scope="session")
+def ref_or_standin():
+    """oracle/_ref where it is built, else oracle.Standin (liblz4 for LZ4, the golden-pinned C port for the filters);
+    which of the two a run used is printed in the report header"""
+    from oracle import oracle
+
+    r = oracle.ref()
+    if r.available:
+        return r
+    s = oracle.standin()
+    if not s.available:
+        pytest.skip("neither oracle/_ref nor liblz4 for oracle.Standin")
+    return s
+
+
+def pytest_report_header(config):
+    from oracle import oracle
+
+    if os.path.exists(oracle._REF_SO):
+        return "reference comparisons: oracle/_ref (the reference's own code)"
+    return "reference comparisons: oracle.Standin (oracle/_ref not built; tests that need the reference itself skip)"
 
 
 @pytest.fixture(scope="session")

@@ -102,7 +102,7 @@ def test_refused_shapes(port, sim, shape):
 
 
 @pytest.mark.parametrize("shape", REFUSED_U8)
-def test_refused_uint8_extents(port, ref, sim, shape):
+def test_refused_uint8_extents(port, sim, shape):
     """uint8 stacks: naive_sum keeps z, y, x in int8 (diff_scheme_utils.hpp:81-89); from 129 on the reference reads from
     wrapped coordinates - what it returns there no longer follows its own rule on the shapes where it does not crash"""
     z, y, x = shape

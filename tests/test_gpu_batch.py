@@ -49,7 +49,7 @@ def test_decode_batch_of_mixed_pipelines(sq, cuda):
         assert np.array_equal(host16(o), w)
 
 
-def test_decode_batch_of_reference_blobs(sq, cuda, ref):
+def test_decode_batch_of_reference_blobs(sq, cuda, ref_or_standin):
     """cfg4 in small: blobs made by the reference's own stage chain, both framings (block-linked frame = sqy CLI default,
     one frame per chunk = the multi-threaded mode), decoded as one batch, bit-exact"""
     name = "bitswap1(num_bits_per_plane=1)->lz4(accel=1,blocksize_kb=256,framestep_kb=256,n_chunks_of_input=0)"
@@ -57,7 +57,7 @@ def test_decode_batch_of_reference_blobs(sq, cuda, ref):
     vols, blobs = [], []
     for i in range(10):
         vol = numpy_volume(shape, "scmos", index=40 + i)
-        payload, _ = ref.pipeline_encode_stages(0, vol, 1 if i % 2 else 8)
+        payload, _ = ref_or_standin.pipeline_encode_stages(0, vol, 1 if i % 2 else 8)
         h = orc.pack_header(vol.shape, name, payload.size, version="0.5.2", headref="4c45a9b")
         vols.append(vol)
         blobs.append(cuda.from_numpy(np.concatenate([np.frombuffer(h.encode(), dtype=np.uint8), payload])).cuda())
@@ -67,7 +67,7 @@ def test_decode_batch_of_reference_blobs(sq, cuda, ref):
         assert np.array_equal(host16(o), v)
 
 
-def test_decode_batch_of_linked_blobs_on_the_deferred_route(sq, cuda, ref):
+def test_decode_batch_of_linked_blobs_on_the_deferred_route(sq, cuda, ref_or_standin):
     """stacks of 12 linked 256 KiB blocks each: every lane of the batch runs the deferred-reference decoder (pass 1 and the
     chain walk side by side on two streams of its own) at the same time as the others"""
     name = "bitswap1(num_bits_per_plane=1)->lz4(accel=1,blocksize_kb=256,framestep_kb=256,n_chunks_of_input=0)"
@@ -75,7 +75,7 @@ def test_decode_batch_of_linked_blobs_on_the_deferred_route(sq, cuda, ref):
     vols, blobs = [], []
     for i in range(9):
         vol = numpy_volume(shape, "scmos" if i % 2 else "ref", index=70 + i)
-        payload, _ = ref.pipeline_encode_stages(0, vol, 1)
+        payload, _ = ref_or_standin.pipeline_encode_stages(0, vol, 1)
         h = orc.pack_header(vol.shape, name, payload.size, version="0.5.2", headref="4c45a9b")
         vols.append(vol)
         blobs.append(cuda.from_numpy(np.concatenate([np.frombuffer(h.encode(), dtype=np.uint8), payload])).cuda())

@@ -88,7 +88,7 @@ def test_diff_refused_shapes(sq, cuda, shape):
                                       "remove_background(threshold=105)->diff3x3x1->lz4", "diff3x3x1->pass_through->lz4",
                                       "bitswap1->diff3x3x1->lz4"])
 @pytest.mark.parametrize("shape", [(16, 128, 256), (5, 33, 77), (40, 24, 32)])
-def test_diff_pipelines(sq, cuda, port, ref, pipeline, shape):
+def test_diff_pipelines(sq, cuda, port, ref_or_standin, pipeline, shape):
     vol = numpy_volume(shape, "scmos", index=11)
     blob = sq.encode(pipeline, vol)
     assert blob.size <= sq.max_compressed_length(pipeline, vol.nbytes)
@@ -104,21 +104,21 @@ def test_diff_pipelines(sq, cuda, port, ref, pipeline, shape):
     # a reader built on the reference: LZ4 frames (liblz4 through the reference's decode loop), then the head filters backwards
     payload = blob[hdr["size"]:]
     if pipeline.endswith("lz4"):
-        rc, payload = ref.lz4_decode_bytes(payload, vol.nbytes)
+        rc, payload = ref_or_standin.lz4_decode_bytes(payload, vol.nbytes)
         assert rc == 0
     stage_out = np.frombuffer(payload.tobytes(), dtype=np.uint16)
     if pipeline.startswith("bitswap1->diff"):
-        assert np.array_equal(stage_out.reshape(shape), ref.diff(port.bitswap_encode(1, want).reshape(shape)))
-        stage_out = port.bitswap_decode(1, ref.diff(stage_out.reshape(shape), decode=True))
+        assert np.array_equal(stage_out.reshape(shape), ref_or_standin.diff(port.bitswap_encode(1, want).reshape(shape)))
+        stage_out = port.bitswap_decode(1, ref_or_standin.diff(stage_out.reshape(shape), decode=True))
     else:
         if "bitswap1" in pipeline:
             stage_out = port.bitswap_decode(1, stage_out)
-        assert np.array_equal(stage_out.reshape(shape), ref.diff(want))
-        stage_out = ref.diff(stage_out.reshape(shape), decode=True)
+        assert np.array_equal(stage_out.reshape(shape), ref_or_standin.diff(want))
+        stage_out = ref_or_standin.diff(stage_out.reshape(shape), decode=True)
     assert np.array_equal(stage_out.reshape(shape), want)
 
 
-def test_diff_uint8_pipelines(sq, cuda, port, ref):
+def test_diff_uint8_pipelines(sq, cuda, port, ref_or_standin):
     rng = np.random.default_rng(8)
     vol = np.clip(np.rint(20 + 2 * rng.standard_normal((9, 120, 128))), 0, 255).astype(np.uint8)
     with pytest.raises(sq.SqeazyError):                      # 130 rows: beyond the reference's int8 coordinates
@@ -128,7 +128,7 @@ def test_diff_uint8_pipelines(sq, cuda, port, ref):
         assert np.array_equal(sq.decode_u8(blob).reshape(vol.shape), vol)
         if pipeline == "diff3x3x1":
             hdr = orc.unpack_header(blob.tobytes())
-            assert np.array_equal(np.frombuffer(blob[hdr["size"]:].tobytes(), dtype=np.uint8).reshape(vol.shape), ref.diff(vol))
+            assert np.array_equal(np.frombuffer(blob[hdr["size"]:].tobytes(), dtype=np.uint8).reshape(vol.shape), ref_or_standin.diff(vol))
 
 
 def test_diff_device_pipeline_and_ratio(sq, cuda):

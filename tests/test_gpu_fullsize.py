@@ -197,7 +197,7 @@ def test_lossless_pipeline_on_eight_gib(sq, cuda, roomy):
     del blob, out, vol
 
 
-def test_cfg2_slab_ratio_against_the_reference_on_the_same_voxels(sq, cuda, ref):
+def test_cfg2_slab_ratio_against_the_reference_on_the_same_voxels(sq, cuda, ref_or_standin):
     """DESIGN.md 5: on background-removed, very compressible stacks the blob may be at most 10 % larger than the reference's
     (ratio >= 0.90 x): 16 KiB independent blocks against liblz4's 64 KiB window inside 256 KiB blocks. Same 2^26 voxels through
     both encoders (the reference's own stage chain, dynamic_pipeline.hpp:560-690 re-driven by oracle/ref_harness.cpp), and the
@@ -205,13 +205,13 @@ def test_cfg2_slab_ratio_against_the_reference_on_the_same_voxels(sq, cuda, ref)
     from sqeazy_b200.synth import numpy_volume
 
     vol = numpy_volume((16, 2048, 2048), "scmos", index=0)
-    theirs, _ = ref.pipeline_encode_stages(1, vol, 8)
+    theirs, _ = ref_or_standin.pipeline_encode_stages(1, vol, 8)
     blob = sq.encode("rmestbkrd->bitswap1->lz4", vol)
     hs = sq.header_size(blob)
     ours = blob.size - hs
     assert ours <= theirs.size / 0.90, (ours, theirs.size, vol.nbytes / ours, vol.nbytes / theirs.size)
-    rc, back_theirs, _ = ref.pipeline_decode_stages(1, theirs, vol.size)
-    rc2, back_ours, _ = ref.pipeline_decode_stages(1, blob[hs:], vol.size)
+    rc, back_theirs, _ = ref_or_standin.pipeline_decode_stages(1, theirs, vol.size)
+    rc2, back_ours, _ = ref_or_standin.pipeline_decode_stages(1, blob[hs:], vol.size)
     assert rc == 0 and rc2 == 0
     assert np.array_equal(back_ours, back_theirs)
     assert np.array_equal(sq.decode(blob).reshape(-1), back_theirs.reshape(-1))

@@ -33,12 +33,12 @@ def test_foreign_frames_with_any_offset(sq, cuda, port, period):
     assert np.array_equal(out.cpu().numpy(), a)
 
 
-def test_reference_frames(sq, cuda, ref):
+def test_reference_frames(sq, cuda, ref_or_standin):
     """liblz4 frames made by the reference's lz4_scheme: serial (linked: always the warp decoder), parallel, 64 KiB blocks"""
     vol = numpy_volume((10, 256, 512), "ref", index=9)
-    planes = ref.bitswap_encode(1, vol)
+    planes = ref_or_standin.bitswap_encode(1, vol)
     for nthreads, config in ((1, b""), (8, b""), (3, b"n_chunks_of_input=7"), (4, b"blocksize_kb=64,framestep_kb=64")):
-        payload = ref.lz4_encode(planes, nthreads=nthreads, config=config)
+        payload = ref_or_standin.lz4_encode(planes, nthreads=nthreads, config=config)
         out = cuda.zeros(planes.size, dtype=cuda.int16, device="cuda")
         assert sq.lz4_decode_device(dev(cuda, payload), out) == planes.nbytes, (nthreads, config)
         assert np.array_equal(host16(out), planes), (nthreads, config)
@@ -124,14 +124,14 @@ def _mixed_content(rng, n):
 
 
 @pytest.mark.parametrize("seed", range(10))
-def test_random_mixed_streams_from_liblz4_and_own_encoder(sq, cuda, ref, seed):
+def test_random_mixed_streams_from_liblz4_and_own_encoder(sq, cuda, ref_or_standin, seed):
     """the batch walk, the single-sequence path, near / far / overlapping copies and the length chains
     on streams with every kind of sequence: liblz4 frames (64 KiB and 256 KiB blocks, linked and independent) and our own"""
     rng = np.random.default_rng(1000 + seed)
     a = _mixed_content(rng, int(rng.integers(200_000, 900_000)))
     configs = ((1, b""), (4, b""), (2, b"blocksize_kb=64,framestep_kb=64"), (3, b"n_chunks_of_input=3"))
     nthreads, config = configs[seed % len(configs)]
-    for payload in (ref.lz4_encode(a, nthreads=nthreads, config=config), sq.lz4_encode_device(dev(cuda, a)).cpu().numpy()):
+    for payload in (ref_or_standin.lz4_encode(a, nthreads=nthreads, config=config), sq.lz4_encode_device(dev(cuda, a)).cpu().numpy()):
         out = cuda.full((a.size + 32,), 0x42, dtype=cuda.uint8, device="cuda")
         assert sq.lz4_decode_device(dev(cuda, payload), out[: a.size]) == a.size
         h = out.cpu().numpy()

@@ -283,7 +283,7 @@ def test_lz4_random_blocks_are_stored(sq, cuda):
     assert payload.numel() == sq.lz4_bound(a.size)
 
 
-def test_lz4_noise_blocks_are_stored_early(sq, cuda, port, ref):
+def test_lz4_noise_blocks_are_stored_early(sq, cuda, port, ref_or_standin):
     """blocks with fewer than 128 match candidates — fixed-offset ones of the whole block + hash ones of the first 2 KiB —
     (camera-noise bit planes, 8-bit quantiser codes of a noisy stack) are stored without a parse (lz4_encode.cu: kEarlyBytes /
     kEarlyMin; tools/lz4_model2.c EARLY=2048 DUMP=1: noise blocks count <= 29, every compressible block of the sample sets >= 243). The
@@ -295,12 +295,12 @@ def test_lz4_noise_blocks_are_stored_early(sq, cuda, port, ref):
     payload = sq.lz4_encode_device(dev(cuda, codes))
     st = sq.last_lz4_stats()
     assert st["stored_blocks"] >= 0.9 * (codes.size // 16384), st
-    theirs = ref.lz4_encode(codes, nthreads=8).size    # (lz4_scheme<char>, the quantiser's tail)
+    theirs = ref_or_standin.lz4_encode(codes, nthreads=8).size    # (lz4_scheme<char>, the quantiser's tail)
     assert payload.numel() <= 1.03 * theirs, (payload.numel(), theirs)
     out = cuda.zeros(codes.size, dtype=cuda.uint8, device="cuda")
     assert sq.lz4_decode_device(payload, out) == codes.size
     assert np.array_equal(out.cpu().numpy(), codes)
-    rc, back = ref.lz4_decode_bytes(payload.cpu().numpy(), codes.size)
+    rc, back = ref_or_standin.lz4_decode_bytes(payload.cpu().numpy(), codes.size)
     assert rc == 0 and np.array_equal(back, codes)
     # bit planes of the same stack: the noise planes (low bits) are stored, everything else is parsed; a block that is noise
     # in its first 4 KiB only but full of runs elsewhere is parsed too (short-offset candidates count over the whole block)
@@ -330,11 +330,11 @@ def test_lz4_decodes_reference_payloads(sq, cuda, port, golden, key, src):
     assert np.array_equal(host16(out).ravel(), expect.ravel())
 
 
-def test_lz4_decodes_live_reference_payloads(sq, cuda, ref):
+def test_lz4_decodes_live_reference_payloads(sq, cuda, ref_or_standin):
     vol = numpy_volume((10, 256, 512), "ref", index=6)
-    planes = ref.bitswap_encode(1, vol)
+    planes = ref_or_standin.bitswap_encode(1, vol)
     for nthreads, config in ((1, b""), (8, b""), (2, b"n_chunks_of_input=5"), (1, b"blocksize_kb=64,framestep_kb=128")):
-        payload = ref.lz4_encode(planes, nthreads=nthreads, config=config)
+        payload = ref_or_standin.lz4_encode(planes, nthreads=nthreads, config=config)
         out = cuda.zeros(planes.size, dtype=cuda.int16, device="cuda")
         got = sq.lz4_decode_device(dev(cuda, payload), out)
         assert got == planes.nbytes, (nthreads, config)
@@ -360,11 +360,11 @@ def test_lz4_decodes_foreign_frames_with_any_offset(sq, cuda, port, period):
     assert np.array_equal(out.cpu().numpy(), a)
 
 
-def test_lz4_decodes_long_literal_runs_in_big_blocks(sq, cuda, ref):
+def test_lz4_decodes_long_literal_runs_in_big_blocks(sq, cuda, ref_or_standin):
     """a 256 KiB liblz4 block with ~200 KB of literals carries ~800 length bytes: the stream window must follow them"""
     rng = np.random.default_rng(8)
     a = np.concatenate([np.zeros(30000, np.uint8), rng.integers(0, 256, size=200000, dtype=np.uint8), np.zeros(32144, np.uint8)])
-    payload = ref.lz4_encode(a, nthreads=1)
+    payload = ref_or_standin.lz4_encode(a, nthreads=1)
     out = cuda.zeros(a.size, dtype=cuda.uint8, device="cuda")
     assert sq.lz4_decode_device(dev(cuda, payload), out) == a.size
     assert np.array_equal(out.cpu().numpy(), a)
@@ -377,13 +377,13 @@ def test_lz4_rejects_garbage(sq, cuda):
         sq.lz4_decode_device(dev(cuda, bad), out)
 
 
-def test_lz4_ratio_close_to_reference(sq, cuda, ref):
+def test_lz4_ratio_close_to_reference(sq, cuda, ref_or_standin):
     """compression ratio within 5 % of the reference's (lz4_scheme, 8 threads) on bit-plane data of both presets"""
     for preset in ("scmos", "ref"):
         vol = numpy_volume((32, 256, 512), preset, index=7)
-        planes = ref.bitswap_encode(1, vol)
+        planes = ref_or_standin.bitswap_encode(1, vol)
         ours = sq.lz4_encode_device(dev(cuda, planes)).numel()
-        theirs = ref.lz4_encode(planes, nthreads=8).size
+        theirs = ref_or_standin.lz4_encode(planes, nthreads=8).size
         assert ours <= theirs * 1.05, (preset, ours, theirs)
 
 
@@ -441,35 +441,35 @@ def test_java_boundary_cases(sq, cuda):
     assert np.array_equal(sq.decode(blob), vol)  # 8 distinct values: lossless mapping
 
 
-def test_blob_is_decodable_by_the_reference_chain(sq, cuda, port, ref):
+def test_blob_is_decodable_by_the_reference_chain(sq, cuda, port, ref_or_standin):
     """header parsed by the restated reference reader, payload by the reference's lz4 decoder + bitswap decoder"""
     vol = numpy_volume((16, 128, 256), "scmos", index=9)
     blob = sq.encode("bitswap1->lz4", vol)
     hdr = orc.unpack_header(blob.tobytes())
     assert hdr["pipeline"] == "bitswap1(num_bits_per_plane=1)->lz4(accel=1,blocksize_kb=256,framestep_kb=256,n_chunks_of_input=0)"
-    rc, out, _ = ref.pipeline_decode_stages(1, blob[hdr["size"]:], vol.size)
+    rc, out, _ = ref_or_standin.pipeline_decode_stages(1, blob[hdr["size"]:], vol.size)
     assert rc == 0 and np.array_equal(out.reshape(vol.shape), vol)
 
 
-def test_reference_blob_decodes_on_gpu(sq, cuda, ref):
+def test_reference_blob_decodes_on_gpu(sq, cuda, ref_or_standin):
     """blob = reference-style header (oracle restatement of header::pack) + payload made by the reference's stage chain"""
     vol = numpy_volume((16, 128, 256), "scmos", index=10)
     name = "bitswap1(num_bits_per_plane=1)->lz4(accel=1,blocksize_kb=256,framestep_kb=256,n_chunks_of_input=0)"
     for nthreads in (1, 8):
-        payload, _ = ref.pipeline_encode_stages(0, vol, nthreads)
+        payload, _ = ref_or_standin.pipeline_encode_stages(0, vol, nthreads)
         h = orc.pack_header(vol.shape, name, payload.size, version="0.5.2", headref="4c45a9b")
         blob = np.concatenate([np.frombuffer(h.encode(), dtype=np.uint8), payload])
         assert np.array_equal(sq.decode(blob), vol)
 
 
-def test_quantiser_blob_matches_reference_encode(sq, cuda, port, ref):
+def test_quantiser_blob_matches_reference_encode(sq, cuda, port, ref_or_standin):
     vol = numpy_volume((8, 128, 256), "ref", index=11)
     blob = sq.encode("quantiser", vol)
     hdr = orc.unpack_header(blob.tobytes())
-    codes_ref, dec_ref = ref.quantiser_encode(vol)
+    codes_ref, dec_ref = ref_or_standin.quantiser_encode(vol)
     assert np.array_equal(blob[hdr["size"]:], codes_ref.ravel())
     lut = orc.minors(orc.to_pairs(hdr["pipeline"])[0][1])["decode_lut_string"]
-    assert lut == ref.quantiser_lut_string(dec_ref)
+    assert lut == ref_or_standin.quantiser_lut_string(dec_ref)
 
 
 def test_device_api_matches_host_api(sq, cuda, port):

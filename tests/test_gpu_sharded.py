@@ -40,7 +40,7 @@ def _host_volume(cuda, kind, index):
 
 @pytest.mark.parametrize("kind", ["pinned", "pageable"])
 @pytest.mark.parametrize("pipeline", ["bitswap1->lz4", "rmestbkrd->bitswap1->lz4", "remove_background(threshold=110)->bitswap4->lz4"])
-def test_sharded_planes_blob_is_the_single_gpu_blob(sq, cuda, ref, two_gpus, pipeline, kind):
+def test_sharded_planes_blob_is_the_single_gpu_blob(sq, cuda, ref_or_standin, two_gpus, pipeline, kind):
     h = _host_volume(cuda, kind, 21)
     vol = h.numpy().view(np.uint16)
     sq.set_device(0)
@@ -71,7 +71,7 @@ def test_sharded_planes_blob_is_the_single_gpu_blob(sq, cuda, ref, two_gpus, pip
     assert np.array_equal(o, want.reshape(-1))
     # the reference's own decoder (LZ4F loop + scalar bitswap decode) reads the sharded blob
     if "bitswap1" in pipeline:
-        rc, back, _ = ref.pipeline_decode_stages(1, blobn[sq.header_size(blobn):], vol.size)
+        rc, back, _ = ref_or_standin.pipeline_decode_stages(1, blobn[sq.header_size(blobn):], vol.size)
         assert rc == 0 and np.array_equal(back, want.reshape(-1))
 
 

@@ -98,11 +98,11 @@ def test_u8_payload_is_the_oracles_bit_planes(sq, cuda, port):
     assert vol.size / blob.size > 1.5
 
 
-def test_reference_style_u8_blob_decodes_on_gpu(sq, cuda, ref):
+def test_reference_style_u8_blob_decodes_on_gpu(sq, cuda, ref_or_standin):
     """a blob put together from the reference's own uint8 stage code (bitswap_scheme<uint8_t>, lz4_scheme) + header"""
     vol = vol8((12, 96, 160), seed=4)
-    planes = ref.bitswap8_encode(1, vol)
-    payload = ref.lz4_encode(planes, nthreads=4)
+    planes = ref_or_standin.bitswap8_encode(1, vol)
+    payload = ref_or_standin.lz4_encode(planes, nthreads=4)
     name = "bitswap1(num_bits_per_plane=1)->lz4(accel=1,blocksize_kb=256,framestep_kb=256,n_chunks_of_input=0)"
     h = orc.pack_header(vol.shape, name, payload.size, raw_type="uint8", sizeof_raw=1, version="0.5.2", headref="4c45a9b")
     blob = np.concatenate([np.frombuffer(h.encode(), dtype=np.uint8), payload])

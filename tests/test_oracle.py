@@ -146,23 +146,38 @@ def test_lz4_decode_reference_payloads(port, golden):
     assert np.array_equal(got.view(np.uint16), golden["lz4_linked_in"])
 
 
-def test_lz4_port_encoder_is_reference_decodable(port, ref):
+def test_standin_lz4_encoder_writes_the_reference_payloads(port, golden):
+    """oracle.Standin restates the reference's lz4_scheme encode over liblz4: the same bytes as the reference made for the
+    golden vectors (one linked frame, a frame per 256 KiB chunk, cross-block matches) and the same default config"""
+    s = orc.standin()
+    if not s.available:
+        pytest.skip("liblz4 not present")
+    planes = port.bitswap_encode(1, golden["lz4_vol"])
+    assert np.array_equal(s.lz4_encode(planes, nthreads=1), golden["lz4_serial"])
+    assert np.array_equal(s.lz4_encode(planes, nthreads=4), golden["lz4_parallel"])
+    assert np.array_equal(s.lz4_encode(golden["lz4_linked_in"], nthreads=1), golden["lz4_linked"])
+    assert s.lz4_config(b"").encode() == golden["lz4_default_config"].tobytes()
+    rc, out = s.lz4_decode_u16(golden["lz4_parallel"], planes.size)
+    assert rc == 0 and np.array_equal(out, planes)
+
+
+def test_lz4_port_encoder_is_reference_decodable(port, ref_or_standin):
     rng = np.random.default_rng(9)
     a = np.repeat(rng.integers(0, 50, 40000, dtype=np.uint16), 7)[: 3 * 131072 + 77]
     payload = port.lz4_frames_encode(a, chunk=262144)
-    rc, out = ref.lz4_decode_u16(payload, a.size)
+    rc, out = ref_or_standin.lz4_decode_u16(payload, a.size)
     assert rc == 0 and np.array_equal(out, a)
     assert np.array_equal(port.lz4_frames_decode(payload, a.nbytes).view(np.uint16), a)
 
 
-def test_lz4_skippable_frames_pass_the_reference_decoder(port, ref):
+def test_lz4_skippable_frames_pass_the_reference_decoder(port, ref_or_standin):
     """the block index this library prepends is a skippable LZ4 frame; the reference's loop (lz4.hpp:257-339) skips it"""
     import struct
 
     a = (np.arange(1 << 16) % 251).astype(np.uint16)
     payload = port.lz4_frames_encode(a)
     skip = np.frombuffer(struct.pack("<II", 0x184D2A5B, 12) + b"x" * 12, dtype=np.uint8)
-    rc, out = ref.lz4_decode_u16(np.concatenate([skip, payload]), a.size)
+    rc, out = ref_or_standin.lz4_decode_u16(np.concatenate([skip, payload]), a.size)
     assert rc == 0 and np.array_equal(out, a)
     assert np.array_equal(port.lz4_frames_decode(np.concatenate([skip, payload]), a.nbytes).view(np.uint16), a)
 
@@ -194,9 +209,10 @@ def test_header_roundtrip():
 
 # ------------------------------------------------------------------------------------------------ uint8 volumes
 @pytest.mark.parametrize("w", [1, 2, 4])
-def test_bitswap8_kat_and_ref_live(port, ref, w):
+def test_bitswap8_kat_and_ref_live(port, w):
     """the scalar template of bitplane_reorder_scalar.hpp:27-116 with raw_type = uint8_t: first element of a group in the
     most significant field, most significant plane first; the C port equals the reference's own instantiation"""
+    ref = orc.ref()
     a = np.arange(8, dtype=np.uint8)
     e = port.bitswap8_encode(w, a)
     if w == 1:   # planes 7..3 empty; bit 2 of 0..7 = 00001111, bit 1 = 00110011, bit 0 = 01010101
@@ -213,7 +229,8 @@ def test_bitswap8_kat_and_ref_live(port, ref, w):
             assert np.array_equal(ref.bitswap8_decode(w, y), x)
 
 
-def test_remove_background8_vs_ref_live(port, ref):
+def test_remove_background8_vs_ref_live(port):
+    ref = orc.ref()
     x = np.random.default_rng(5).integers(0, 256, 5000, dtype=np.uint8)
     for t in (0, 1, 100, 255, 300):   # 300 is stored as uint8 (44), remove_background_scheme_impl.hpp:41-44
         y = port.remove_background8(x, t)

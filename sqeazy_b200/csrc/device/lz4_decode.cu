@@ -69,6 +69,8 @@ struct DecTables {
   uint32_t* dsize;               // decoded size (0 = unknown until the size pass)
   uint32_t* link;                // previous block of the same linked frame or kNoLink
   uint32_t* done;                // completion flags for linked frames
+  uint32_t* reach;               // linked blocks: bytes of their frame in front of them, at most 65535 (the directory stores
+                                 // the frame's first block here, lz4_offsets_kernel turns it into the byte count)
 };
 
 __device__ __forceinline__ uint32_t rd32(const uint8_t* p) {
@@ -206,6 +208,7 @@ __global__ void __launch_bounds__(kDirThreads) lz4_directory_kernel(const uint8_
               T.dsize[nb] = (word & kLz4StoredFlag) ? sz : (measure_all ? 0u : maxblock);
               if (measure_all && !(word & kLz4StoredFlag)) sh_need++;
               T.link[nb] = indep ? kNoLink : (nb > first_of_frame ? nb - 1 : kLinkHead);
+              T.reach[nb] = first_of_frame;
               if (!indep && nb > first_of_frame) sh_linked++;
               nb++;
               p += 4ull + sz + (bchk ? 4 : 0);
@@ -434,7 +437,7 @@ struct WinOut {
 // access; the per-sequence work therefore carries no bounds branches, only a sticky `bad` flag.
 __device__ __forceinline__ uint32_t decode_block_window(const uint8_t* __restrict__ s, uint32_t csize, WinOut& O,
                                                         uint8_t* ring8, const uint8_t* sbeg, const uint8_t* send,
-                                                        unsigned long long before, uint32_t link, const uint32_t* done,
+                                                        const uint32_t* reach, uint32_t link, const uint32_t* done,
                                                         bool& waited, uint32_t& err, int lane) {
   const uint8_t* A = reinterpret_cast<const uint8_t*>((uintptr_t)s & ~(uintptr_t)15);
   const uint32_t shift = (uint32_t)(s - A);
@@ -468,7 +471,8 @@ __device__ __forceinline__ uint32_t decode_block_window(const uint8_t* __restric
   auto do_match = [&](uint32_t op, uint32_t offset, uint32_t mlen) -> bool {
     if (offset > op) {
         // reaches in front of this block: only legal inside a linked frame, after the predecessor is complete
-        if (link == kNoLink || (unsigned long long)(offset - op) > before) { err = kErrBadBlock; return false; }
+        // (a linked block behind its frame's first one is block link + 1; its window is looked up only here, off the hot path)
+        if (link == kNoLink || offset - op > reach[link + 1]) { err = kErrBadBlock; return false; }
         if (!waited) {
           if (lane == 0) {
             while (atomicAdd(const_cast<uint32_t*>(done) + link, 0u) == 0u) __nanosleep(100);
@@ -953,6 +957,14 @@ __global__ void __launch_bounds__(kDirThreads) lz4_offsets_kernel(DecCtl* ctl, D
     running += total;
     __syncthreads();
   }
+  // the window of a linked block ends at the first byte of its frame (liblz4 refuses matches that reach further)
+  for (uint32_t i = tid; i < nblk; i += kDirThreads) {
+    const uint32_t link = T.link[i];
+    if (link != kNoLink && link != kLinkHead) {
+      const unsigned long long in_frame = T.dst_off[i] - T.dst_off[T.reach[i]];
+      T.reach[i] = (uint32_t)(in_frame < 65535ull ? in_frame : 65535ull);
+    }
+  }
   if (tid == 0) {
     ctl->total_decoded = running;
     // the reference accepts 0 < decoded <= expected (encoders/lz4.hpp:334-338); we refuse overruns
@@ -1037,8 +1049,8 @@ __global__ void __launch_bounds__(kWinWarps * 32, CTAS) lz4_decode_kernel(const 
       O.line_aligned = (((uintptr_t)d) & 127) == 0;
       O.overflow = false;
       O.lane = lane;
-      const unsigned long long before = link != kNoLink ? doff : 0ull;
-      const uint32_t got = decode_block_window(s, csize, O, ring8, src, src + src_bytes, before, link, T.done, waited, err, lane);
+      // a linked block may reach back to the first byte of its frame (T.reach), never into the frame in front of it
+      const uint32_t got = decode_block_window(s, csize, O, ring8, src, src + src_bytes, T.reach, link, T.done, waited, err, lane);
       if (!err) O.finish(got);
       if (!err && (O.overflow || got != dsize)) err = kErrSizeMismatch;
     }
@@ -1092,7 +1104,7 @@ __global__ void __launch_bounds__(256) lz4_decode_deferred_kernel(const uint8_t*
     uint8_t* d = dst + doff;
     uint16_t* o = origin + doff;
     // bytes that exist in front of this block inside its frame's reach
-    const unsigned long long before = link == kLinkHead ? 0ull : (doff < 65535ull ? doff : 65535ull);
+    const unsigned long long before = link == kLinkHead ? 0ull : T.reach[b];
     uint32_t err = 0;
     if (word & kLz4StoredFlag) {
       if (csize != dsize) err = kErrSizeMismatch;
@@ -1363,7 +1375,7 @@ size_t k_lz4_decode_capacity(uint64_t dst_bytes) { return (size_t)(dst_bytes / k
 
 size_t k_lz4_decode_workspace_bytes(uint64_t dst_bytes) {
   const size_t cap = k_lz4_decode_capacity(dst_bytes);
-  return 256 + cap * (8 + 8 + 4 + 4 + 4 + 4) + 8 * (cap / kTile + 2) + 256;
+  return 256 + cap * (8 + 8 + 4 + 4 + 4 + 4 + 4) + 8 * (cap / kTile + 2) + 256;
 }
 
 // Enqueues the whole decode; the status lands in workspace (see k_lz4_decode_status).
@@ -1378,6 +1390,7 @@ static DecTables dec_tables(void* workspace, uint64_t dst_bytes, unsigned long l
   T.dsize = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
   T.link = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
   T.done = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
+  T.reach = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
   if (tile_sums_out) *tile_sums_out = reinterpret_cast<unsigned long long*>((reinterpret_cast<uintptr_t>(p) + 7) & ~(uintptr_t)7);
   return T;
 }
@@ -1429,17 +1442,9 @@ int k_lz4_decode_linked(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, ui
 int k_lz4_decode_tables(const uint8_t* src, uint64_t src_bytes, uint64_t dst_bytes, void* workspace, int measure_all,
                         int allow_deferred, cudaStream_t st) {
   const size_t cap = k_lz4_decode_capacity(dst_bytes);
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  DecCtl* ctl = reinterpret_cast<DecCtl*>(ws);
-  DecTables T;
-  uint8_t* p = ws + 256;
-  T.src_off = reinterpret_cast<unsigned long long*>(p); p += 8 * cap;
-  T.dst_off = reinterpret_cast<unsigned long long*>(p); p += 8 * cap;
-  T.word = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
-  T.dsize = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
-  T.link = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
-  T.done = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
-  unsigned long long* tile_sums = reinterpret_cast<unsigned long long*>((reinterpret_cast<uintptr_t>(p) + 7) & ~(uintptr_t)7);
+  DecCtl* ctl = reinterpret_cast<DecCtl*>(workspace);
+  unsigned long long* tile_sums = nullptr;
+  const DecTables T = dec_tables(workspace, dst_bytes, &tile_sums);
   const uint32_t tiles = (uint32_t)(cap / kTile + 1), tile_grid = tiles < 1024u ? tiles : 1024u;
   SQYB_CUDA_OK(cudaMemsetAsync(ctl, 0, sizeof(DecCtl), st));
   lz4_directory_kernel<<<1, kDirThreads, 0, st>>>(src, src_bytes, ctl, T, (uint32_t)cap, measure_all,

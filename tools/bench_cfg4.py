@@ -1,4 +1,5 @@
-"""cfg4 probe: GPU decode of REFERENCE-produced bitswap1->lz4 blobs (oracle/_ref = the reference's stage code + liblz4):
+"""cfg4 probe: GPU decode of REFERENCE-produced bitswap1->lz4 blobs (oracle/_ref = the reference's stage code + liblz4;
+oracle.Standin, the reference's frame encoder restated over liblz4, where oracle/_ref is not built):
 serial mode = one block-linked frame (sqy CLI default), parallel mode = one frame per 256 KiB chunk.
 usage: bench_cfg4.py [ZxYxX] [serial|parallel] [both-routes]   (both-routes: the linked frame also block after block)"""
 import os, sys
@@ -9,8 +10,9 @@ from oracle import oracle as orc
 from sqeazy_b200.synth import numpy_volume
 
 shape = (64, 2048, 2048) if len(sys.argv) < 2 else tuple(int(v) for v in sys.argv[1].split("x"))
-ref = orc.ref()
+ref = orc.ref() if orc.ref().available else orc.standin()
 assert ref.available
+print(f"payloads from {type(ref).__name__}")
 torch.cuda.set_device(0); sq.set_device(0)
 vol = numpy_volume(shape, "scmos", index=0)
 name = "bitswap1(num_bits_per_plane=1)->lz4(accel=1,blocksize_kb=256,framestep_kb=256,n_chunks_of_input=0)"

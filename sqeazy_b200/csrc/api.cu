@@ -512,18 +512,57 @@ struct HostSink {
 };
 
 // ---- decode ----
+// The transpose back of a uint16 bitswapW that directly follows the LZ4 stage can run inside the LZ4 block decoder
+// (k_lz4_decode_fused). It pays from stacks of kFuseMinBytes on: there the 1.4 ms-per-4-GiB launch it replaces ran alone on the
+// stream; below, the transposes the decoder's warps do at L2 latency and the tail of the last ranges cost more than that launch
+// (measured, profiles/README.md round 3). SQYB_FUSE_TRANSPOSE=0 builds the two-launch route only (A/B: tools/ab_fused.py).
+#ifndef SQYB_FUSE_TRANSPOSE
+#define SQYB_FUSE_TRANSPOSE 1
+#endif
+#ifndef SQYB_FUSE_MIN_BYTES
+#define SQYB_FUSE_MIN_BYTES (uint64_t(1) << 30)
+#endif
+constexpr uint64_t kFuseMinBytes = SQYB_FUSE_MIN_BYTES;
+
+// where the fused decoder puts the voxels of the bit planes it decodes (lz4_decode_checked)
+struct FusedTarget {
+  int w;            // bits per plane of the bitswap
+  uint16_t* vox;    // 32-byte aligned, dst_bytes / 2 voxels
+};
+
+// `fuse`: when the stream turns out to be one frame of this library whose 16 KiB blocks hold exactly the dst_bytes plane bytes,
+// the planes are also transposed back into fuse->vox and *fused is set. The block table is built once either way: any other
+// stream goes on to the block decoders over that table.
 int lz4_decode_checked(Arena& A, const uint8_t* src, uint64_t nbytes, uint8_t* dst, uint64_t dst_bytes, uint64_t* decoded,
-                       cudaStream_t st) {
+                       cudaStream_t st, const FusedTarget* fuse = nullptr, bool* fused = nullptr) {
   void* ws = nullptr;
   if (A.get(kSlotWs, k_lz4_decode_workspace_bytes(dst_bytes), &ws)) return 1;
   for (int attempt = 0; attempt < 2; ++attempt) {
+    bool go_fused = false;
     {
       ScopedStageTimer tm(kTLz4Dec, st);
-      CKK(k_lz4_decode(src, nbytes, dst, dst_bytes, ws, attempt, 1, st));
+      CKK(k_lz4_decode_tables(src, nbytes, dst_bytes, ws, attempt, 1, st));
+      if (fuse && attempt == 0) {
+        uint32_t err = 0, own = 0, nblk = 0, bb = 0;
+        if (k_lz4_decode_peek(ws, &err, &own, &nblk, &bb, st)) return 1;
+        go_fused = !err && own && bb == (uint32_t)kLz4BlockBytes && (uint64_t)nblk * bb == dst_bytes;
+      }
+      if (go_fused) CKK(k_lz4_decode_fused(src, nbytes, dst, dst_bytes, ws, fuse->w, fuse->vox, st));
+      else CKK(k_lz4_decode_run(src, nbytes, dst, dst_bytes, ws, 0, 0, 0, 0, 0, st));
     }
     uint32_t err = 0, deferred = 0;
     uint64_t total = 0;
     if (k_lz4_decode_status(ws, &err, &total, &deferred, st)) return 1;
+    if (go_fused) {
+      // the index promised every block in full: a frame of this library that decodes to less is broken
+      if (err || total != dst_bytes) {
+        std::fprintf(stderr, "[sqeazy_b200] lz4 decode failed (code %u)\n", err ? err : 5u);
+        return 1;
+      }
+      if (decoded) *decoded = total;
+      *fused = true;
+      return 0;
+    }
     if (err == 0 && deferred) {
       // block-linked frames (reference serial mode / sqy CLI default): deferred cross-block references, lz4_decode.cu
       void* origins = nullptr;
@@ -636,6 +675,15 @@ int decode_device_impl(Arena& A, const Header& hdr, const Pipeline& pl, const ui
     if (pl.head[i].kind == StageKind::Bitshuffle) swaps.push_back(-1 - (int)pl.head[i].block_size);
   }
 
+  // The transpose back of a uint16 bitswapW that directly follows the LZ4 stage may run inside the LZ4 block decoder when the
+  // 16 KiB blocks hold whole groups of the P = 16/W planes (N a multiple of 8192P) and the stack is large enough to gain from it
+  // (kFuseMinBytes). A host call that ships the volume slab by slab behind the last transpose keeps that.
+  int fuse_w = 0;
+  if (SQYB_FUSE_TRANSPOSE && !u8 && raw_bytes >= kFuseMinBytes && pl.has_sink && pl.sink.kind == StageKind::Lz4 && !swaps.empty() &&
+      (swaps[0] == 1 || swaps[0] == 2 || swaps[0] == 4 || swaps[0] == 8) && N % (8192ull * (16 / swaps[0])) == 0 &&
+      !(host && swaps.size() == 1 && raw_bytes >= kStreamMinBytes))
+    fuse_w = swaps[0];
+
   uint16_t* bufs[2] = {nullptr, nullptr};
   auto scratch = [&](int which, uint16_t** out) -> int {
     if (!bufs[which]) {
@@ -657,12 +705,23 @@ int decode_device_impl(Arena& A, const Header& hdr, const Pipeline& pl, const ui
 
   const uint16_t* cur = nullptr;
   size_t remaining = swaps.size();
+  size_t first_swap = 0;   // 1: the LZ4 decoder did the first transpose back
   if (pl.has_sink) {
     uint16_t* out = nullptr;
     if (out_for(remaining, &out)) return 1;
     if (pl.sink.kind == StageKind::Lz4) {
+      FusedTarget target{fuse_w, nullptr};
+      if (fuse_w && out_for(remaining - 1, &target.vox)) return 1;
+      const bool try_fused = fuse_w && (((uintptr_t)target.vox) & 31) == 0;
+      bool fused = false;
       uint64_t got = 0;
-      if (lz4_decode_checked(A, d_payload, payload_bytes, reinterpret_cast<uint8_t*>(out), raw_bytes, &got, st)) return 11;
+      if (lz4_decode_checked(A, d_payload, payload_bytes, reinterpret_cast<uint8_t*>(out), raw_bytes, &got, st,
+                             try_fused ? &target : nullptr, &fused))
+        return 11;
+      if (fused) {
+        out = target.vox;
+        first_swap = 1;
+      }
     } else if (pl.sink.kind == StageKind::PassThrough) {
       if (pl.has_tail) {
         uint64_t got = 0;
@@ -707,7 +766,7 @@ int decode_device_impl(Arena& A, const Header& hdr, const Pipeline& pl, const ui
       cur = d_dst;
     }
   }
-  for (size_t k = 0; k < swaps.size(); ++k) {
+  for (size_t k = first_swap; k < swaps.size(); ++k) {
     uint16_t* out = nullptr;
     remaining = swaps.size() - 1 - k;
     if (remaining == 0) out = d_dst;

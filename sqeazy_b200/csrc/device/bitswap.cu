@@ -11,7 +11,8 @@
 // delta-swap stages (a PxP transpose of w-bit atoms in registers), and stores W consecutive
 // 32-bit words per plane, so a warp writes 128*W contiguous bytes per plane. The optional
 // threshold filter (remove_background, encoders/remove_background_scheme_impl.hpp:82-89) is
-// fused into the load (sat_sub_u16x2, common.cuh).
+// fused into the load (sat_sub_u16x2, common.cuh). The thread program lives in bitswap_thread.h.
+#include "bitswap_thread.h"
 #include "common.cuh"
 #include "kernels.h"
 
@@ -19,141 +20,23 @@ namespace sqyb {
 
 namespace {
 
-template <int W>
-struct Geo {
-  static constexpr int P = 16 / W;   // planes == voxels per group
-  static constexpr int SETS = W;     // register sets per thread (32 voxels / 2P)
-};
-
-__host__ __device__ constexpr uint32_t atom_mask16(int W, int k) {
-  // atoms c (c = 0 at bit 0) with (c & k) == 0
-  uint32_t m = 0;
-  for (int c = 0; c < 16 / W; ++c)
-    if ((c & k) == 0) m |= ((1u << W) - 1u) << (c * W);
-  return m;
-}
-
-template <int W>
-__device__ __forceinline__ void transpose_sets(uint32_t (&reg)[16]) {
-  constexpr int P = Geo<W>::P;
-#pragma unroll
-  for (int s = 0; s < Geo<W>::SETS; ++s) {
-#pragma unroll
-    for (int k = P / 2; k >= 1; k >>= 1) {
-      constexpr uint32_t dummy = 0;
-      (void)dummy;
-      const uint32_t m16 = atom_mask16(W, k);
-      const uint32_t mask = m16 | (m16 << 16);
-      const int sh = k * W;
-#pragma unroll
-      for (int r = 0; r < P; ++r) {
-        if ((r & k) == 0) {
-          uint32_t a = reg[s * P + r], b = reg[s * P + r + k];
-          uint32_t t = ((a >> sh) ^ b) & mask;
-          b ^= t;
-          a ^= t << sh;
-          reg[s * P + r] = a;
-          reg[s * P + r + k] = b;
-        }
-      }
-    }
-  }
-}
-
-__device__ __forceinline__ void ld256(const void* p, uint32_t* r) {
-  asm volatile("ld.global.nc.L1::no_allocate.v8.u32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "l"(p));
-}
-__device__ __forceinline__ void st256(void* p, const uint32_t* r) {
-  asm volatile("st.global.L1::no_allocate.v8.u32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "r"(r[0]), "r"(r[1]),
-               "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-               : "memory");
-}
+using bitswap_thread::Geo;
 
 // ---- encode: n32 = number of 32-voxel chunks, S = words per segment --------------------------
 template <int W, bool SUB>
 __global__ void __launch_bounds__(256) bitswap_encode_fast(const uint16_t* __restrict__ in, uint16_t* __restrict__ out,
                                                             uint64_t n32, uint64_t S, uint32_t thr /* threshold, < 65536 */) {
-  constexpr int P = Geo<W>::P;
   const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-  for (uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n32; t += stride) {
-    uint32_t L[16];
-    ld256(in + t * 32, L);
-    ld256(in + t * 32 + 16, L + 8);
-    if (SUB) {
-#pragma unroll
-      for (int k = 0; k < 16; ++k) L[k] = sat_sub_u16x2(L[k], thr);
-    }
-    uint32_t reg[16];
-#pragma unroll
-    for (int s = 0; s < Geo<W>::SETS; ++s) {
-#pragma unroll
-      for (int r = 0; r < P; ++r) {
-        const int j = P - 1 - r;
-        const int a = (2 * s) * P + j, b = (2 * s + 1) * P + j;
-        const uint32_t sel = (2 * (a & 1)) | ((2 * (a & 1) + 1) << 4) | ((4 + 2 * (b & 1)) << 8) | ((5 + 2 * (b & 1)) << 12);
-        reg[s * P + r] = __byte_perm(L[a >> 1], L[b >> 1], sel);
-      }
-    }
-    transpose_sets<W>(reg);
-    // plane p -> segment (P-1-p); this chunk's first group index is t*32/P
-#pragma unroll
-    for (int p = 0; p < P; ++p) {
-      uint32_t* dst = reinterpret_cast<uint32_t*>(out + (uint64_t)(P - 1 - p) * S + t * (32 / P));
-      if (W == 1) {
-        st_stream(dst, reg[p]);
-      } else if (W == 2) {
-        st_stream(reinterpret_cast<uint2*>(dst), make_uint2(reg[p], reg[P + p]));
-      } else if (W == 4) {
-        st_stream(reinterpret_cast<uint4*>(dst), make_uint4(reg[p], reg[P + p], reg[2 * P + p], reg[3 * P + p]));
-      } else {
-        uint32_t v[8];
-#pragma unroll
-        for (int s = 0; s < 8; ++s) v[s] = reg[s * P + p];
-        st256(dst, v);
-      }
-    }
-  }
+  for (uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n32; t += stride)
+    bitswap_thread::encode_chunk<W, SUB>(in, out, t, S, thr);
 }
 
 template <int W>
 __global__ void __launch_bounds__(256) bitswap_decode_fast(const uint16_t* __restrict__ in, uint16_t* __restrict__ out,
                                                             uint64_t n32, uint64_t S) {
-  constexpr int P = Geo<W>::P;
   const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
-  for (uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n32; t += stride) {
-    uint32_t reg[16];
-#pragma unroll
-    for (int p = 0; p < P; ++p) {
-      const uint32_t* src = reinterpret_cast<const uint32_t*>(in + (uint64_t)(P - 1 - p) * S + t * (32 / P));
-      if (W == 1) {
-        reg[p] = __ldg(src);
-      } else if (W == 2) {
-        uint2 v = __ldg(reinterpret_cast<const uint2*>(src));
-        reg[p] = v.x; reg[P + p] = v.y;
-      } else if (W == 4) {
-        uint4 v = ld_stream(reinterpret_cast<const uint4*>(src));
-        reg[p] = v.x; reg[P + p] = v.y; reg[2 * P + p] = v.z; reg[3 * P + p] = v.w;
-      } else {
-        uint32_t v[8];
-        ld256(src, v);
-#pragma unroll
-        for (int s = 0; s < 8; ++s) reg[s * P + p] = v[s];
-      }
-    }
-    transpose_sets<W>(reg);  // the atom transpose is an involution
-    uint32_t L[16];
-#pragma unroll
-    for (int k = 0; k < 16; ++k) {
-      const int m0 = 2 * k;
-      const int g = m0 / P, j0 = m0 % P, s = g / 2, h = g & 1;
-      const uint32_t sel = (2 * h) | ((2 * h + 1) << 4) | ((4 + 2 * h) << 8) | ((5 + 2 * h) << 12);
-      L[k] = __byte_perm(reg[s * P + (P - 1 - j0)], reg[s * P + (P - 2 - j0)], sel);
-    }
-    st256(out + t * 32, L);
-    st256(out + t * 32 + 16, L + 8);
-  }
+  for (uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; t < n32; t += stride)
+    bitswap_thread::decode_chunk<W, false>(in, out, t, S);
 }
 
 // ---- generic path: any N, any alignment; one thread per group of P voxels --------------------

@@ -82,6 +82,12 @@ int k_lz4_decode_tables(const uint8_t* src, uint64_t src_bytes, uint64_t dst_byt
                         cudaStream_t st);
 int k_lz4_decode_run(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, uint64_t dst_bytes, void* workspace, uint32_t first,
                      uint32_t count, uint32_t nsets, uint32_t set_stride, uint32_t slot, cudaStream_t st);
+// the block-decode launch for a stream that k_lz4_decode_tables + k_lz4_decode_peek found to be one frame of this library with
+// 16 KiB blocks that hold the bit planes of a uint16 bitswap`w` (w = 1, 2, 4, 8; plane_bytes = the volume's bytes, a multiple
+// of 16 KiB * 16/w): the planes are decoded into `planes` and transposed back into `vox` (32-byte aligned, plane_bytes / 2
+// voxels) by the same launch. Always the 48-register build of the decoder: the caller takes this route for stacks of 1 GiB and more
+int k_lz4_decode_fused(const uint8_t* src, uint64_t src_bytes, uint8_t* planes, uint64_t plane_bytes, void* workspace, int w,
+                       uint16_t* vox, cudaStream_t st);
 int k_lz4_decode_peek(void* workspace, uint32_t* error, uint32_t* own_frame, uint32_t* nblocks, uint32_t* block_bytes, cudaStream_t st);
 size_t k_lz4_decode_linked_workspace_bytes(uint64_t dst_bytes);
 int k_lz4_decode_linked(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, uint64_t dst_bytes, void* workspace, void* origins,

@@ -20,6 +20,7 @@
 //               ring; complete 512-byte chunks are flushed with 16-byte stores. Far matches and bytes in front of a
 //               linked block are read back from global memory; linked blocks wait on their predecessor's flag only
 //               when a match reaches in front of the block.
+#include "bitswap_thread.h"
 #include "common.cuh"
 #include "kernels.h"
 #include "lz4_format.h"
@@ -49,7 +50,8 @@ struct DecCtl {          // lives at the start of the workspace
   uint32_t ticket_size;
   uint32_t ticket_decode;
   uint32_t need_sizes;   // number of blocks whose decoded size must be measured
-  uint32_t reserved[3];
+  uint32_t own;          // the stream is exactly one frame of this library; fast_nblk / fast_bb hold its geometry
+  uint32_t reserved[2];
   // fast path: the stream is exactly one frame of this library -> the block table is built by many CTAs
   uint32_t fast, fast_nblk, fast_bb, fast_pad;
   unsigned long long fast_idx, fast_first, fast_raw;
@@ -71,6 +73,7 @@ struct DecTables {
   uint32_t* done;                // completion flags for linked frames
   uint32_t* reach;               // linked blocks: bytes of their frame in front of them, at most 65535 (the directory stores
                                  // the frame's first block here, lz4_offsets_kernel turns it into the byte count)
+  uint32_t* range;               // fused transpose: decoded blocks of each range of bit-plane blocks (lz4_decode_kernel)
 };
 
 __device__ __forceinline__ uint32_t rd32(const uint8_t* p) {
@@ -143,12 +146,16 @@ __global__ void __launch_bounds__(kDirThreads) lz4_directory_kernel(const uint8_
                   (src[fstart + 4] & 0x1D) == 0 /* no checksums, no content size, no dict */ &&
                   (unsigned long long)nblk * bb >= raw && (nblk == 0 || (unsigned long long)(nblk - 1) * bb < raw)) {
                 ours = true;
-                if ((unsigned long long)sh_nb + nblk > capacity) sh_err = kErrTooManyBlocks;
-                else if (pos == 0 && sh_nb == 0 && fstart + fbytes == src_bytes && nblk >= 2u * kTile && bb <= 65536u) {
-                  // the whole stream is one frame of ours: lz4_tile_sums_kernel + lz4_expand_kernel build the table
-                  ctl->fast = 1u;
+                const bool whole = pos == 0 && sh_nb == 0 && fstart + fbytes == src_bytes;
+                if (whole) {
+                  ctl->own = 1u;
                   ctl->fast_nblk = nblk;
                   ctl->fast_bb = bb;
+                }
+                if ((unsigned long long)sh_nb + nblk > capacity) sh_err = kErrTooManyBlocks;
+                else if (whole && nblk >= 2u * kTile && bb <= 65536u) {
+                  // the whole stream is one frame of ours: lz4_tile_sums_kernel + lz4_expand_kernel build the table
+                  ctl->fast = 1u;
                   ctl->fast_idx = body + sizeof(SqybIndexHeader);
                   ctl->fast_first = fstart + kLz4FrameHeaderBytes;
                   ctl->fast_raw = raw;
@@ -921,6 +928,7 @@ __global__ void __launch_bounds__(256) lz4_expand_kernel(const uint8_t* __restri
         T.link[i] = kNoLink;
         T.dst_off[i] = (unsigned long long)i * bb;
         T.done[i] = 0u;
+        T.range[i] = 0u;
       }
     }
     __syncthreads();
@@ -951,6 +959,7 @@ __global__ void __launch_bounds__(kDirThreads) lz4_offsets_kernel(DecCtl* ctl, D
       if (i < nblk) {
         T.dst_off[i] = off;
         T.done[i] = 0;
+        T.range[i] = 0;
         off += d[k];
       }
     }
@@ -972,17 +981,47 @@ __global__ void __launch_bounds__(kDirThreads) lz4_offsets_kernel(DecCtl* ctl, D
   }
 }
 
+// fused transpose (lz4_decode_kernel, FW != 0): a range's voxels go back in pieces of kPieceChunks 32-voxel chunks (16384 voxels).
+// The range counter holds the range's decoded blocks in its low half and the pieces claimed so far in its high half.
+constexpr uint32_t kPieceChunks = 512;
+
+// transposes the still unclaimed pieces of a complete range (its planes were written by other warps of this launch: fence, then
+// L2 loads). One chunk per lane at a time: a second one in flight costs the 48-register decoder spills.
+template <int FW>
+__device__ __forceinline__ void transpose_range(const uint16_t* planes, uint16_t* vox, uint32_t* counter, uint32_t range, uint64_t S,
+                                                int lane) {
+  constexpr uint32_t P = 16 / FW, kChunks = 8192u * P / 32u, kPieces = kChunks / kPieceChunks;
+  __threadfence();
+  while (true) {
+    uint32_t piece = 0;
+    if (lane == 0) piece = atomicAdd(counter, 1u << 16) >> 16;
+    piece = __shfl_sync(0xffffffffu, piece, 0);
+    if (piece >= kPieces) return;
+    const uint64_t t0 = (uint64_t)range * kChunks + piece * kPieceChunks;
+#pragma unroll 1
+    for (uint32_t c = lane; c < kPieceChunks; c += 32u) bitswap_thread::decode_chunk<FW, true>(planes, vox, t0 + c, S);
+  }
+}
+
 // Every block is taken here; the stored / closed-form blocks are handled inline: their 16-byte-store fills are
 // memory-bound and hide under the issue-bound decoding of the other warps, whereas a separate classification pass in
 // front of this kernel cost 0.63 ms per 4 GiB.
 // CTAS = CTAs per SM the registers are budgeted for: 5 (48 registers, 40 warps per SM) for streams that fill the machine,
 // 4 (64 registers, no spills) for small ones, which are bound by the serial chain of their slowest blocks and not by the
 // number of warps in flight (512x512x256 stack: 1.00 -> 0.75 ms; 4 GiB: 5.80 -> 6.25 ms)
-template <int CTAS>
+// FW != 0: the stream is one frame of this library holding the 16 KiB blocks of the P = 16/FW bit planes of a uint16 bitswapFW
+// (plane-major, bpp blocks per plane), and the kernel also transposes the planes back into `vox`. A range = block r of every
+// plane = voxels [r * 8192P, (r+1) * 8192P). Tickets are dealt range by range; the warp that finishes the last block of a
+// range (per-range counter) transposes it while its planes are still in L2, so the transpose, which needs memory bandwidth,
+// runs beside the decode of other blocks, which needs issue slots, instead of as a launch of its own behind them. Warps that find
+// no block left help with the pieces of the last ranges dealt instead of leaving a range's transpose to one warp at the end.
+// Two instantiations chosen at launch cost nothing; the plain one has no trace of the fused code.
+template <int CTAS, int FW>
 __global__ void __launch_bounds__(kWinWarps * 32, CTAS) lz4_decode_kernel(const uint8_t* __restrict__ src, uint64_t src_bytes,
                                                                         uint8_t* __restrict__ dst, DecCtl* ctl, DecTables T,
                                                                         uint32_t first, uint32_t count,
-                                                                        uint32_t nsets, uint32_t set_stride, uint32_t slot) {
+                                                                        uint32_t nsets, uint32_t set_stride, uint32_t slot,
+                                                                        uint16_t* __restrict__ vox, uint32_t bpp) {
   extern __shared__ __align__(16) unsigned char dsm[];
   if (ctl->error) return;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -993,11 +1032,30 @@ __global__ void __launch_bounds__(kWinWarps * 32, CTAS) lz4_decode_kernel(const 
   // bit planes that make up one z-slab), with a work counter of their own
   const uint32_t total = count ? count * nsets : nblocks;
   uint32_t* ticket = count ? &ctl->set_ticket[slot & 31u] : &ctl->ticket_decode;
+  constexpr uint32_t P = FW ? 16 / FW : 1;
+  const uint64_t S = (uint64_t)bpp * (kLz4BlockBytes / 2);   // (fused only) 16-bit words per plane
   while (true) {
     uint32_t b = 0;
     if (lane == 0) b = atomicAdd(ticket, 1u);
     b = __shfl_sync(0xffffffffu, b, 0);
+    if constexpr (FW != 0) {
+      if (b >= total) {
+        // every block is held by a running warp: wait for one of the last ranges dealt and take pieces of its transpose
+        constexpr uint32_t kPieces = 8192u * P / 32u / kPieceChunks;
+        const uint32_t nranges = total / P, h = b - total;
+        const uint32_t helped = min(nranges, gridDim.x * (uint32_t)kWinWarps / P + 2u);
+        if (h >= helped * kPieces) return;
+        const uint32_t r = nranges - 1u - h / kPieces;
+        if (lane == 0)
+          while ((atomicAdd(T.range + r, 0u) & 0xffffu) < P) __nanosleep(256);
+        __syncwarp();
+        transpose_range<FW>(reinterpret_cast<const uint16_t*>(dst), vox, T.range + r, r, S, lane);
+        continue;
+      }
+    }
     if (b >= total) return;
+    const uint32_t range = b / P;                      // (fused only)
+    if (FW) b = (b % P) * bpp + range;
     if (count) {
       const uint32_t j = b / count;
       b = first + j * set_stride + (b - j * count);
@@ -1055,6 +1113,19 @@ __global__ void __launch_bounds__(kWinWarps * 32, CTAS) lz4_decode_kernel(const 
       if (!err && (O.overflow || got != dsize)) err = kErrSizeMismatch;
     }
     if (err && lane == 0) atomicMax(&ctl->error, err);
+    if constexpr (FW != 0) {
+      // the planes of a complete range go back to voxels (a broken block sets ctl->error; the range is transposed all the same,
+      // inside `vox`, and the caller reports the error)
+      __syncwarp();
+      uint32_t last = 0;
+      if (lane == 0) {
+        __threadfence();
+        last = (atomicAdd(T.range + range, 1u) & 0xffffu) == P - 1u;
+      }
+      if (__shfl_sync(0xffffffffu, last, 0))
+        transpose_range<FW>(reinterpret_cast<const uint16_t*>(dst), vox, T.range + range, range, S, lane);
+      continue;
+    }
     // publish completion (linked frames): a block is done when it and its predecessor are done
     __syncwarp();
     if (lane == 0) {
@@ -1375,7 +1446,7 @@ size_t k_lz4_decode_capacity(uint64_t dst_bytes) { return (size_t)(dst_bytes / k
 
 size_t k_lz4_decode_workspace_bytes(uint64_t dst_bytes) {
   const size_t cap = k_lz4_decode_capacity(dst_bytes);
-  return 256 + cap * (8 + 8 + 4 + 4 + 4 + 4 + 4) + 8 * (cap / kTile + 2) + 256;
+  return 256 + cap * (8 + 8 + 4 + 4 + 4 + 4 + 4 + 4) + 8 * (cap / kTile + 2) + 256;
 }
 
 // Enqueues the whole decode; the status lands in workspace (see k_lz4_decode_status).
@@ -1391,6 +1462,7 @@ static DecTables dec_tables(void* workspace, uint64_t dst_bytes, unsigned long l
   T.link = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
   T.done = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
   T.reach = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
+  T.range = reinterpret_cast<uint32_t*>(p); p += 4 * cap;
   if (tile_sums_out) *tile_sums_out = reinterpret_cast<unsigned long long*>((reinterpret_cast<uintptr_t>(p) + 7) & ~(uintptr_t)7);
   return T;
 }
@@ -1466,9 +1538,37 @@ int k_lz4_decode_run(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, uint6
   const DecTables T = dec_tables(workspace, dst_bytes, nullptr);
   const size_t win_smem = kWinWarps * kWinWarpSmem;
   if (count == 0 && dst_bytes <= kSmallStreamBytes)
-    lz4_decode_kernel<4><<<kNumSMs * 4, kWinWarps * 32, win_smem, st>>>(src, src_bytes, dst, ctl, T, first, count, nsets, set_stride, slot);
+    lz4_decode_kernel<4, 0><<<kNumSMs * 4, kWinWarps * 32, win_smem, st>>>(src, src_bytes, dst, ctl, T, first, count, nsets, set_stride,
+                                                                           slot, nullptr, 0);
   else
-    lz4_decode_kernel<5><<<kNumSMs * 5, kWinWarps * 32, win_smem, st>>>(src, src_bytes, dst, ctl, T, first, count, nsets, set_stride, slot);
+    lz4_decode_kernel<5, 0><<<kNumSMs * 5, kWinWarps * 32, win_smem, st>>>(src, src_bytes, dst, ctl, T, first, count, nsets, set_stride,
+                                                                           slot, nullptr, 0);
+  SQYB_COUNT_LAUNCH(1);
+  return (int)cudaGetLastError();
+}
+
+// (the fused route is taken for stacks of 1 GiB and more, api.cu: kFuseMinBytes — always the 48-register build)
+template <int FW>
+static void launch_decode_fused(const uint8_t* src, uint64_t src_bytes, uint8_t* planes, DecCtl* ctl, const DecTables& T,
+                                uint16_t* vox, uint32_t bpp, cudaStream_t st) {
+  lz4_decode_kernel<5, FW><<<kNumSMs * 5, kWinWarps * 32, kWinWarps * kWinWarpSmem, st>>>(src, src_bytes, planes, ctl, T, 0, 0, 0, 0, 0,
+                                                                                        vox, bpp);
+}
+
+int k_lz4_decode_fused(const uint8_t* src, uint64_t src_bytes, uint8_t* planes, uint64_t plane_bytes, void* workspace, int w,
+                       uint16_t* vox, cudaStream_t st) {
+  if (w != 1 && w != 2 && w != 4 && w != 8) return -1;
+  const uint64_t range_bytes = (uint64_t)kLz4BlockBytes * (16 / w);
+  if (plane_bytes == 0 || plane_bytes % range_bytes || ((((uintptr_t)planes) | ((uintptr_t)vox)) & 31)) return -3;
+  DecCtl* ctl = reinterpret_cast<DecCtl*>(workspace);
+  const DecTables T = dec_tables(workspace, plane_bytes, nullptr);
+  const uint32_t bpp = (uint32_t)(plane_bytes / range_bytes);
+  switch (w) {
+    case 1: launch_decode_fused<1>(src, src_bytes, planes, ctl, T, vox, bpp, st); break;
+    case 2: launch_decode_fused<2>(src, src_bytes, planes, ctl, T, vox, bpp, st); break;
+    case 4: launch_decode_fused<4>(src, src_bytes, planes, ctl, T, vox, bpp, st); break;
+    case 8: launch_decode_fused<8>(src, src_bytes, planes, ctl, T, vox, bpp, st); break;
+  }
   SQYB_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }
@@ -1486,9 +1586,9 @@ int k_lz4_decode_peek(void* workspace, uint32_t* error, uint32_t* own_frame, uin
   SQYB_CUDA_OK(cudaMemcpyAsync(&h, workspace, sizeof(DecCtl), cudaMemcpyDeviceToHost, st));
   SQYB_CUDA_OK(cudaStreamSynchronize(st));
   *error = h.error;
-  *own_frame = h.fast;
-  *nblocks = h.fast ? h.fast_nblk : h.nblocks;
-  *block_bytes = h.fast ? h.fast_bb : 0u;
+  *own_frame = h.own;
+  *nblocks = h.own ? h.fast_nblk : h.nblocks;
+  *block_bytes = h.own ? h.fast_bb : 0u;
   return 0;
 }
 

@@ -312,6 +312,28 @@ int estimate_background_host(Arena& A, const uint16_t* h_src, uint64_t Z, uint64
 }
 
 // ---- encode ----
+// payload size of the LZ4 encode whose workspace is `ws`, once `st` has drained; the block-kind counts go to A.last_stats
+int lz4_encode_result(Arena& A, const void* ws, cudaStream_t st, uint64_t* payload_bytes) {
+  unsigned long long hres[4] = {0, 0, 0, 0};
+  CK(cudaMemcpyAsync(hres, ws, 32, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  *payload_bytes = hres[0];
+  const uint32_t* stats = reinterpret_cast<const uint32_t*>(reinterpret_cast<const uint8_t*>(hres) + 16);
+  A.last_stats[0] = stats[0]; A.last_stats[1] = stats[1]; A.last_stats[2] = stats[2]; A.last_stats[3] = (long)hres[0];
+  return 0;
+}
+
+// the blob's text header, right-aligned in its `reserve`-byte slot (leading blanks are what header::pack itself pads with)
+int header_slot(const Pipeline& pl, const std::vector<uint64_t>& shape, uint64_t payload_bytes, size_t reserve, std::string* slot) {
+  const std::string hdr = pack_header(pl.type_name(), pl.elem, shape, pl.canonical(), payload_bytes);
+  if (hdr.size() > reserve) {
+    std::fprintf(stderr, "[sqeazy_b200] header (%zu B) exceeds its slot (%zu B)\n", hdr.size(), reserve);
+    return 1;
+  }
+  *slot = std::string(reserve - hdr.size(), ' ') + hdr;
+  return 0;
+}
+
 int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src_any, const std::vector<uint64_t>& shape, uint8_t* d_dst,
                        uint64_t dst_cap, uint64_t* dst_bytes, const uint32_t* d_global_hist, cudaStream_t st) {
   Pipeline pl = pl_in;
@@ -399,13 +421,7 @@ int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src_any, c
       ScopedStageTimer tm(kTLz4Enc, st);
       CKK(k_lz4_encode(src, nbytes, payload, ws, lz4_pitch_hint(pl, shape), st));
     }
-    unsigned long long hres[4] = {0, 0, 0, 0};
-    CK(cudaMemcpyAsync(hres, ws, 32, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    payload_bytes = hres[0];
-    const uint32_t* stats = reinterpret_cast<const uint32_t*>(reinterpret_cast<const uint8_t*>(hres) + 16);
-    A.last_stats[0] = stats[0]; A.last_stats[1] = stats[1]; A.last_stats[2] = stats[2]; A.last_stats[3] = (long)payload_bytes;
-    return 0;
+    return lz4_encode_result(A, ws, st, &payload_bytes);
   };
 
   if (!pl.has_sink) {
@@ -465,14 +481,8 @@ int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src_any, c
     }
   }
 
-  // header, right-aligned in its slot (leading blanks are what header::pack itself pads with)
-  const std::string hdr = pack_header(pl.type_name(), pl.elem, shape, pl.canonical(), payload_bytes);
-  if (hdr.size() > reserve) {
-    std::fprintf(stderr, "[sqeazy_b200] header (%zu B) exceeds its slot (%zu B)\n", hdr.size(), reserve);
-    return 1;
-  }
-  std::string slot(reserve - hdr.size(), ' ');
-  slot += hdr;
+  std::string slot;
+  if (header_slot(pl, shape, payload_bytes, reserve, &slot)) return 1;
   CK(cudaMemcpyAsync(d_dst, slot.data(), slot.size(), cudaMemcpyHostToDevice, st));
   CK(cudaStreamSynchronize(st));
   *dst_bytes = reserve + payload_bytes;
@@ -542,11 +552,7 @@ int lz4_decode_checked(Arena& A, const uint8_t* src, uint64_t nbytes, uint8_t* d
     {
       ScopedStageTimer tm(kTLz4Dec, st);
       CKK(k_lz4_decode_tables(src, nbytes, dst_bytes, ws, attempt, 1, st));
-      if (fuse && attempt == 0) {
-        uint32_t err = 0, own = 0, nblk = 0, bb = 0;
-        if (k_lz4_decode_peek(ws, &err, &own, &nblk, &bb, st)) return 1;
-        go_fused = !err && own && bb == (uint32_t)kLz4BlockBytes && (uint64_t)nblk * bb == dst_bytes;
-      }
+      if (fuse && attempt == 0 && k_lz4_decode_own_frame(ws, dst_bytes, &go_fused, st)) return 1;
       if (go_fused) CKK(k_lz4_decode_fused(src, nbytes, dst, dst_bytes, ws, fuse->w, fuse->vox, st));
       else CKK(k_lz4_decode_run(src, nbytes, dst, dst_bytes, ws, 0, 0, 0, 0, 0, st));
     }
@@ -587,43 +593,15 @@ int lz4_decode_checked(Arena& A, const uint8_t* src, uint64_t nbytes, uint8_t* d
   return 1;
 }
 
-// Host decode of `[filters ->] bitswapN -> lz4` blobs of this library, >= 512 MiB: the LZ4 blocks are decoded slab by slab (the
-// blocks of all 16/N bit planes that make up a z-slab: one block-set launch), each slab is transposed back and leaves for the
-// host while the next one is decoded; only the first slab's kernels run in front of the bus. Returns -1 when the blob is not
-// of that kind (the caller takes the general route), 0 on success, an error code otherwise.
-int decode_streamed(Arena& A, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes, uint16_t* d_dst, uint64_t N,
-                    cudaStream_t st, HostSink* host, uint64_t slab_voxels = kStreamSlabBytes / 2, uint64_t min_bytes = kStreamMinBytes) {
-  const uint64_t raw_bytes = 2 * N;
-  if (pl.elem != 2 || !pl.has_sink || pl.sink.kind != StageKind::Lz4 || pl.has_tail || g_timing.load()) return -1;
-  if (raw_bytes < min_bytes || N % kStreamGrainVoxels) return -1;
-  int w = 0, nswaps = 0;
-  for (const Stage& s : pl.head) {
-    if (s.kind == StageKind::Bitswap) { w = s.w; nswaps++; }
-    else if (s.kind == StageKind::Bitshuffle || s.kind == StageKind::Diff) return -1;
-  }
-  if (nswaps != 1) return -1;
-  const int P = 16 / w;
-  void *ws = nullptr, *planes_v = nullptr;
-  if (A.get(kSlotWs, k_lz4_decode_workspace_bytes(raw_bytes), &ws) || A.get(kSlotA, raw_bytes, &planes_v)) return 1;
-  uint8_t* planes = static_cast<uint8_t*>(planes_v);
-  if (((((uintptr_t)planes) | ((uintptr_t)d_dst)) & 31) != 0) return -1;
-  CKK(k_lz4_decode_tables(d_payload, payload_bytes, raw_bytes, ws, 0, 0, st));
-  uint32_t err = 0, own = 0, nblk = 0, bb = 0;
-  if (k_lz4_decode_peek(ws, &err, &own, &nblk, &bb, st)) return 1;
-  if (err || !own || bb != kLz4BlockBytes || (uint64_t)nblk * bb != raw_bytes) return -1;
+// Runs make(first, count) on `st` for every slab of `slab` voxels of the N-voxel volume at d_vox; each slab leaves for the host on
+// the device's copy stream as soon as the kernels that made it are done. Returns make's code, or 0 when every slab is there.
+template <class Make>
+int ship_slabs(HostSink* host, const uint16_t* d_vox, uint64_t N, uint64_t slab, cudaStream_t st, Make&& make) {
   cudaStream_t cs = nullptr;
   if (copy_stream(&cs)) return 1;
-  // at most 32 slabs (one work counter each)
-  uint64_t slab = slab_voxels;
-  while ((N + slab - 1) / slab > 32) slab *= 2;
-  const uint32_t blocks_per_plane = (uint32_t)(raw_bytes / P / kLz4BlockBytes);
   EventList events;
-  uint32_t slot = 0;
-  for (uint64_t first = 0; first < N; first += slab, ++slot) {
-    const uint64_t count = std::min(slab, N - first);
-    CKK(k_lz4_decode_run(d_payload, payload_bytes, planes, raw_bytes, ws, (uint32_t)(2 * first / P / kLz4BlockBytes),
-                         (uint32_t)(2 * count / P / kLz4BlockBytes), (uint32_t)P, blocks_per_plane, slot, st));
-    if (k_bitswap_decode_range(w, reinterpret_cast<const uint16_t*>(planes), d_dst, N, first, count, st)) return 101;
+  for (uint64_t first = 0; first < N; first += slab) {
+    if (int rc = make(first, std::min(slab, N - first))) return rc;
     cudaEvent_t e = nullptr;
     if (events.next(&e)) return 1;
     CK(cudaEventRecord(e, st));
@@ -631,22 +609,74 @@ int decode_streamed(Arena& A, const Pipeline& pl, const uint8_t* d_payload, uint
   size_t i = 0;
   for (uint64_t first = 0; first < N; first += slab, ++i) {
     CK(cudaStreamWaitEvent(cs, events.ev[i], 0));
-    CK((cudaError_t)staged_d2h(host->dst + 2 * first, d_dst + first, 2 * std::min(slab, N - first), host->nthreads, cs));
+    CK((cudaError_t)staged_d2h(host->dst + 2 * first, d_vox + first, 2 * std::min(slab, N - first), host->nthreads, cs));
   }
-  uint64_t total = 0;
-  uint32_t none = 0;
-  if (k_lz4_decode_status(ws, &err, &total, &none, st)) return 1;
   CK(cudaStreamSynchronize(cs));
-  if (err || total != raw_bytes) {
+  return 0;
+}
+
+// Host decode of a blob of this library, >= min_bytes, of one of two kinds:
+//   planes: `[filters ->] bitswapW -> lz4`. A slab's LZ4 blocks are those of all P = 16/W bit planes that make up its voxels (one
+//           block-set launch of P sets), transposed back by k_bitswap_decode_range. The filters decode as identity, so any
+//           number of them may stand anywhere in the head: wider on purpose than what the streamed encoders write (shard_kind).
+//   codes:  `quantiser -> lz4`. A slab's LZ4 blocks are one run of the code stream, turned into voxels by k_lut_decode.
+// Every slab leaves for the host while the next one is decoded; only the first slab's kernels run in front of the bus. Returns -1
+// when the blob is not of these kinds (the caller takes the general route), 0 on success, an error code otherwise.
+int decode_streamed(Arena& A, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes, uint16_t* d_dst, uint64_t N,
+                    cudaStream_t st, HostSink* host, uint64_t slab_voxels = kStreamSlabBytes / 2, uint64_t min_bytes = kStreamMinBytes) {
+  if (pl.elem != 2 || !pl.has_sink || g_timing.load() || 2 * N < min_bytes) return -1;
+  const bool planes = pl.sink.kind == StageKind::Lz4 && !pl.has_tail;
+  int w = 0, nswaps = 0;
+  if (planes) {
+    for (const Stage& s : pl.head) {
+      if (s.kind == StageKind::Bitswap) { w = s.w; nswaps++; }
+      else if (s.kind == StageKind::Bitshuffle || s.kind == StageKind::Diff) return -1;
+    }
+    if (nswaps != 1 || N % kStreamGrainVoxels) return -1;
+  } else if (pl.sink.kind != StageKind::Quantiser || !pl.has_tail || !pl.head.empty() || !pl.sink.has_decode_lut || N % kLz4BlockBytes) {
+    return -1;
+  }
+  const uint64_t voxel_bytes = planes ? 2 : 1;                   // LZ4 bytes per voxel
+  const uint32_t sets = planes ? (uint32_t)(16 / w) : 1u;        // LZ4 streams a slab has blocks in
+  const uint64_t lz4_bytes = voxel_bytes * N;
+  const uint32_t set_stride = planes ? (uint32_t)(lz4_bytes / sets / kLz4BlockBytes) : 0u;
+  void *ws = nullptr, *dec_v = nullptr;
+  if (A.get(kSlotWs, k_lz4_decode_workspace_bytes(lz4_bytes), &ws) || A.get(kSlotA, lz4_bytes, &dec_v)) return 1;
+  uint8_t* dec = static_cast<uint8_t*>(dec_v);
+  uint16_t* d_lut = nullptr;
+  if (planes) {
+    if (((((uintptr_t)dec) | ((uintptr_t)d_dst)) & 31) != 0) return -1;
+  } else {
+    void* sp = nullptr;
+    if (A.get(kSlotSmall, 4 * 65536 * sizeof(uint32_t) + 4096, &sp)) return 1;
+    d_lut = reinterpret_cast<uint16_t*>(static_cast<uint8_t*>(sp) + 4 * 65536 * sizeof(uint32_t));
+    CK(cudaMemcpyAsync(d_lut, pl.sink.decode_lut, 512, cudaMemcpyHostToDevice, st));
+  }
+  CKK(k_lz4_decode_tables(d_payload, payload_bytes, lz4_bytes, ws, 0, 0, st));
+  bool own = false;
+  if (k_lz4_decode_own_frame(ws, lz4_bytes, &own, st)) return 1;
+  if (!own) return -1;
+  uint64_t slab = slab_voxels;
+  while ((N + slab - 1) / slab > 32) slab *= 2;   // one work counter per block-set launch, 32 of them
+  uint32_t slot = 0;
+  const int rc = ship_slabs(host, d_dst, N, slab, st, [&](uint64_t first, uint64_t count) -> int {
+    CKK(k_lz4_decode_run(d_payload, payload_bytes, dec, lz4_bytes, ws, (uint32_t)(voxel_bytes * first / sets / kLz4BlockBytes),
+                         (uint32_t)(voxel_bytes * count / sets / kLz4BlockBytes), sets, set_stride, slot++, st));
+    if (planes) return k_bitswap_decode_range(w, reinterpret_cast<const uint16_t*>(dec), d_dst, N, first, count, st) ? 101 : 0;
+    CKK(k_lut_decode(dec + first, d_dst + first, count, d_lut, st));
+    return 0;
+  });
+  if (rc) return rc;
+  uint32_t err = 0, none = 0;
+  uint64_t total = 0;
+  if (k_lz4_decode_status(ws, &err, &total, &none, st)) return 1;
+  if (err || total != lz4_bytes) {
     std::fprintf(stderr, "[sqeazy_b200] lz4 decode failed (code %u)\n", err);
-    return 11;
+    return planes ? 11 : 101;   // what the general route returns for a broken `lz4` sink / `lz4` tail
   }
   host->done = true;
   return 0;
 }
-
-int decode_streamed_codes(Arena& A, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes, uint16_t* d_dst, uint64_t N,
-                          cudaStream_t st, HostSink* host, uint64_t slab_voxels, uint64_t min_bytes);   // sharded.inl
 
 int decode_device_impl(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes,
                        void* d_dst_any, uint64_t dst_cap, cudaStream_t st, HostSink* host = nullptr) {
@@ -657,9 +687,7 @@ int decode_device_impl(Arena& A, const Header& hdr, const Pipeline& pl, const ui
   if (dst_cap < raw_bytes) return 1;
   if (N == 0) return 0;
   if (host) {
-    int rc = decode_streamed(A, pl, d_payload, payload_bytes, d_dst, N, st, host);
-    if (rc >= 0) return rc;
-    rc = decode_streamed_codes(A, pl, d_payload, payload_bytes, d_dst, N, st, host, kStreamSlabBytes / 2, kStreamMinBytes);
+    const int rc = decode_streamed(A, pl, d_payload, payload_bytes, d_dst, N, st, host);
     if (rc >= 0) return rc;
   }
 
@@ -790,22 +818,10 @@ int decode_device_impl(Arena& A, const Header& hdr, const Pipeline& pl, const ui
     if (remaining == 0 && host && !u8 && raw_bytes >= kStreamMinBytes && N % 128 == 0 && !g_timing.load() &&
         ((((uintptr_t)cur) | ((uintptr_t)out)) & 31) == 0) {
       // last stage of a host call: transpose back slab by slab, every slab leaves for the host as soon as it is done
-      cudaStream_t cs = nullptr;
-      if (copy_stream(&cs)) return 1;
-      EventList events;
-      const uint64_t slab = kStreamSlabBytes / 2;
-      for (uint64_t first = 0; first < N; first += slab) {
-        if (k_bitswap_decode_range(swaps[k], cur, out, N, first, std::min(slab, N - first), st)) return 100 + 1;
-        cudaEvent_t e = nullptr;
-        if (events.next(&e)) return 1;
-        CK(cudaEventRecord(e, st));
-      }
-      size_t i = 0;
-      for (uint64_t first = 0; first < N; first += slab, ++i) {
-        CK(cudaStreamWaitEvent(cs, events.ev[i], 0));
-        CK((cudaError_t)staged_d2h(host->dst + 2 * first, out + first, 2 * std::min(slab, N - first), host->nthreads, cs));
-      }
-      CK(cudaStreamSynchronize(cs));
+      const int rc = ship_slabs(host, out, N, kStreamSlabBytes / 2, st, [&](uint64_t first, uint64_t count) -> int {
+        return k_bitswap_decode_range(swaps[k], cur, out, N, first, count, st) ? 100 + 1 : 0;
+      });
+      if (rc) return rc;
       host->done = true;
       cur = out;
       continue;
@@ -1239,12 +1255,9 @@ int sqyx_lz4_encode_ex(const void* d_src, long nbytes, void* d_dst, long dst_cap
   const long pitch = pitch_bytes & ~(long)kLz4HintNoNoise;
   const uint32_t hint = (pitch > 0 && pitch <= 8192 ? (uint32_t)pitch : 0u) | (uint32_t)(pitch_bytes & (long)kLz4HintNoNoise);
   CKK(k_lz4_encode(static_cast<const uint8_t*>(d_src), (uint64_t)nbytes, static_cast<uint8_t*>(d_dst), ws, hint, st));
-  unsigned long long hres[4] = {0, 0, 0, 0};
-  CK(cudaMemcpyAsync(hres, ws, 32, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  *payload_bytes = (long)hres[0];
-  const uint32_t* stats = reinterpret_cast<const uint32_t*>(reinterpret_cast<const uint8_t*>(hres) + 16);
-  A->last_stats[0] = stats[0]; A->last_stats[1] = stats[1]; A->last_stats[2] = stats[2]; A->last_stats[3] = (long)hres[0];
+  uint64_t got = 0;
+  if (lz4_encode_result(*A, ws, st, &got)) return 1;
+  *payload_bytes = (long)got;
   return 0;
 }
 
@@ -1389,16 +1402,8 @@ int SQY_Pipeline_Max_Compressed_Length_3D_UI8(const char* pipeline, long* shape,
 // 16 KiB LZ4 blocks it completes in each of the 16/N bit planes are compressed, while the next slab is still on the bus.
 // Only the last slab's kernels, the offset scan and the compaction remain after the last byte has arrived. Decode: the final
 // inverse transpose runs slab by slab and every slab leaves for the host as soon as it is done.
-bool streamable_encode(const Pipeline& pl, const std::vector<uint64_t>& shape, uint64_t N) {
-  if (pl.elem != 2 || !pl.has_sink || pl.sink.kind != StageKind::Lz4 || pl.has_tail) return false;
-  if (2 * N < kStreamMinBytes || N % kStreamGrainVoxels) return false;
-  if (pl.head.size() == 1) return pl.head[0].kind == StageKind::Bitswap;
-  if (pl.head.size() != 2 || pl.head[1].kind != StageKind::Bitswap) return false;
-  if (pl.head[0].kind == StageKind::RmEstBkrd) return shape.size() == 3 && shape[0] >= 3;
-  return pl.head[0].kind == StageKind::RemoveBackground;
-}
-
-// returns 0 and the blob size, or an error; the caller has checked streamable_encode()
+// returns 0 and the blob size, or an error; the caller has checked that the pipeline is one of these (shard_kind: PlanesLz4),
+// that the stack has at least kStreamMinBytes and that N is a multiple of kStreamGrainVoxels
 int host_encode_streamed(Arena& A, const Pipeline& pl, const char* src, const std::vector<uint64_t>& shape, uint64_t N, char* dst,
                          uint64_t cap, uint64_t* out_bytes, int nthreads) {
   const uint64_t raw_bytes = 2 * N;
@@ -1453,18 +1458,9 @@ int host_encode_streamed(Arena& A, const Pipeline& pl, const char* src, const st
                             blocks_per_plane, lz4_pitch_hint(pl, shape), st));
   }
   CKK(k_lz4_encode_end(reinterpret_cast<const uint8_t*>(d_planes), raw_bytes, payload, ws, st));
-  unsigned long long hres[4] = {0, 0, 0, 0};
-  CK(cudaMemcpyAsync(hres, ws, 32, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  const uint64_t payload_bytes = hres[0];
-  const uint32_t* stats = reinterpret_cast<const uint32_t*>(reinterpret_cast<const uint8_t*>(hres) + 16);
-  A.last_stats[0] = stats[0]; A.last_stats[1] = stats[1]; A.last_stats[2] = stats[2]; A.last_stats[3] = (long)payload_bytes;
-
-  Pipeline named = pl;
-  const std::string hdr = pack_header(named.type_name(), named.elem, shape, named.canonical(), payload_bytes);
-  if (hdr.size() > reserve) return 1;
-  std::string slot(reserve - hdr.size(), ' ');
-  slot += hdr;
+  uint64_t payload_bytes = 0;
+  std::string slot;
+  if (lz4_encode_result(A, ws, st, &payload_bytes) || header_slot(pl, shape, payload_bytes, reserve, &slot)) return 1;
   CK(cudaMemcpyAsync(d_out, slot.data(), slot.size(), cudaMemcpyHostToDevice, st));
   CK((cudaError_t)staged_d2h(dst, d_out, reserve + payload_bytes, nthreads, st));
   CK(cudaStreamSynchronize(st));
@@ -1503,7 +1499,7 @@ static int host_encode(int elem, const char* pipeline, const char* src, long* sh
     DevLock dl;
     if (dl.acquire()) return 1;
     Arena* A = &dl.dev->arena;
-    if (streamable_encode(pl, shp, N) && !g_timing.load()) {
+    if (shard_kind(pl, shp) == ShardKind::PlanesLz4 && 2 * N >= kStreamMinBytes && N % kStreamGrainVoxels == 0 && !g_timing.load()) {
       uint64_t out = 0;
       if (host_encode_streamed(*A, pl, src, shp, N, dst, cap, &out, nthreads)) return 1;
       *dstlength = (long)out;

@@ -71,28 +71,27 @@ int k_lz4_encode_end(const uint8_t* src, uint64_t raw_bytes, uint8_t* dst, void*
 
 // lz4_decode.cu
 size_t k_lz4_decode_workspace_bytes(uint64_t dst_bytes);
+// A decode in two steps, so that callers can take the blocks of one z-slab at a time (the host entry points ship a slab while
+// the next one is decoded): the block table, then any number of block-set launches over it (count == 0: the whole stream).
 // allow_deferred: streams with many block-LINKED blocks (the reference's serial mode) only get their block table here; their
 // blocks are decoded by k_lz4_decode_linked (deferred cross-block references) once the caller has seen deferred_blocks > 0
 // in the status and provided the origin buffer.
-int k_lz4_decode(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, uint64_t dst_bytes, void* workspace, int measure_all,
-                 int allow_deferred, cudaStream_t st);
-// k_lz4_decode in two steps, for callers that want the blocks of one z-slab at a time (the host entry points ship a slab while
-// the next one is decoded): the block table, then any number of block-set launches over it (count == 0: the whole stream).
 int k_lz4_decode_tables(const uint8_t* src, uint64_t src_bytes, uint64_t dst_bytes, void* workspace, int measure_all, int allow_deferred,
                         cudaStream_t st);
 int k_lz4_decode_run(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, uint64_t dst_bytes, void* workspace, uint32_t first,
                      uint32_t count, uint32_t nsets, uint32_t set_stride, uint32_t slot, cudaStream_t st);
-// the block-decode launch for a stream that k_lz4_decode_tables + k_lz4_decode_peek found to be one frame of this library with
+// whether the table k_lz4_decode_tables left in `workspace` describes one frame of this library whose 16 KiB blocks hold exactly
+// dst_bytes: the geometry that the slab-by-slab host decode and the fused decoder rely on. Synchronises `st`.
+int k_lz4_decode_own_frame(void* workspace, uint64_t dst_bytes, bool* own_frame, cudaStream_t st);
+// the block-decode launch for a stream that k_lz4_decode_own_frame found to be one frame of this library with
 // 16 KiB blocks that hold the bit planes of a uint16 bitswap`w` (w = 1, 2, 4, 8; plane_bytes = the volume's bytes, a multiple
 // of 16 KiB * 16/w): the planes are decoded into `planes` and transposed back into `vox` (32-byte aligned, plane_bytes / 2
 // voxels) by the same launch. Always the 48-register build of the decoder: the caller takes this route for stacks of 1 GiB and more
 int k_lz4_decode_fused(const uint8_t* src, uint64_t src_bytes, uint8_t* planes, uint64_t plane_bytes, void* workspace, int w,
                        uint16_t* vox, cudaStream_t st);
-int k_lz4_decode_peek(void* workspace, uint32_t* error, uint32_t* own_frame, uint32_t* nblocks, uint32_t* block_bytes, cudaStream_t st);
 size_t k_lz4_decode_linked_workspace_bytes(uint64_t dst_bytes);
 int k_lz4_decode_linked(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, uint64_t dst_bytes, void* workspace, void* origins,
                         cudaStream_t st);
-// decoded-size limit of the lane-serial block decoder (0 = warp-per-block decoder only); returns the previous value
 // linked blocks from which a stream takes the deferred-reference path (default 8, 0 = never); returns the previous value
 long k_lz4_set_defer_min(long nblocks);
 int k_lz4_decode_status(void* workspace, uint32_t* error, uint64_t* total_decoded, uint32_t* deferred_blocks, cudaStream_t st);

@@ -1470,7 +1470,7 @@ static DecTables dec_tables(void* workspace, uint64_t dst_bytes, unsigned long l
 size_t k_lz4_decode_linked_workspace_bytes(uint64_t dst_bytes) { return 2 * (size_t)dst_bytes + 256; }
 
 // second step for streams of block-linked frames (k_lz4_decode_status reported them as deferred): `workspace` still
-// holds the block table of the k_lz4_decode call, `origins` has room for one uint16 per output byte
+// holds the block table of k_lz4_decode_tables, `origins` has room for one uint16 per output byte
 int k_lz4_decode_linked(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, uint64_t dst_bytes, void* workspace, void* origins,
                         cudaStream_t st) {
   (void)src_bytes;
@@ -1573,22 +1573,13 @@ int k_lz4_decode_fused(const uint8_t* src, uint64_t src_bytes, uint8_t* planes, 
   return (int)cudaGetLastError();
 }
 
-int k_lz4_decode(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, uint64_t dst_bytes, void* workspace, int measure_all,
-                 int allow_deferred, cudaStream_t st) {
-  if (int e = k_lz4_decode_tables(src, src_bytes, dst_bytes, workspace, measure_all, allow_deferred, st)) return e;
-  return k_lz4_decode_run(src, src_bytes, dst, dst_bytes, workspace, 0, 0, 0, 0, 0, st);
-}
-
-// what kind of stream the tables describe (synchronises the stream): one indexed frame of this library = regular geometry
-int k_lz4_decode_peek(void* workspace, uint32_t* error, uint32_t* own_frame, uint32_t* nblocks, uint32_t* block_bytes,
-                      cudaStream_t st) {
+// whether the table describes one indexed frame of this library whose 16 KiB blocks hold exactly dst_bytes (synchronises the
+// stream)
+int k_lz4_decode_own_frame(void* workspace, uint64_t dst_bytes, bool* own_frame, cudaStream_t st) {
   DecCtl h;
   SQYB_CUDA_OK(cudaMemcpyAsync(&h, workspace, sizeof(DecCtl), cudaMemcpyDeviceToHost, st));
   SQYB_CUDA_OK(cudaStreamSynchronize(st));
-  *error = h.error;
-  *own_frame = h.own;
-  *nblocks = h.own ? h.fast_nblk : h.nblocks;
-  *block_bytes = h.own ? h.fast_bb : 0u;
+  *own_frame = !h.error && h.own && h.fast_bb == (uint32_t)kLz4BlockBytes && (uint64_t)h.fast_nblk * h.fast_bb == dst_bytes;
   return 0;
 }
 

@@ -947,24 +947,10 @@ __global__ void __launch_bounds__(256) lz4_scatter_kernel(const uint8_t* __restr
 __global__ void lz4_write_prefix_kernel(uint8_t* dst, uint64_t raw_bytes, uint32_t nblocks,
                                         unsigned long long* payload_bytes_out) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
-  auto put32 = [&](uint64_t off, uint32_t v) { for (int k = 0; k < 4; ++k) dst[off + k] = (uint8_t)(v >> (8 * k)); };
-  auto put64 = [&](uint64_t off, uint64_t v) { for (int k = 0; k < 8; ++k) dst[off + k] = (uint8_t)(v >> (8 * k)); };
-  put32(0, kSqybSkippableMagic);
-  put32(4, (uint32_t)(sizeof(SqybIndexHeader) + 4ull * nblocks));
-  put32(8, kSqybIndexMagic);
-  put32(12, 1u);
-  put32(16, (uint32_t)kB);
-  put32(20, nblocks);
-  put64(24, raw_bytes);
-  put64(32, kLz4FrameHeaderBytes + kLz4EndMarkBytes);
-  const uint64_t f = kSkippableHeaderBytes + sizeof(SqybIndexHeader) + 4ull * nblocks;
-  put32(f, kLz4FrameMagic);
-  dst[f + 4] = 0x60;  // FLG: version 01, block independent
-  dst[f + 5] = 0x40;  // BD: 64 KiB max block
-  dst[f + 6] = 0x82;  // HC = (xxh32(FLG BD) >> 8) & 0xff
+  const uint64_t end = lz4_write_prefix(dst, nblocks, raw_bytes, kLz4FrameHeaderBytes + kLz4EndMarkBytes);
   if (nblocks == 0) {
-    put32(f + 7, 0);
-    *payload_bytes_out = f + 7 + 4;
+    lz4_put32(dst + end, 0);   // EndMark
+    *payload_bytes_out = end + kLz4EndMarkBytes;
   }
 }
 

@@ -229,6 +229,23 @@ uint64_t shape_product(const std::vector<uint64_t>& shape) {
   return shape.empty() ? 0 : n;
 }
 
+// the arena's small slot: what the histogram, quantiser and estimate steps keep on the device. Fields that overlap are never
+// used by the same step.
+struct SmallSlot {
+  uint32_t* hist;      // four 65536-bin histograms (the quantiser uses the first)
+  uint8_t* enc_lut;    // quantiser encode LUT, 65536 codes, over the second histogram
+  uint16_t* dec_lut;   // quantiser decode LUT, 256 voxels, behind the histograms
+  uint32_t* support;   // the estimate's 16 support indices, behind the histograms
+};
+
+int small_slot(Arena& A, SmallSlot* s) {
+  void* p = nullptr;
+  if (A.get(kSlotSmall, 4 * 65536 * sizeof(uint32_t) + 4096, &p)) return 1;
+  uint32_t* h = static_cast<uint32_t*>(p);
+  *s = SmallSlot{h, reinterpret_cast<uint8_t*>(h + 65536), reinterpret_cast<uint16_t*>(h + 4 * 65536), h + 4 * 65536};
+  return 0;
+}
+
 // ---- rmestbkrd threshold: GPU histograms of the sampled faces/rows + host support formula ----
 // what the estimate reads, as device pointers: the first `portion` voxels of the z = 0 and z = Z-1 faces and the rows y = 0 /
 // y = Y-1 at z in {1, Z/2, Z-2} (nullptr: that z does not exist). The callers whose stack is not resident as a whole (streamed
@@ -256,9 +273,9 @@ EstimateSamples estimate_samples_of(const uint16_t* d_src, uint64_t Z, uint64_t 
 }
 
 int estimate_background_samples(Arena& A, const EstimateSamples& S, float* supports, int* threshold, cudaStream_t st) {
-  void* p = nullptr;
-  if (A.get(kSlotSmall, 4 * 65536 * sizeof(uint32_t) + 4096, &p)) return 1;
-  uint32_t* d_h = static_cast<uint32_t*>(p);
+  SmallSlot small;
+  if (small_slot(A, &small)) return 1;
+  uint32_t* d_h = small.hist;
   CK(cudaMemsetAsync(d_h, 0, 4 * 65536 * sizeof(uint32_t), st));
   // z = 0 and z = Z-1 faces (first `portion` elements), background_scheme_utils.hpp:57-77
   CKK(k_histogram_u16(S.face[0], S.portion, d_h, st));
@@ -267,10 +284,9 @@ int estimate_background_samples(Arena& A, const EstimateSamples& S, float* suppo
     for (int k = 0; k < 3; ++k)
       if (S.row[i][k]) CKK(k_histogram_u16(S.row[i][k], S.X, d_h + (2 + i) * 65536, st));
   // support index of the four histograms on the device; 64 bytes come back instead of 1 MiB of bins
-  uint32_t* d_idx = d_h + 4 * 65536;
-  CKK(k_support_index(d_h, 4, 0.99f, d_idx, st));
+  CKK(k_support_index(d_h, 4, 0.99f, small.support, st));
   uint32_t idx[16];
-  CK(cudaMemcpyAsync(idx, d_idx, sizeof(idx), cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(idx, small.support, sizeof(idx), cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   float mn = 0.f;
   for (int i = 0; i < 4; ++i) {
@@ -288,13 +304,15 @@ int estimate_background(Arena& A, const uint16_t* d_src, uint64_t Z, uint64_t Y,
   return estimate_background_samples(A, estimate_samples_of(d_src, Z, Y, X, l2), supports, threshold, st);
 }
 
-// the same from a stack in HOST memory: only the sampled pieces cross the bus, packed into `d_scratch` (>= 4*portion + 12*X bytes)
-int estimate_background_host(Arena& A, const uint16_t* h_src, uint64_t Z, uint64_t Y, uint64_t X, uint16_t* d_scratch, int* threshold,
-                             cudaStream_t st) {
+// the same from a stack in HOST memory: only the sampled pieces cross the bus, packed into the arena's kSlotB (which the streamed
+// and sharded host encoders have no other use for)
+int estimate_background_host(Arena& A, const uint16_t* h_src, uint64_t Z, uint64_t Y, uint64_t X, int* threshold, cudaStream_t st) {
   if (Z == 0 || Y == 0 || X == 0) return 1;
   const EstimateSamples H = estimate_samples_of(h_src, Z, Y, X, host_l2_cache_bytes());
   EstimateSamples D = H;
-  uint16_t* q = d_scratch;
+  void* scratch = nullptr;
+  if (A.get(kSlotB, 2 * (2 * H.portion + 6 * X), &scratch)) return 1;
+  uint16_t* q = static_cast<uint16_t*>(scratch);
   for (int f = 0; f < 2; ++f) {
     CK(cudaMemcpyAsync(q, H.face[f], 2 * H.portion, cudaMemcpyHostToDevice, st));
     D.face[f] = q;
@@ -332,6 +350,14 @@ int header_slot(const Pipeline& pl, const std::vector<uint64_t>& shape, uint64_t
   }
   *slot = std::string(reserve - hdr.size(), ' ') + hdr;
   return 0;
+}
+
+// the quantiser's LUTs for the histogram of a whole stack: the encode LUT into enc (65536 codes); the decode LUT travels in the
+// header (quantiser_scheme_impl.hpp:200-204)
+void quantiser_luts(Pipeline& pl, const uint32_t* hist, uint8_t* enc) {
+  uint16_t dec[256];
+  quantiser_luts_from_histogram(hist, enc, dec);
+  pl.sink.kv["decode_lut_string"] = std::string(kVerbatimOpen) + base64_encode(dec, sizeof(dec)) + kVerbatimClose;
 }
 
 int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src_any, const std::vector<uint64_t>& shape, uint8_t* d_dst,
@@ -441,10 +467,9 @@ int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src_any, c
     }
   } else {  // Quantiser
     if (u8) return 1;   // (the planner never builds it for uint8)
-    void* sp = nullptr;
-    if (A.get(kSlotSmall, 4 * 65536 * sizeof(uint32_t) + 4096, &sp)) return 1;
-    uint32_t* d_hist = static_cast<uint32_t*>(sp);
-    uint8_t* d_lut = reinterpret_cast<uint8_t*>(d_hist + 65536);
+    SmallSlot small;
+    if (small_slot(A, &small)) return 1;
+    uint32_t* d_hist = small.hist;
     std::vector<uint32_t> h(65536);
     if (N > 0 || d_global_hist) {
       if (d_global_hist) {
@@ -459,23 +484,20 @@ int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src_any, c
       CK(cudaStreamSynchronize(st));
     }
     std::vector<uint8_t> enc(65536);
-    uint16_t dec[256];
-    quantiser_luts_from_histogram(h.data(), enc.data(), dec);
-    // the decode LUT travels in the header (quantiser_scheme_impl.hpp:200-204)
-    pl.sink.kv["decode_lut_string"] = std::string(kVerbatimOpen) + base64_encode(dec, sizeof(dec)) + kVerbatimClose;
-    CK(cudaMemcpyAsync(d_lut, enc.data(), 65536, cudaMemcpyHostToDevice, st));
+    quantiser_luts(pl, h.data(), enc.data());
+    CK(cudaMemcpyAsync(small.enc_lut, enc.data(), 65536, cudaMemcpyHostToDevice, st));
     if (pl.has_tail) {
       uint16_t* codes16 = nullptr;
       if (next_buf(&codes16)) return 1;
       uint8_t* codes = reinterpret_cast<uint8_t*>(codes16);
       {
         ScopedStageTimer tm(kTLutApply, st);
-        CKK(k_lut_apply(cur, codes, N, d_lut, st));
+        CKK(k_lut_apply(cur, codes, N, small.enc_lut, st));
       }
       if (lz4_into_payload(codes, N)) return 1;
     } else {
       if (payload_cap < N) return 1;
-      CKK(k_lut_apply(cur, payload, N, d_lut, st));
+      CKK(k_lut_apply(cur, payload, N, small.enc_lut, st));
       CK(cudaStreamSynchronize(st));  // enc (host vector) must outlive the H2D copy
       payload_bytes = N;
     }
@@ -493,6 +515,23 @@ int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src_any, c
 constexpr uint64_t kStreamSlabBytes = uint64_t(256) << 20;
 constexpr uint64_t kStreamMinBytes = uint64_t(512) << 20;
 constexpr uint64_t kStreamGrainVoxels = 131072;   // a 16 KiB block of a 1-bit plane covers 131072 voxels (8192 * P for wider atoms)
+
+// The LZ4 stream of n voxels that the host entry points encode and decode slab by slab: `sets` streams of equal length one
+// after the other, in 16 KiB blocks. Voxels [first, first + count) make up blocks [block(first), block(first + count)) of every
+// set when first and count are multiples of the block's voxels in one set.
+struct StreamGeom {
+  uint64_t n;              // voxels
+  uint32_t sets;           // the 16/w bit planes of a uint16 bitswapW, or the one stream of 8-bit quantiser codes
+  uint32_t voxel_bytes;    // LZ4 bytes per voxel, over all sets
+  static StreamGeom planes(uint64_t n, int w) { return {n, (uint32_t)(16 / w), 2}; }
+  static StreamGeom codes(uint64_t n) { return {n, 1, 1}; }
+  StreamGeom of(uint64_t voxels) const { return {voxels, sets, voxel_bytes}; }   // the same kind of stream over other voxels
+  uint64_t bytes() const { return voxel_bytes * n; }
+  uint64_t blocks() const { return bytes() / kLz4BlockBytes; }
+  uint32_t block(uint64_t v) const { return (uint32_t)(voxel_bytes * v / sets / kLz4BlockBytes); }
+  uint32_t set_blocks() const { return block(n); }   // blocks per set: the set stride
+};
+
 int copy_stream(cudaStream_t* cs) {   // of the current device; its lock is held
   int dev = 0;
   CK(cudaGetDevice(&dev));
@@ -615,6 +654,50 @@ int ship_slabs(HostSink* host, const uint16_t* d_vox, uint64_t N, uint64_t slab,
   return 0;
 }
 
+// The mirror image of ship_slabs: sends the n voxels at h_src to d_vox slab by slab on the device's copy stream, and `st` runs
+// make(first, count) on a slab as soon as it has arrived. ahead() runs once, when the first slab's copy has been issued and
+// before `st` waits for it: the bus does not wait for what it puts on `st`, and that work does not wait for the bus.
+template <class Ahead, class Make>
+int take_slabs(const char* h_src, uint16_t* d_vox, uint64_t n, uint64_t slab, int nthreads, cudaStream_t st, Ahead&& ahead, Make&& make) {
+  cudaStream_t cs = nullptr;
+  if (copy_stream(&cs)) return 1;
+  EventList events;
+  for (uint64_t first = 0; first < n; first += slab) {
+    const uint64_t count = std::min(slab, n - first);
+    CK((cudaError_t)staged_h2d(d_vox + first, h_src + 2 * first, 2 * count, nthreads, cs));
+    cudaEvent_t arrived = nullptr;
+    if (events.next(&arrived)) return 1;
+    CK(cudaEventRecord(arrived, cs));
+    if (first == 0)
+      if (int rc = ahead()) return rc;
+    CK(cudaStreamWaitEvent(st, arrived, 0));
+    if (int rc = make(first, count)) return rc;
+  }
+  return 0;
+}
+
+// LZ4 of the bit planes (bitswap w) of the geo.n uint16 voxels at h_src. The stack arrives in d_in slab by slab; each slab is
+// filtered with the threshold and transposed into its place in the plane-major d_planes, and the blocks it completes in every
+// plane are compressed into d_lz4 while the next slab is on the bus. threshold(&t) gives the threshold once the first slab is
+// on its way (take_slabs' ahead).
+template <class Threshold>
+int encode_planes_slabs(const StreamGeom& geo, int w, Threshold&& threshold, uint32_t pitch_hint, uint64_t slab, const char* h_src,
+                        uint16_t* d_in, uint16_t* d_planes, uint8_t* d_lz4, void* ws, int nthreads, cudaStream_t st) {
+  const uint8_t* planes = reinterpret_cast<const uint8_t*>(d_planes);
+  int thr = 0;
+  CKK(k_lz4_encode_begin(geo.bytes(), d_lz4, ws, st));
+  const int rc = take_slabs(h_src, d_in, geo.n, slab, nthreads, st, [&] { return threshold(&thr); },
+                            [&](uint64_t first, uint64_t count) -> int {
+                              CKK(k_bitswap_encode_range(w, d_in, d_planes, geo.n, first, count, thr, st));
+                              CKK(k_lz4_encode_blocks(planes, geo.bytes(), d_lz4, ws, geo.block(first), geo.block(count), geo.sets,
+                                                      geo.set_blocks(), pitch_hint, st));
+                              return 0;
+                            });
+  if (rc) return rc;
+  CKK(k_lz4_encode_end(planes, geo.bytes(), d_lz4, ws, st));
+  return 0;
+}
+
 // Host decode of a blob of this library, >= min_bytes, of one of two kinds:
 //   planes: `[filters ->] bitswapW -> lz4`. A slab's LZ4 blocks are those of all P = 16/W bit planes that make up its voxels (one
 //           block-set launch of P sets), transposed back by k_bitswap_decode_range. The filters decode as identity, so any
@@ -636,41 +719,36 @@ int decode_streamed(Arena& A, const Pipeline& pl, const uint8_t* d_payload, uint
   } else if (pl.sink.kind != StageKind::Quantiser || !pl.has_tail || !pl.head.empty() || !pl.sink.has_decode_lut || N % kLz4BlockBytes) {
     return -1;
   }
-  const uint64_t voxel_bytes = planes ? 2 : 1;                   // LZ4 bytes per voxel
-  const uint32_t sets = planes ? (uint32_t)(16 / w) : 1u;        // LZ4 streams a slab has blocks in
-  const uint64_t lz4_bytes = voxel_bytes * N;
-  const uint32_t set_stride = planes ? (uint32_t)(lz4_bytes / sets / kLz4BlockBytes) : 0u;
+  const StreamGeom geo = planes ? StreamGeom::planes(N, w) : StreamGeom::codes(N);
   void *ws = nullptr, *dec_v = nullptr;
-  if (A.get(kSlotWs, k_lz4_decode_workspace_bytes(lz4_bytes), &ws) || A.get(kSlotA, lz4_bytes, &dec_v)) return 1;
+  if (A.get(kSlotWs, k_lz4_decode_workspace_bytes(geo.bytes()), &ws) || A.get(kSlotA, geo.bytes(), &dec_v)) return 1;
   uint8_t* dec = static_cast<uint8_t*>(dec_v);
-  uint16_t* d_lut = nullptr;
+  SmallSlot small{};
   if (planes) {
     if (((((uintptr_t)dec) | ((uintptr_t)d_dst)) & 31) != 0) return -1;
   } else {
-    void* sp = nullptr;
-    if (A.get(kSlotSmall, 4 * 65536 * sizeof(uint32_t) + 4096, &sp)) return 1;
-    d_lut = reinterpret_cast<uint16_t*>(static_cast<uint8_t*>(sp) + 4 * 65536 * sizeof(uint32_t));
-    CK(cudaMemcpyAsync(d_lut, pl.sink.decode_lut, 512, cudaMemcpyHostToDevice, st));
+    if (small_slot(A, &small)) return 1;
+    CK(cudaMemcpyAsync(small.dec_lut, pl.sink.decode_lut, 512, cudaMemcpyHostToDevice, st));
   }
-  CKK(k_lz4_decode_tables(d_payload, payload_bytes, lz4_bytes, ws, 0, 0, st));
+  CKK(k_lz4_decode_tables(d_payload, payload_bytes, geo.bytes(), ws, 0, 0, st));
   bool own = false;
-  if (k_lz4_decode_own_frame(ws, lz4_bytes, &own, st)) return 1;
+  if (k_lz4_decode_own_frame(ws, geo.bytes(), &own, st)) return 1;
   if (!own) return -1;
   uint64_t slab = slab_voxels;
   while ((N + slab - 1) / slab > 32) slab *= 2;   // one work counter per block-set launch, 32 of them
   uint32_t slot = 0;
   const int rc = ship_slabs(host, d_dst, N, slab, st, [&](uint64_t first, uint64_t count) -> int {
-    CKK(k_lz4_decode_run(d_payload, payload_bytes, dec, lz4_bytes, ws, (uint32_t)(voxel_bytes * first / sets / kLz4BlockBytes),
-                         (uint32_t)(voxel_bytes * count / sets / kLz4BlockBytes), sets, set_stride, slot++, st));
+    CKK(k_lz4_decode_run(d_payload, payload_bytes, dec, geo.bytes(), ws, geo.block(first), geo.block(count), geo.sets,
+                         geo.set_blocks(), slot++, st));
     if (planes) return k_bitswap_decode_range(w, reinterpret_cast<const uint16_t*>(dec), d_dst, N, first, count, st) ? 101 : 0;
-    CKK(k_lut_decode(dec + first, d_dst + first, count, d_lut, st));
+    CKK(k_lut_decode(dec + first, d_dst + first, count, small.dec_lut, st));
     return 0;
   });
   if (rc) return rc;
   uint32_t err = 0, none = 0;
   uint64_t total = 0;
   if (k_lz4_decode_status(ws, &err, &total, &none, st)) return 1;
-  if (err || total != lz4_bytes) {
+  if (err || total != geo.bytes()) {
     std::fprintf(stderr, "[sqeazy_b200] lz4 decode failed (code %u)\n", err);
     return planes ? 11 : 101;   // what the general route returns for a broken `lz4` sink / `lz4` tail
   }
@@ -775,13 +853,12 @@ int decode_device_impl(Arena& A, const Header& hdr, const Pipeline& pl, const ui
       } else if (payload_bytes < N) {
         return 11;
       }
-      void* sp = nullptr;
-      if (A.get(kSlotSmall, 4 * 65536 * sizeof(uint32_t) + 4096, &sp)) return 1;
-      uint16_t* d_lut = reinterpret_cast<uint16_t*>(static_cast<uint8_t*>(sp) + 4 * 65536 * sizeof(uint32_t));
-      CK(cudaMemcpyAsync(d_lut, pl.sink.decode_lut, 512, cudaMemcpyHostToDevice, st));
+      SmallSlot small;
+      if (small_slot(A, &small)) return 1;
+      CK(cudaMemcpyAsync(small.dec_lut, pl.sink.decode_lut, 512, cudaMemcpyHostToDevice, st));
       {
         ScopedStageTimer tm(kTLutDec, st);
-        CKK(k_lut_decode(codes, out, N, d_lut, st));
+        CKK(k_lut_decode(codes, out, N, small.dec_lut, st));
       }
       CK(cudaStreamSynchronize(st));
     }
@@ -1218,10 +1295,10 @@ int sqyx_lut_apply_UI16(const void* d_src, void* d_codes, long n, const unsigned
   if (dl.acquire()) return 1;
   Arena* A = &dl.dev->arena;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  void* sp = nullptr;
-  if (A->get(kSlotSmall, 4 * 65536 * sizeof(uint32_t) + 4096, &sp)) return 1;
-  CK(cudaMemcpyAsync(sp, enc_host, 65536, cudaMemcpyHostToDevice, st));
-  CKK(k_lut_apply(static_cast<const uint16_t*>(d_src), static_cast<uint8_t*>(d_codes), (uint64_t)n, static_cast<uint8_t*>(sp), st));
+  SmallSlot small;
+  if (small_slot(*A, &small)) return 1;
+  CK(cudaMemcpyAsync(small.enc_lut, enc_host, 65536, cudaMemcpyHostToDevice, st));
+  CKK(k_lut_apply(static_cast<const uint16_t*>(d_src), static_cast<uint8_t*>(d_codes), (uint64_t)n, small.enc_lut, st));
   CK(cudaStreamSynchronize(st));
   return 0;
 }
@@ -1232,10 +1309,10 @@ int sqyx_lut_decode_UI16(const void* d_codes, void* d_dst, long n, const unsigne
   if (dl.acquire()) return 1;
   Arena* A = &dl.dev->arena;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  void* sp = nullptr;
-  if (A->get(kSlotSmall, 4 * 65536 * sizeof(uint32_t) + 4096, &sp)) return 1;
-  CK(cudaMemcpyAsync(sp, dec_host, 512, cudaMemcpyHostToDevice, st));
-  CKK(k_lut_decode(static_cast<const uint8_t*>(d_codes), static_cast<uint16_t*>(d_dst), (uint64_t)n, static_cast<uint16_t*>(sp), st));
+  SmallSlot small;
+  if (small_slot(*A, &small)) return 1;
+  CK(cudaMemcpyAsync(small.dec_lut, dec_host, 512, cudaMemcpyHostToDevice, st));
+  CKK(k_lut_decode(static_cast<const uint8_t*>(d_codes), static_cast<uint16_t*>(d_dst), (uint64_t)n, small.dec_lut, st));
   CK(cudaStreamSynchronize(st));
   return 0;
 }
@@ -1397,67 +1474,33 @@ int SQY_Pipeline_Max_Compressed_Length_3D_UI8(const char* pipeline, long* shape,
 }
 
 // ---- streamed host paths: the PCIe hop of a large stack overlaps the kernels ----
-// `[remove_background | rmestbkrd ->] bitswapN -> lz4` on uint16 (the headline pipelines): the stack arrives in z-slabs on a
-// copy stream; as soon as a slab is there it is filtered + transposed into its place in the plane-major buffer and the
-// 16 KiB LZ4 blocks it completes in each of the 16/N bit planes are compressed, while the next slab is still on the bus.
+// `[remove_background | rmestbkrd ->] bitswapN -> lz4` on uint16 (the headline pipelines): the stack arrives in 256 MiB z-slabs
+// and each slab is filtered, transposed and LZ4-compressed while the next one is still on the bus (encode_planes_slabs).
 // Only the last slab's kernels, the offset scan and the compaction remain after the last byte has arrived. Decode: the final
 // inverse transpose runs slab by slab and every slab leaves for the host as soon as it is done.
 // returns 0 and the blob size, or an error; the caller has checked that the pipeline is one of these (shard_kind: PlanesLz4),
 // that the stack has at least kStreamMinBytes and that N is a multiple of kStreamGrainVoxels
 int host_encode_streamed(Arena& A, const Pipeline& pl, const char* src, const std::vector<uint64_t>& shape, uint64_t N, char* dst,
                          uint64_t cap, uint64_t* out_bytes, int nthreads) {
-  const uint64_t raw_bytes = 2 * N;
-  cudaStream_t st = nullptr, cs = nullptr;
-  if (copy_stream(&cs)) return 1;
-  void *d_in_v = nullptr, *d_out_v = nullptr, *d_planes_v = nullptr, *ws = nullptr;
-  if (A.get(kSlotIn, raw_bytes, &d_in_v) || A.get(kSlotOut, cap, &d_out_v) || A.get(kSlotA, raw_bytes, &d_planes_v) ||
-      A.get(kSlotWs, k_lz4_encode_workspace_bytes(raw_bytes), &ws))
+  const StreamGeom geo = StreamGeom::planes(N, pl.head.back().w);
+  cudaStream_t st = nullptr;
+  void *d_in = nullptr, *d_out_v = nullptr, *d_planes = nullptr, *ws = nullptr;
+  if (A.get(kSlotIn, 2 * N, &d_in) || A.get(kSlotOut, cap, &d_out_v) || A.get(kSlotA, geo.bytes(), &d_planes) ||
+      A.get(kSlotWs, k_lz4_encode_workspace_bytes(geo.bytes()), &ws))
     return 1;
-  uint16_t* d_in = static_cast<uint16_t*>(d_in_v);
-  uint16_t* d_planes = static_cast<uint16_t*>(d_planes_v);
   uint8_t* d_out = static_cast<uint8_t*>(d_out_v);
   const size_t reserve = header_reserve_bytes(pl, shape);
-  if (cap < reserve || cap - reserve < lz4_payload_bound(raw_bytes)) return 1;
-  uint8_t* payload = d_out + reserve;
-  const Stage& swap = pl.head.back();
-  const int P = 16 / swap.w;
-
-  int thr = pl.head.size() == 2 ? pl.head[0].threshold : 0;
-  // rmestbkrd: the estimate samples the two z faces and six border rows. They are sent on their own (behind the first slab,
-  // which is already on its way: the bus never waits for the estimate) and the threshold is there before the first kernel.
-  auto estimate = [&]() -> int {
+  if (cap < reserve || cap - reserve < lz4_payload_bound(geo.bytes())) return 1;
+  // rmestbkrd: the estimate's two z faces and six border rows are sent on their own behind the first slab, which is already on
+  // its way: the bus never waits for the estimate, and the threshold is there before the first kernel.
+  auto threshold = [&](int* t) -> int {
+    *t = pl.head.size() == 2 ? pl.head[0].threshold : 0;
     if (pl.head.size() != 2 || pl.head[0].kind != StageKind::RmEstBkrd) return 0;
-    const uint64_t Z = shape[0], Y = shape[1], X = shape[2], frame = Y * X;
-    const uint64_t portion = rmest_frame_portion(frame, host_l2_cache_bytes());
-    const uint16_t* h = reinterpret_cast<const uint16_t*>(src);
-    CK(cudaMemcpyAsync(d_in, h, 2 * portion, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(d_in + (Z - 1) * frame, h + (Z - 1) * frame, 2 * portion, cudaMemcpyHostToDevice, st));
-    const uint64_t zs[3] = {1, Z / 2, Z - 2}, ys[2] = {0, Y - 1};
-    for (uint64_t z : zs)
-      for (uint64_t y : ys) CK(cudaMemcpyAsync(d_in + z * frame + y * X, h + z * frame + y * X, 2 * X, cudaMemcpyHostToDevice, st));
-    float sup[4];
-    return estimate_background(A, d_in, Z, Y, X, -1, sup, &thr, st);
+    return estimate_background_host(A, reinterpret_cast<const uint16_t*>(src), shape[0], shape[1], shape[2], t, st);
   };
-
-  CKK(k_lz4_encode_begin(raw_bytes, payload, ws, st));
-  const uint64_t slab_voxels = kStreamSlabBytes / 2;          // a multiple of the grain
-  const uint32_t blocks_per_plane = (uint32_t)(raw_bytes / P / kLz4BlockBytes);
-  EventList events;
-  for (uint64_t first = 0; first < N; first += slab_voxels) {
-    const uint64_t count = std::min(slab_voxels, N - first);
-    CK((cudaError_t)staged_h2d(d_in + first, src + 2 * first, 2 * count, nthreads, cs));
-    cudaEvent_t arrived = nullptr;
-    if (events.next(&arrived)) return 1;
-    CK(cudaEventRecord(arrived, cs));
-    if (first == 0 && estimate()) return 1;
-    CK(cudaStreamWaitEvent(st, arrived, 0));
-    CKK(k_bitswap_encode_range(swap.w, d_in, d_planes, N, first, count, thr, st));
-    // plane piece of this slab: bytes [2*first/P, 2*(first+count)/P) of every plane
-    CKK(k_lz4_encode_blocks(reinterpret_cast<const uint8_t*>(d_planes), raw_bytes, payload, ws,
-                            (uint32_t)(2 * first / P / kLz4BlockBytes), (uint32_t)(2 * count / P / kLz4BlockBytes), (uint32_t)P,
-                            blocks_per_plane, lz4_pitch_hint(pl, shape), st));
-  }
-  CKK(k_lz4_encode_end(reinterpret_cast<const uint8_t*>(d_planes), raw_bytes, payload, ws, st));
+  if (encode_planes_slabs(geo, pl.head.back().w, threshold, lz4_pitch_hint(pl, shape), kStreamSlabBytes / 2, src,
+                          static_cast<uint16_t*>(d_in), static_cast<uint16_t*>(d_planes), d_out + reserve, ws, nthreads, st))
+    return 1;
   uint64_t payload_bytes = 0;
   std::string slot;
   if (lz4_encode_result(A, ws, st, &payload_bytes) || header_slot(pl, shape, payload_bytes, reserve, &slot)) return 1;

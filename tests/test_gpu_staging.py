@@ -53,7 +53,7 @@ def test_staging_uint8(sq, cuda):
                                       "rmbkrd(threshold=104)->bitswap2->lz4", "quantiser->lz4"])
 @pytest.mark.parametrize("kind", ["pageable", "pinned"])
 def test_streamed_host_paths_match_the_device_path(sq, cuda, pipeline, kind):
-    """stacks of >= 512 MiB take the streamed host paths (api.cu: host_encode_streamed, decode_streamed, ship_slabs):
+    """stacks of >= 512 MiB take the streamed host paths (api.cu: host_encode_streamed, take_slabs, decode_streamed, ship_slabs):
     z-slabs are transposed and LZ4-compressed while the next slab is still on the PCIe bus; slabs of the decoded stack leave
     as soon as they are transposed back. 80 frames of 2048x2048 = 640 MiB = 2.5 slabs (ragged last slab). The voxels must be
     the ones the all-at-once device path produces."""

@@ -8,7 +8,7 @@ CSRC      := sqeazy_b200/csrc
 OBJDIR    := build/obj
 LIB       := sqeazy_b200/libsqeazy.so
 
-CU_SRCS   := $(CSRC)/api.cu $(CSRC)/staging.cu $(CSRC)/device/bitswap.cu $(CSRC)/device/bitswap8.cu $(CSRC)/device/bitshuffle.cu $(CSRC)/device/diff.cu $(CSRC)/device/quantise.cu $(CSRC)/device/lz4_encode.cu $(CSRC)/device/lz4_decode.cu
+CU_SRCS   := $(CSRC)/api.cu $(CSRC)/staging.cu $(CSRC)/device/bitswap.cu $(CSRC)/device/bitshuffle.cu $(CSRC)/device/diff.cu $(CSRC)/device/quantise.cu $(CSRC)/device/lz4_encode.cu $(CSRC)/device/lz4_decode.cu
 CPP_SRCS  := $(CSRC)/host/text.cpp $(CSRC)/host/numerics.cpp $(CSRC)/host/pipeline.cpp $(CSRC)/host/h5_filter.cpp
 CU_OBJS   := $(patsubst $(CSRC)/%.cu,$(OBJDIR)/%.o,$(CU_SRCS))
 CPP_OBJS  := $(patsubst $(CSRC)/%.cpp,$(OBJDIR)/%.o,$(CPP_SRCS))

@@ -9,7 +9,6 @@
 
 #include <algorithm>
 #include <atomic>
-#include <climits>
 #include <condition_variable>
 #include <cstdio>
 #include <cstdlib>
@@ -360,82 +359,107 @@ void quantiser_luts(Pipeline& pl, const uint32_t* hist, uint8_t* enc) {
   pl.sink.kv["decode_lut_string"] = std::string(kVerbatimOpen) + base64_encode(dec, sizeof(dec)) + kVerbatimClose;
 }
 
-int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src_any, const std::vector<uint64_t>& shape, uint8_t* d_dst,
+// Where a stage of a device call writes: the last stage that moves data writes the destination, every other one the arena slot
+// (kSlotA / kSlotB) that does not hold its input (kSlotA when the input is in neither).
+struct Scratch {
+  Arena& A;
+  uint64_t bytes;
+  void* slot[2] = {nullptr, nullptr};
+  int next(const void* in, void** out) {
+    const int k = in == slot[0] ? 1 : 0;
+    if (!slot[k] && A.get(k ? kSlotB : kSlotA, bytes, &slot[k])) return 1;
+    *out = slot[k];
+    return 0;
+  }
+};
+
+int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src, const std::vector<uint64_t>& shape, uint8_t* d_dst,
                        uint64_t dst_cap, uint64_t* dst_bytes, const uint32_t* d_global_hist, cudaStream_t st) {
   Pipeline pl = pl_in;
   const uint64_t N = shape_product(shape);
-  const bool u8 = pl.elem == 1;                       // dypeline<uint8_t>: bitswap / remove_background / lz4 / pass_through only
   const uint64_t raw_bytes = (uint64_t)pl.elem * N;
-  const uint16_t* d_src = static_cast<const uint16_t*>(d_src_any);   // (typed per stage below)
-  auto b8 = [](const uint16_t* q) { return reinterpret_cast<const uint8_t*>(q); };
-  auto m8 = [](uint16_t* q) { return reinterpret_cast<uint8_t*>(q); };
   const size_t reserve = header_reserve_bytes(pl, shape);
   uint8_t* payload = d_dst + reserve;
   if (dst_cap < reserve) return 1;
   const uint64_t payload_cap = dst_cap - reserve;
 
-  const uint16_t* cur = d_src;
-  uint16_t* bufs[2] = {nullptr, nullptr};
-  int next = 0;
-  auto next_buf = [&](uint16_t** out) -> int {
-    if (!bufs[next]) {
-      void* p = nullptr;
-      if (A.get(next == 0 ? kSlotA : kSlotB, raw_bytes, &p)) return 1;
-      bufs[next] = static_cast<uint16_t*>(p);
-    }
-    *out = bufs[next];
-    next ^= 1;
-    return 0;
-  };
-
+  Scratch scratch{A, raw_bytes};
+  const void* cur = d_src;
   for (size_t i = 0; i < pl.head.size(); ++i) {
     const Stage& s = pl.head[i];
-    uint16_t* out = nullptr;
     ScopedStageTimer tm(kTFilterSwap, st);
+    int t = s.threshold;
+    if (s.kind == StageKind::RmEstBkrd) {
+      if (shape.size() != 3) {
+        std::fprintf(stderr, "[sqeazy_b200] rmestbkrd needs a rank-3 shape\n");
+        return 1;
+      }
+      float sup[4];
+      if (estimate_background(A, static_cast<const uint16_t*>(cur), shape[0], shape[1], shape[2], -1, sup, &t, st)) return 1;
+    }
+    void* out = nullptr;
+    if (scratch.next(cur, &out)) return 1;
     if (s.kind == StageKind::RemoveBackground || s.kind == StageKind::RmEstBkrd) {
-      int t = s.threshold;
-      if (s.kind == StageKind::RmEstBkrd) {
-        if (shape.size() != 3) {
-          std::fprintf(stderr, "[sqeazy_b200] rmestbkrd needs a rank-3 shape\n");
-          return 1;
-        }
-        float sup[4];
-        if (estimate_background(A, cur, shape[0], shape[1], shape[2], -1, sup, &t, st)) return 1;
-      }
-      if (next_buf(&out)) return 1;
-      if (i + 1 < pl.head.size() && pl.head[i + 1].kind == StageKind::Bitswap && t > 0) {
-        // filter fused into the transpose
-        if (u8) CKK(k_bitswap8_encode(pl.head[i + 1].w, b8(cur), m8(out), N, t, st));
-        else CKK(k_bitswap_encode(pl.head[i + 1].w, cur, out, N, t, st));
-        ++i;
-      } else if (u8) {
-        CKK(k_remove_background8(b8(cur), m8(out), N, t, st));
-      } else {
-        CKK(k_remove_background(cur, out, N, t, st));
-      }
+      if (i + 1 < pl.head.size() && pl.head[i + 1].kind == StageKind::Bitswap && t > 0)   // filter fused into the transpose
+        CKK(k_bitswap_encode(pl.elem, pl.head[++i].w, cur, out, N, t, st));
+      else
+        CKK(k_remove_background(pl.elem, cur, out, N, t, st));
     } else if (s.kind == StageKind::Bitshuffle) {
-      if (next_buf(&out)) return 1;
-      if (u8 ? k_bitshuffle8_encode(b8(cur), m8(out), N, s.block_size, st) : k_bitshuffle16_encode(cur, out, N, s.block_size, st)) {
+      if (k_bitshuffle_encode(pl.elem, cur, out, N, s.block_size, st)) {
         std::fprintf(stderr, "[sqeazy_b200] bitshuffle failed (block_size=%u must be a multiple of 8)\n", s.block_size);
         return 1;
       }
     } else if (s.kind == StageKind::Diff) {
-      if (next_buf(&out)) return 1;
       if (shape.size() != 3 || k_diff_encode(pl.elem, cur, out, shape[0], shape[1], shape[2], st)) {
         // diff_scheme_impl.hpp:84-87 needs rank 3; shapes on which the reference's own loops leave the plane are refused
         std::fprintf(stderr, "[sqeazy_b200] diff3x3x1: shape not supported\n");
         return 1;
       }
-    } else {  // Bitswap
-      if (next_buf(&out)) return 1;
-      if (u8) CKK(k_bitswap8_encode(s.w, b8(cur), m8(out), N, 0, st));
-      else CKK(k_bitswap_encode(s.w, cur, out, N, 0, st));
+    } else {
+      CKK(k_bitswap_encode(pl.elem, s.w, cur, out, N, 0, st));
     }
     cur = out;
   }
 
-  uint64_t payload_bytes = 0;
-  auto lz4_into_payload = [&](const uint8_t* src, uint64_t nbytes) -> int {
+  // the sink's bytes: the head's output, or the quantiser's codes
+  const void* bytes = cur;
+  uint64_t nbytes = raw_bytes;
+  const bool lz4 = pl.has_sink && (pl.sink.kind == StageKind::Lz4 || pl.has_tail);
+  if (pl.has_sink && pl.sink.kind == StageKind::Quantiser) {
+    if (pl.elem != 2) return 1;   // (the planner never builds it for uint8)
+    SmallSlot small;
+    if (small_slot(A, &small)) return 1;
+    std::vector<uint32_t> h(65536);
+    if (N > 0 || d_global_hist) {
+      if (d_global_hist) {
+        CK(cudaMemcpyAsync(h.data(), d_global_hist, 65536 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+      } else {
+        CK(cudaMemsetAsync(small.hist, 0, 65536 * sizeof(uint32_t), st));
+        ScopedStageTimer tm(kTHist, st);
+        CKK(k_histogram_u16(static_cast<const uint16_t*>(cur), N, small.hist, st));
+        tm.stop();
+        CK(cudaMemcpyAsync(h.data(), small.hist, 65536 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+      }
+      CK(cudaStreamSynchronize(st));
+    }
+    std::vector<uint8_t> enc(65536);
+    quantiser_luts(pl, h.data(), enc.data());
+    CK(cudaMemcpyAsync(small.enc_lut, enc.data(), 65536, cudaMemcpyHostToDevice, st));
+    void* codes = payload;   // without an LZ4 tail the codes are the payload
+    if (lz4 && scratch.next(cur, &codes)) return 1;
+    if (!lz4 && payload_cap < N) return 1;
+    {
+      ScopedStageTimer tm(kTLutApply, st);
+      CKK(k_lut_apply(static_cast<const uint16_t*>(cur), static_cast<uint8_t*>(codes), N, small.enc_lut, st));
+    }
+    if (!lz4) CK(cudaStreamSynchronize(st));  // enc (host vector) must outlive the H2D copy; the LZ4 encode waits for it below
+    bytes = codes;
+    nbytes = N;
+  }
+
+  // then LZ4 them (an `lz4` sink or an `lz4` tail), or copy them into the payload
+  uint64_t payload_bytes = nbytes;
+  if (lz4) {
     if (payload_cap < lz4_payload_bound(nbytes)) {
       std::fprintf(stderr, "[sqeazy_b200] destination too small for lz4 (%llu < %llu)\n", (unsigned long long)payload_cap,
                    (unsigned long long)lz4_payload_bound(nbytes));
@@ -445,62 +469,12 @@ int encode_device_impl(Arena& A, const Pipeline& pl_in, const void* d_src_any, c
     if (A.get(kSlotWs, k_lz4_encode_workspace_bytes(nbytes), &ws)) return 1;
     {
       ScopedStageTimer tm(kTLz4Enc, st);
-      CKK(k_lz4_encode(src, nbytes, payload, ws, lz4_pitch_hint(pl, shape), st));
+      CKK(k_lz4_encode(static_cast<const uint8_t*>(bytes), nbytes, payload, ws, lz4_pitch_hint(pl, shape), st));
     }
-    return lz4_encode_result(A, ws, st, &payload_bytes);
-  };
-
-  if (!pl.has_sink) {
-    if (payload_cap < raw_bytes) return 1;
-    if (raw_bytes) CK(cudaMemcpyAsync(payload, cur, raw_bytes, cudaMemcpyDeviceToDevice, st));
-    payload_bytes = raw_bytes;
-  } else if (pl.sink.kind == StageKind::Lz4) {
-    if (lz4_into_payload(reinterpret_cast<const uint8_t*>(cur), raw_bytes)) return 1;
-  } else if (pl.sink.kind == StageKind::PassThrough) {
-    const uint8_t* bytes = reinterpret_cast<const uint8_t*>(cur);
-    if (pl.has_tail) {
-      if (lz4_into_payload(bytes, raw_bytes)) return 1;
-    } else {
-      if (payload_cap < raw_bytes) return 1;
-      if (raw_bytes) CK(cudaMemcpyAsync(payload, bytes, raw_bytes, cudaMemcpyDeviceToDevice, st));
-      payload_bytes = raw_bytes;
-    }
-  } else {  // Quantiser
-    if (u8) return 1;   // (the planner never builds it for uint8)
-    SmallSlot small;
-    if (small_slot(A, &small)) return 1;
-    uint32_t* d_hist = small.hist;
-    std::vector<uint32_t> h(65536);
-    if (N > 0 || d_global_hist) {
-      if (d_global_hist) {
-        CK(cudaMemcpyAsync(h.data(), d_global_hist, 65536 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-      } else {
-        CK(cudaMemsetAsync(d_hist, 0, 65536 * sizeof(uint32_t), st));
-        ScopedStageTimer tm(kTHist, st);
-        CKK(k_histogram_u16(cur, N, d_hist, st));
-        tm.stop();
-        CK(cudaMemcpyAsync(h.data(), d_hist, 65536 * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-      }
-      CK(cudaStreamSynchronize(st));
-    }
-    std::vector<uint8_t> enc(65536);
-    quantiser_luts(pl, h.data(), enc.data());
-    CK(cudaMemcpyAsync(small.enc_lut, enc.data(), 65536, cudaMemcpyHostToDevice, st));
-    if (pl.has_tail) {
-      uint16_t* codes16 = nullptr;
-      if (next_buf(&codes16)) return 1;
-      uint8_t* codes = reinterpret_cast<uint8_t*>(codes16);
-      {
-        ScopedStageTimer tm(kTLutApply, st);
-        CKK(k_lut_apply(cur, codes, N, small.enc_lut, st));
-      }
-      if (lz4_into_payload(codes, N)) return 1;
-    } else {
-      if (payload_cap < N) return 1;
-      CKK(k_lut_apply(cur, payload, N, small.enc_lut, st));
-      CK(cudaStreamSynchronize(st));  // enc (host vector) must outlive the H2D copy
-      payload_bytes = N;
-    }
+    if (lz4_encode_result(A, ws, st, &payload_bytes)) return 1;
+  } else if (bytes != payload) {
+    if (payload_cap < nbytes) return 1;
+    if (nbytes) CK(cudaMemcpyAsync(payload, bytes, nbytes, cudaMemcpyDeviceToDevice, st));
   }
 
   std::string slot;
@@ -757,157 +731,122 @@ int decode_streamed(Arena& A, const Pipeline& pl, const uint8_t* d_payload, uint
 }
 
 int decode_device_impl(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes,
-                       void* d_dst_any, uint64_t dst_cap, cudaStream_t st, HostSink* host = nullptr) {
+                       void* d_dst, uint64_t dst_cap, cudaStream_t st, HostSink* host = nullptr) {
   const uint64_t N = shape_product(hdr.shape);
-  const bool u8 = pl.elem == 1;
   const uint64_t raw_bytes = (uint64_t)pl.elem * N;
-  uint16_t* d_dst = static_cast<uint16_t*>(d_dst_any);
   if (dst_cap < raw_bytes) return 1;
   if (N == 0) return 0;
   if (host) {
-    const int rc = decode_streamed(A, pl, d_payload, payload_bytes, d_dst, N, st, host);
+    const int rc = decode_streamed(A, pl, d_payload, payload_bytes, static_cast<uint16_t*>(d_dst), N, st, host);
     if (rc >= 0) return rc;
   }
 
-  // data-moving head stages in decode order (reverse); the background filters decode as identity
-  std::vector<int> swaps;                 // bitswap: bits per plane; bitshuffle: -1 - block_size; diff3x3x1: kDiffOp
-  constexpr int kDiffOp = INT_MIN;
-  for (size_t i = pl.head.size(); i-- > 0;) {
-    if (pl.head[i].kind == StageKind::Bitswap) swaps.push_back(pl.head[i].w);
-    if (pl.head[i].kind == StageKind::Diff) {
-      if (hdr.shape.size() != 3 || !diff_shape_supported(hdr.shape[0], hdr.shape[1], hdr.shape[2], pl.elem)) return 100 + 1;
-      swaps.push_back(kDiffOp);
-    }
-    if (pl.head[i].kind == StageKind::Bitshuffle) swaps.push_back(-1 - (int)pl.head[i].block_size);
+  // the head stages that move data, decoded from the last one (`top`) down; the background filters decode as identity
+  auto moves = [](const Stage& s) { return s.kind != StageKind::RemoveBackground && s.kind != StageKind::RmEstBkrd; };
+  size_t left = 0;   // data-moving stages still to decode
+  const Stage* top = nullptr;
+  for (const Stage& s : pl.head) {
+    if (!moves(s)) continue;
+    if (s.kind == StageKind::Diff && (hdr.shape.size() != 3 || !diff_shape_supported(hdr.shape[0], hdr.shape[1], hdr.shape[2], pl.elem)))
+      return 100 + 1;
+    ++left;
+    top = &s;
   }
+  Scratch scratch{A, raw_bytes};
+  // the output of a step that reads `in` and behind which `following` data-moving stages still decode
+  auto out_for = [&](const void* in, size_t following, void** out) -> int {
+    if (following == 0) {
+      *out = d_dst;
+      return 0;
+    }
+    return scratch.next(in, out);
+  };
 
   // The transpose back of a uint16 bitswapW that directly follows the LZ4 stage may run inside the LZ4 block decoder when the
   // 16 KiB blocks hold whole groups of the P = 16/W planes (N a multiple of 8192P) and the stack is large enough to gain from it
   // (kFuseMinBytes). A host call that ships the volume slab by slab behind the last transpose keeps that.
-  int fuse_w = 0;
-  if (SQYB_FUSE_TRANSPOSE && !u8 && raw_bytes >= kFuseMinBytes && pl.has_sink && pl.sink.kind == StageKind::Lz4 && !swaps.empty() &&
-      (swaps[0] == 1 || swaps[0] == 2 || swaps[0] == 4 || swaps[0] == 8) && N % (8192ull * (16 / swaps[0])) == 0 &&
-      !(host && swaps.size() == 1 && raw_bytes >= kStreamMinBytes))
-    fuse_w = swaps[0];
+  const bool try_fuse = SQYB_FUSE_TRANSPOSE && pl.elem == 2 && raw_bytes >= kFuseMinBytes && pl.has_sink &&
+                        pl.sink.kind == StageKind::Lz4 && top && top->kind == StageKind::Bitswap &&
+                        N % (8192ull * (16 / top->w)) == 0 && !(host && left == 1 && raw_bytes >= kStreamMinBytes);
 
-  uint16_t* bufs[2] = {nullptr, nullptr};
-  auto scratch = [&](int which, uint16_t** out) -> int {
-    if (!bufs[which]) {
-      void* p = nullptr;
-      if (A.get(which == 0 ? kSlotA : kSlotB, raw_bytes, &p)) return 1;
-      bufs[which] = static_cast<uint16_t*>(p);
-    }
-    *out = bufs[which];
-    return 0;
-  };
-  int toggle = 0;
-  // destination of the op after which `remaining` data-moving ops still follow
-  auto out_for = [&](size_t remaining, uint16_t** out) -> int {
-    if (remaining == 0) { *out = d_dst; return 0; }
-    const int r = scratch(toggle, out);
-    toggle ^= 1;
-    return r;
-  };
-
-  const uint16_t* cur = nullptr;
-  size_t remaining = swaps.size();
-  size_t first_swap = 0;   // 1: the LZ4 decoder did the first transpose back
+  const void* cur = d_payload;   // the head's input
+  size_t end = pl.head.size();   // the head decodes from pl.head[end - 1] down
   if (pl.has_sink) {
-    uint16_t* out = nullptr;
-    if (out_for(remaining, &out)) return 1;
-    if (pl.sink.kind == StageKind::Lz4) {
-      FusedTarget target{fuse_w, nullptr};
-      if (fuse_w && out_for(remaining - 1, &target.vox)) return 1;
-      const bool try_fused = fuse_w && (((uintptr_t)target.vox) & 31) == 0;
+    const bool quantiser = pl.sink.kind == StageKind::Quantiser;
+    void* out = nullptr;         // the sink's output
+    if (out_for(d_payload, left, &out)) return 1;
+    if (quantiser && pl.elem != 2) return 11;
+    if (quantiser && !pl.sink.has_decode_lut) {
+      std::fprintf(stderr, "[sqeazy_b200] quantiser stage without decode_lut_string in the header\n");
+      return 11;
+    }
+    // LZ4 (an `lz4` sink or an `lz4` tail), or the payload as it is
+    const uint64_t nbytes = quantiser ? N : raw_bytes;
+    const void* bytes = d_payload;
+    if (pl.sink.kind == StageKind::Lz4 || pl.has_tail) {
+      void* lz4_out = out;
+      if (quantiser && scratch.next(out, &lz4_out)) return 1;   // codes in the scratch slot that is not the LUT's output
+      void* vox = nullptr;       // where the fused transpose puts the voxels
+      if (try_fuse && out_for(out, left - 1, &vox)) return 1;
+      FusedTarget target{try_fuse ? top->w : 0, static_cast<uint16_t*>(vox)};
       bool fused = false;
-      uint64_t got = 0;
-      if (lz4_decode_checked(A, d_payload, payload_bytes, reinterpret_cast<uint8_t*>(out), raw_bytes, &got, st,
-                             try_fused ? &target : nullptr, &fused))
-        return 11;
+      if (lz4_decode_checked(A, d_payload, payload_bytes, static_cast<uint8_t*>(lz4_out), nbytes, nullptr, st,
+                             try_fuse && (((uintptr_t)target.vox) & 31) == 0 ? &target : nullptr, &fused))
+        return pl.has_tail ? 101 : 11;
+      bytes = lz4_out;
       if (fused) {
         out = target.vox;
-        first_swap = 1;
+        bytes = out;
+        end = size_t(top - pl.head.data());
+        --left;
       }
-    } else if (pl.sink.kind == StageKind::PassThrough) {
-      if (pl.has_tail) {
-        uint64_t got = 0;
-        if (lz4_decode_checked(A, d_payload, payload_bytes, reinterpret_cast<uint8_t*>(out), raw_bytes, &got, st)) return 101;
-      } else {
-        if (payload_bytes < raw_bytes) return 11;
-        CK(cudaMemcpyAsync(out, d_payload, raw_bytes, cudaMemcpyDeviceToDevice, st));
-      }
-    } else {  // Quantiser
-      if (u8) return 11;
-      if (!pl.sink.has_decode_lut) {
-        std::fprintf(stderr, "[sqeazy_b200] quantiser stage without decode_lut_string in the header\n");
-        return 11;
-      }
-      const uint8_t* codes = d_payload;
-      if (pl.has_tail) {
-        uint16_t* cbuf = nullptr;
-        // codes (N bytes) live in the scratch buffer that is NOT the LUT output
-        if (scratch(out == bufs[0] ? 1 : 0, &cbuf)) return 1;
-        uint64_t got = 0;
-        if (lz4_decode_checked(A, d_payload, payload_bytes, reinterpret_cast<uint8_t*>(cbuf), N, &got, st)) return 101;
-        codes = reinterpret_cast<const uint8_t*>(cbuf);
-      } else if (payload_bytes < N) {
-        return 11;
-      }
+    } else if (payload_bytes < nbytes) {
+      return 11;
+    }
+    // then the quantiser's LUT, or the bytes as the head's input
+    if (quantiser) {
       SmallSlot small;
       if (small_slot(A, &small)) return 1;
       CK(cudaMemcpyAsync(small.dec_lut, pl.sink.decode_lut, 512, cudaMemcpyHostToDevice, st));
       {
         ScopedStageTimer tm(kTLutDec, st);
-        CKK(k_lut_decode(codes, out, N, small.dec_lut, st));
+        CKK(k_lut_decode(static_cast<const uint8_t*>(bytes), static_cast<uint16_t*>(out), N, small.dec_lut, st));
       }
       CK(cudaStreamSynchronize(st));
+    } else if (bytes != out) {
+      CK(cudaMemcpyAsync(out, bytes, raw_bytes, cudaMemcpyDeviceToDevice, st));
     }
     cur = out;
   } else {
     if (payload_bytes < raw_bytes) return 1;
-    cur = reinterpret_cast<const uint16_t*>(d_payload);
-    if (remaining == 0) {
-      CK(cudaMemcpyAsync(d_dst, cur, raw_bytes, cudaMemcpyDeviceToDevice, st));
+    if (left == 0) {
+      CK(cudaMemcpyAsync(d_dst, d_payload, raw_bytes, cudaMemcpyDeviceToDevice, st));
       cur = d_dst;
     }
   }
-  for (size_t k = first_swap; k < swaps.size(); ++k) {
-    uint16_t* out = nullptr;
-    remaining = swaps.size() - 1 - k;
-    if (remaining == 0) out = d_dst;
-    else {
-      // pick the scratch buffer that does not hold `cur`
-      if (scratch(cur == bufs[0] ? 1 : 0, &out)) return 1;
-    }
-    if (swaps[k] == kDiffOp) {
+
+  for (size_t i = end; i-- > 0;) {
+    const Stage& s = pl.head[i];
+    if (!moves(s)) continue;
+    void* out = nullptr;
+    if (out_for(cur, --left, &out)) return 1;
+    if (s.kind == StageKind::Diff) {
       if (k_diff_decode(pl.elem, cur, out, hdr.shape[0], hdr.shape[1], hdr.shape[2], st)) return 100 + 1;
-      cur = out;
-      continue;
-    }
-    if (swaps[k] < 0) {
-      const uint32_t bsz = (uint32_t)(-1 - swaps[k]);
-      if (u8 ? k_bitshuffle8_decode(reinterpret_cast<const uint8_t*>(cur), reinterpret_cast<uint8_t*>(out), N, bsz, st)
-             : k_bitshuffle16_decode(cur, out, N, bsz, st))
-        return 100 + 1;
-      cur = out;
-      continue;
-    }
-    if (remaining == 0 && host && !u8 && raw_bytes >= kStreamMinBytes && N % 128 == 0 && !g_timing.load() &&
-        ((((uintptr_t)cur) | ((uintptr_t)out)) & 31) == 0) {
+    } else if (s.kind == StageKind::Bitshuffle) {
+      if (k_bitshuffle_decode(pl.elem, cur, out, N, s.block_size, st)) return 100 + 1;
+    } else if (left == 0 && host && pl.elem == 2 && raw_bytes >= kStreamMinBytes && N % 128 == 0 && !g_timing.load() &&
+               ((((uintptr_t)cur) | ((uintptr_t)out)) & 31) == 0) {
       // last stage of a host call: transpose back slab by slab, every slab leaves for the host as soon as it is done
-      const int rc = ship_slabs(host, out, N, kStreamSlabBytes / 2, st, [&](uint64_t first, uint64_t count) -> int {
-        return k_bitswap_decode_range(swaps[k], cur, out, N, first, count, st) ? 100 + 1 : 0;
+      const uint16_t* in16 = static_cast<const uint16_t*>(cur);
+      uint16_t* out16 = static_cast<uint16_t*>(out);
+      const int rc = ship_slabs(host, out16, N, kStreamSlabBytes / 2, st, [&](uint64_t first, uint64_t count) -> int {
+        return k_bitswap_decode_range(s.w, in16, out16, N, first, count, st) ? 100 + 1 : 0;
       });
       if (rc) return rc;
       host->done = true;
-      cur = out;
-      continue;
-    }
-    {
+    } else {
       ScopedStageTimer tm(kTSwapDec, st);
-      if (u8 ? k_bitswap8_decode(swaps[k], reinterpret_cast<const uint8_t*>(cur), reinterpret_cast<uint8_t*>(out), N, st)
-             : k_bitswap_decode(swaps[k], cur, out, N, st))
-        return 100 + 1;
+      if (k_bitswap_decode(pl.elem, s.w, cur, out, N, st)) return 100 + 1;
     }
     cur = out;
   }
@@ -933,6 +872,42 @@ std::vector<uint64_t> to_shape(const long* shape, unsigned n) {
   std::vector<uint64_t> v;
   for (unsigned i = 0; i < n; ++i) v.push_back(shape[i] < 0 ? 0 : (uint64_t)shape[i]);
   return v;
+}
+
+// what the device entry points do around decode_device_impl: the blob's header, its element size and its pipeline
+int decode_device_blob(Arena& A, int elem, const void* d_blob, long blob_bytes, void* d_dst, long dst_capacity, cudaStream_t st) {
+  if (!d_blob || blob_bytes <= 0 || !d_dst || dst_capacity < 0) return 1;
+  const uint8_t* blob = static_cast<const uint8_t*>(d_blob);
+  Header hdr;
+  if (parse_blob_header_device(blob, (uint64_t)blob_bytes, hdr, st)) return 1;
+  if (sizeof_typename(hdr.raw_type) != (unsigned)elem) return 1;
+  Pipeline pl;
+  if (!(elem == 1 ? build_pipeline_u8(hdr.pipeline, pl) : build_pipeline_u16(hdr.pipeline, pl)) || pl.empty()) {
+    std::fprintf(stderr, "[sqeazy]\t%s cannot be build with this version of sqeazy\n", hdr.pipeline.c_str());
+    return 1;
+  }
+  return decode_device_impl(A, hdr, pl, blob + hdr.size, (uint64_t)blob_bytes - hdr.size, d_dst, (uint64_t)dst_capacity, st);
+}
+
+// ... and around encode_device_impl: the pipeline for the element size, the blob's size
+int encode_device_blob(Arena& A, int elem, const char* pipeline, const void* d_src, const std::vector<uint64_t>& shape, void* d_dst,
+                       long dst_capacity, long* dst_bytes, const void* d_global_hist, cudaStream_t st) {
+  if (!pipeline || !d_dst || !dst_bytes || dst_capacity < 0) return 1;
+  Pipeline pl;
+  if (!(elem == 1 ? build_pipeline_u8(pipeline, pl) : build_pipeline_u16(pipeline, pl)) || pl.empty()) return 1;
+  uint64_t out = 0;
+  const int rc = encode_device_impl(A, pl, d_src, shape, static_cast<uint8_t*>(d_dst), (uint64_t)dst_capacity, &out,
+                                    static_cast<const uint32_t*>(d_global_hist), st);
+  if (rc == 0) *dst_bytes = (long)out;
+  return rc;
+}
+
+// the bitshuffle entry points: one stage, synchronous
+int bitshuffle_device(bool encode, int elem, const void* d_src, void* d_dst, long n, long block_size, void* stream) {
+  if (n < 0 || block_size < 0 || block_size > (1l << 30)) return 1;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if ((encode ? k_bitshuffle_encode : k_bitshuffle_decode)(elem, d_src, d_dst, (uint64_t)n, (uint32_t)block_size, st)) return 1;
+  return cudaStreamSynchronize(st) == cudaSuccess ? 0 : 1;
 }
 
 #include "sharded.inl"
@@ -1024,18 +999,11 @@ int sqyx_release_scratch(void) {
 int sqyx_encode_device_ex_UI16(const char* pipeline, const void* d_src, const long* shape, unsigned shape_size, void* d_dst,
                                long dst_capacity, long* dst_bytes, const void* d_global_hist, void* stream) {
   try {
-    if (!pipeline || !shape || !d_dst || !dst_bytes || dst_capacity < 0) return 1;
-    Pipeline pl;
-    if (!build_pipeline_u16(pipeline, pl) || pl.empty()) return 1;
+    if (!shape) return 1;
     DevLock dl;
     if (dl.acquire()) return 1;
-    Arena* A = &dl.dev->arena;
-    uint64_t out = 0;
-    const int rc = encode_device_impl(*A, pl, static_cast<const uint16_t*>(d_src), to_shape(shape, shape_size),
-                                      static_cast<uint8_t*>(d_dst), (uint64_t)dst_capacity, &out,
-                                      static_cast<const uint32_t*>(d_global_hist), static_cast<cudaStream_t>(stream));
-    if (rc == 0) *dst_bytes = (long)out;
-    return rc;
+    return encode_device_blob(dl.dev->arena, 2, pipeline, d_src, to_shape(shape, shape_size), d_dst, dst_capacity, dst_bytes,
+                              d_global_hist, static_cast<cudaStream_t>(stream));
   } catch (...) {
     return 1;
   }
@@ -1048,21 +1016,9 @@ int sqyx_encode_device_UI16(const char* pipeline, const void* d_src, const long*
 
 int sqyx_decode_device_UI16(const void* d_blob, long blob_bytes, void* d_dst, long dst_capacity, void* stream) {
   try {
-    if (!d_blob || blob_bytes <= 0 || !d_dst || dst_capacity < 0) return 1;
     DevLock dl;
     if (dl.acquire()) return 1;
-    Arena* A = &dl.dev->arena;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    Header hdr;
-    if (parse_blob_header_device(static_cast<const uint8_t*>(d_blob), (uint64_t)blob_bytes, hdr, st)) return 1;
-    if (sizeof_typename(hdr.raw_type) != 2) return 1;
-    Pipeline pl;
-    if (!build_pipeline_u16(hdr.pipeline, pl) || pl.empty()) {
-      std::fprintf(stderr, "[sqeazy]\t%s cannot be build with this version of sqeazy\n", hdr.pipeline.c_str());
-      return 1;
-    }
-    return decode_device_impl(*A, hdr, pl, static_cast<const uint8_t*>(d_blob) + hdr.size, (uint64_t)blob_bytes - hdr.size,
-                              static_cast<uint16_t*>(d_dst), (uint64_t)dst_capacity, st);
+    return decode_device_blob(dl.dev->arena, 2, d_blob, blob_bytes, d_dst, dst_capacity, static_cast<cudaStream_t>(stream));
   } catch (...) {
     return 1;
   }
@@ -1112,51 +1068,27 @@ int sqyx_decode_batch_device_UI16(int n, const void* const* d_blobs, const long*
                                   const long* dst_capacities, int* rcs) {
   if (n > 0 && (!d_blobs || !blob_bytes || !d_dsts || !dst_capacities)) return 1;
   return run_batch(n, rcs, [&](int i, Arena& A, cudaStream_t st) -> int {
-    if (!d_blobs[i] || blob_bytes[i] <= 0 || !d_dsts[i] || dst_capacities[i] < 0) return 1;
-    Header hdr;
-    if (parse_blob_header_device(static_cast<const uint8_t*>(d_blobs[i]), (uint64_t)blob_bytes[i], hdr, st)) return 1;
-    if (sizeof_typename(hdr.raw_type) != 2) return 1;
-    Pipeline pl;
-    if (!build_pipeline_u16(hdr.pipeline, pl) || pl.empty()) return 1;
-    return decode_device_impl(A, hdr, pl, static_cast<const uint8_t*>(d_blobs[i]) + hdr.size, (uint64_t)blob_bytes[i] - hdr.size,
-                              d_dsts[i], (uint64_t)dst_capacities[i], st);
+    return decode_device_blob(A, 2, d_blobs[i], blob_bytes[i], d_dsts[i], dst_capacities[i], st);
   });
 }
 
 int sqyx_encode_batch_device_UI16(int n, const char* pipeline, const void* const* d_srcs, const long* shape, unsigned shape_size,
                                   void* const* d_dsts, const long* dst_capacities, long* dst_bytes, int* rcs) {
-  if (!pipeline || !shape || (n > 0 && (!d_srcs || !d_dsts || !dst_capacities || !dst_bytes))) return 1;
-  Pipeline pl;
-  try {
-    if (!build_pipeline_u16(pipeline, pl) || pl.empty()) return 1;
-  } catch (...) {
-    return 1;
-  }
+  if (!shape || (n > 0 && (!d_srcs || !d_dsts || !dst_capacities || !dst_bytes)) || !SQY_Pipeline_Possible_UI16(pipeline)) return 1;
   const std::vector<uint64_t> shp = to_shape(shape, shape_size);
   return run_batch(n, rcs, [&](int i, Arena& A, cudaStream_t st) -> int {
-    if (!d_dsts[i] || dst_capacities[i] < 0) return 1;
-    uint64_t out = 0;
-    const int rc = encode_device_impl(A, pl, d_srcs[i], shp, static_cast<uint8_t*>(d_dsts[i]), (uint64_t)dst_capacities[i], &out,
-                                      nullptr, st);
-    if (rc == 0) dst_bytes[i] = (long)out;
-    return rc;
+    return encode_device_blob(A, 2, pipeline, d_srcs[i], shp, d_dsts[i], dst_capacities[i], &dst_bytes[i], nullptr, st);
   });
 }
 
 int sqyx_encode_device_UI8(const char* pipeline, const void* d_src, const long* shape, unsigned shape_size, void* d_dst,
                            long dst_capacity, long* dst_bytes, void* stream) {
   try {
-    if (!pipeline || !shape || !d_dst || !dst_bytes || dst_capacity < 0) return 1;
-    Pipeline pl;
-    if (!build_pipeline_u8(pipeline, pl) || pl.empty()) return 1;
+    if (!shape) return 1;
     DevLock dl;
     if (dl.acquire()) return 1;
-    Arena* A = &dl.dev->arena;
-    uint64_t out = 0;
-    const int rc = encode_device_impl(*A, pl, d_src, to_shape(shape, shape_size), static_cast<uint8_t*>(d_dst), (uint64_t)dst_capacity,
-                                      &out, nullptr, static_cast<cudaStream_t>(stream));
-    if (rc == 0) *dst_bytes = (long)out;
-    return rc;
+    return encode_device_blob(dl.dev->arena, 1, pipeline, d_src, to_shape(shape, shape_size), d_dst, dst_capacity, dst_bytes, nullptr,
+                              static_cast<cudaStream_t>(stream));
   } catch (...) {
     return 1;
   }
@@ -1164,21 +1096,9 @@ int sqyx_encode_device_UI8(const char* pipeline, const void* d_src, const long* 
 
 int sqyx_decode_device_UI8(const void* d_blob, long blob_bytes, void* d_dst, long dst_capacity, void* stream) {
   try {
-    if (!d_blob || blob_bytes <= 0 || !d_dst || dst_capacity < 0) return 1;
     DevLock dl;
     if (dl.acquire()) return 1;
-    Arena* A = &dl.dev->arena;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    Header hdr;
-    if (parse_blob_header_device(static_cast<const uint8_t*>(d_blob), (uint64_t)blob_bytes, hdr, st)) return 1;
-    if (sizeof_typename(hdr.raw_type) != 1) return 1;
-    Pipeline pl;
-    if (!build_pipeline_u8(hdr.pipeline, pl) || pl.empty()) {
-      std::fprintf(stderr, "[sqeazy]\t%s cannot be build with this version of sqeazy\n", hdr.pipeline.c_str());
-      return 1;
-    }
-    return decode_device_impl(*A, hdr, pl, static_cast<const uint8_t*>(d_blob) + hdr.size, (uint64_t)blob_bytes - hdr.size, d_dst,
-                              (uint64_t)dst_capacity, st);
+    return decode_device_blob(dl.dev->arena, 1, d_blob, blob_bytes, d_dst, dst_capacity, static_cast<cudaStream_t>(stream));
   } catch (...) {
     return 1;
   }
@@ -1186,44 +1106,28 @@ int sqyx_decode_device_UI8(const void* d_blob, long blob_bytes, void* d_dst, lon
 
 int sqyx_bitswap_encode_UI8(int w, const void* d_src, void* d_dst, long n, int threshold, void* stream) {
   if (n < 0) return 1;
-  return k_bitswap8_encode(w, static_cast<const uint8_t*>(d_src), static_cast<uint8_t*>(d_dst), (uint64_t)n, threshold,
-                           static_cast<cudaStream_t>(stream)) ? 1 : 0;
+  return k_bitswap_encode(1, w, d_src, d_dst, (uint64_t)n, threshold, static_cast<cudaStream_t>(stream)) ? 1 : 0;
 }
 int sqyx_bitswap_decode_UI8(int w, const void* d_src, void* d_dst, long n, void* stream) {
   if (n < 0) return 1;
-  return k_bitswap8_decode(w, static_cast<const uint8_t*>(d_src), static_cast<uint8_t*>(d_dst), (uint64_t)n,
-                           static_cast<cudaStream_t>(stream)) ? 1 : 0;
+  return k_bitswap_decode(1, w, d_src, d_dst, (uint64_t)n, static_cast<cudaStream_t>(stream)) ? 1 : 0;
 }
 int sqyx_remove_background_UI8(const void* d_src, void* d_dst, long n, int threshold, void* stream) {
   if (n < 0) return 1;
-  return k_remove_background8(static_cast<const uint8_t*>(d_src), static_cast<uint8_t*>(d_dst), (uint64_t)n, threshold,
-                              static_cast<cudaStream_t>(stream)) ? 1 : 0;
+  return k_remove_background(1, d_src, d_dst, (uint64_t)n, threshold, static_cast<cudaStream_t>(stream)) ? 1 : 0;
 }
 
 int sqyx_bitshuffle_encode_UI16(const void* d_src, void* d_dst, long n, long block_size, void* stream) {
-  if (n < 0 || block_size < 0 || block_size > (1l << 30)) return 1;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (k_bitshuffle16_encode(static_cast<const uint16_t*>(d_src), static_cast<uint16_t*>(d_dst), (uint64_t)n, (uint32_t)block_size, st)) return 1;
-  return cudaStreamSynchronize(st) == cudaSuccess ? 0 : 1;
+  return bitshuffle_device(true, 2, d_src, d_dst, n, block_size, stream);
 }
 int sqyx_bitshuffle_decode_UI16(const void* d_src, void* d_dst, long n, long block_size, void* stream) {
-  if (n < 0 || block_size < 0 || block_size > (1l << 30)) return 1;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (k_bitshuffle16_decode(static_cast<const uint16_t*>(d_src), static_cast<uint16_t*>(d_dst), (uint64_t)n, (uint32_t)block_size, st)) return 1;
-  return cudaStreamSynchronize(st) == cudaSuccess ? 0 : 1;
+  return bitshuffle_device(false, 2, d_src, d_dst, n, block_size, stream);
 }
-
 int sqyx_bitshuffle_encode_UI8(const void* d_src, void* d_dst, long n, long block_size, void* stream) {
-  if (n < 0 || block_size < 0 || block_size > (1l << 30)) return 1;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (k_bitshuffle8_encode(static_cast<const uint8_t*>(d_src), static_cast<uint8_t*>(d_dst), (uint64_t)n, (uint32_t)block_size, st)) return 1;
-  return cudaStreamSynchronize(st) == cudaSuccess ? 0 : 1;
+  return bitshuffle_device(true, 1, d_src, d_dst, n, block_size, stream);
 }
 int sqyx_bitshuffle_decode_UI8(const void* d_src, void* d_dst, long n, long block_size, void* stream) {
-  if (n < 0 || block_size < 0 || block_size > (1l << 30)) return 1;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (k_bitshuffle8_decode(static_cast<const uint8_t*>(d_src), static_cast<uint8_t*>(d_dst), (uint64_t)n, (uint32_t)block_size, st)) return 1;
-  return cudaStreamSynchronize(st) == cudaSuccess ? 0 : 1;
+  return bitshuffle_device(false, 1, d_src, d_dst, n, block_size, stream);
 }
 
 int sqyx_diff_device(int decode, int sizeof_voxel, const void* d_src, void* d_dst, long z, long y, long x, void* stream) {
@@ -1242,21 +1146,21 @@ int sqyx_diff_shape_supported(int sizeof_voxel, long z, long y, long x) {
 int sqyx_bitswap_encode_UI16(int w, const void* d_src, void* d_dst, long n, int threshold, void* stream) {
   if (n < 0) return 1;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (k_bitswap_encode(w, static_cast<const uint16_t*>(d_src), static_cast<uint16_t*>(d_dst), (uint64_t)n, threshold, st)) return 1;
+  if (k_bitswap_encode(2, w, d_src, d_dst, (uint64_t)n, threshold, st)) return 1;
   return cudaStreamSynchronize(st) == cudaSuccess ? 0 : 1;
 }
 
 int sqyx_bitswap_decode_UI16(int w, const void* d_src, void* d_dst, long n, void* stream) {
   if (n < 0) return 1;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (k_bitswap_decode(w, static_cast<const uint16_t*>(d_src), static_cast<uint16_t*>(d_dst), (uint64_t)n, st)) return 1;
+  if (k_bitswap_decode(2, w, d_src, d_dst, (uint64_t)n, st)) return 1;
   return cudaStreamSynchronize(st) == cudaSuccess ? 0 : 1;
 }
 
 int sqyx_remove_background_UI16(const void* d_src, void* d_dst, long n, int threshold, void* stream) {
   if (n < 0) return 1;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (k_remove_background(static_cast<const uint16_t*>(d_src), static_cast<uint16_t*>(d_dst), (uint64_t)n, threshold, st)) return 1;
+  if (k_remove_background(2, d_src, d_dst, (uint64_t)n, threshold, st)) return 1;
   return cudaStreamSynchronize(st) == cudaSuccess ? 0 : 1;
 }
 

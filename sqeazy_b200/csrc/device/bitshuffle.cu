@@ -1,4 +1,4 @@
-// bitshuffle head filter for uint16 stacks on sm_100a (SURVEY §8f-4).
+// bitshuffle head filter for uint16 and uint8 stacks on sm_100a (SURVEY §8f-4).
 //
 // Replaces bitshuffle_scheme<uint16_t>::encode/decode (encoders/bitshuffle_scheme_impl.hpp:91-160), which hands the buffer
 // to bshuf_bitshuffle / bshuf_bitunshuffle of the third-party bitshuffle library (github.com/kiyo-masui/bitshuffle,
@@ -213,14 +213,6 @@ __global__ void copy_tail8(const uint8_t* __restrict__ in, uint8_t* __restrict__
   if (threadIdx.x < count) out[first + threadIdx.x] = in[first + threadIdx.x];
 }
 
-int grid_for(uint64_t work, int threads) {
-  uint64_t blocks = (work + threads - 1) / threads;
-  const uint64_t cap = (uint64_t)kNumSMs * 32;
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
-  return (int)blocks;
-}
-
 }  // namespace
 
 uint32_t bitshuffle_block_elems(uint32_t block_size, int elem_size) {
@@ -267,13 +259,6 @@ static int run_bitshuffle16(bool encode, const void* in, void* out, uint64_t n, 
   return (int)cudaGetLastError();
 }
 
-int k_bitshuffle16_encode(const uint16_t* in, uint16_t* out, uint64_t n, uint32_t block_size, cudaStream_t st) {
-  return run_bitshuffle16(true, in, out, n, block_size, st);
-}
-int k_bitshuffle16_decode(const uint16_t* in, uint16_t* out, uint64_t n, uint32_t block_size, cudaStream_t st) {
-  return run_bitshuffle16(false, in, out, n, block_size, st);
-}
-
 static int run_bitshuffle8(bool encode, const uint8_t* in, uint8_t* out, uint64_t n, uint32_t block_size, cudaStream_t st) {
   const uint32_t bs = bitshuffle_block_elems(block_size, 1);
   if (bs % 8u) return -81;
@@ -300,11 +285,13 @@ static int run_bitshuffle8(bool encode, const uint8_t* in, uint8_t* out, uint64_
   return (int)cudaGetLastError();
 }
 
-int k_bitshuffle8_encode(const uint8_t* in, uint8_t* out, uint64_t n, uint32_t block_size, cudaStream_t st) {
-  return run_bitshuffle8(true, in, out, n, block_size, st);
+int k_bitshuffle_encode(int elem, const void* in, void* out, uint64_t n, uint32_t block_size, cudaStream_t st) {
+  return elem == 1 ? run_bitshuffle8(true, static_cast<const uint8_t*>(in), static_cast<uint8_t*>(out), n, block_size, st)
+                   : run_bitshuffle16(true, in, out, n, block_size, st);
 }
-int k_bitshuffle8_decode(const uint8_t* in, uint8_t* out, uint64_t n, uint32_t block_size, cudaStream_t st) {
-  return run_bitshuffle8(false, in, out, n, block_size, st);
+int k_bitshuffle_decode(int elem, const void* in, void* out, uint64_t n, uint32_t block_size, cudaStream_t st) {
+  return elem == 1 ? run_bitshuffle8(false, static_cast<const uint8_t*>(in), static_cast<uint8_t*>(out), n, block_size, st)
+                   : run_bitshuffle16(false, in, out, n, block_size, st);
 }
 
 }  // namespace sqyb

@@ -13,6 +13,15 @@ namespace sqyb {
 
 constexpr int kNumSMs = 148;  // B200: 2 dies x 74 SMs; grids are sized in multiples of this
 
+// blocks of `threads` for `work_items` grid-stride items, at most 32 waves of the 148 SMs
+inline int grid_for(uint64_t work_items, int threads) {
+  uint64_t blocks = (work_items + threads - 1) / threads;
+  const uint64_t cap = (uint64_t)kNumSMs * 32;
+  if (blocks > cap) blocks = cap;
+  if (blocks < 1) blocks = 1;
+  return (int)blocks;
+}
+
 // 128-bit streaming load/store: data crosses the SM exactly once, keep it out of L1.
 __device__ __forceinline__ uint4 ld_stream(const uint4* p) {
   uint4 r;

@@ -13,33 +13,28 @@ namespace sqyb {
 extern std::atomic<long> g_kernel_launches;
 #define SQYB_COUNT_LAUNCH(n) ::sqyb::g_kernel_launches.fetch_add((n), std::memory_order_relaxed)
 
-// bitswap.cu
-int k_bitswap_encode(int w, const uint16_t* in, uint16_t* out, uint64_t n, int threshold, cudaStream_t st);
-int k_bitswap_decode(int w, const uint16_t* in, uint16_t* out, uint64_t n, cudaStream_t st);
-int k_remove_background(const uint16_t* in, uint16_t* out, uint64_t n, int threshold, cudaStream_t st);
-// voxels [first, first+count) of an n-voxel volume (in/out = whole-volume base pointers; multiples of 128 voxels): lets the
+// The head stages take elem = bytes per voxel: 1 (uint8 volumes, the *_UI8 entry points) or 2 (uint16).
+// bitswap.cu: w = 1, 2, 4 (uint8) or 1, 2, 4, 8 (uint16); the threshold is taken as a voxel value
+int k_bitswap_encode(int elem, int w, const void* in, void* out, uint64_t n, int threshold, cudaStream_t st);
+int k_bitswap_decode(int elem, int w, const void* in, void* out, uint64_t n, cudaStream_t st);
+int k_remove_background(int elem, const void* in, void* out, uint64_t n, int threshold, cudaStream_t st);
+// uint16 only: voxels [first, first+count) of an n-voxel volume (in/out = whole-volume base pointers; multiples of 128 voxels): lets the
 // host entry points transpose a z-slab as soon as it has arrived / ship a slab as soon as it is transposed back
 int k_bitswap_encode_range(int w, const uint16_t* in, uint16_t* out, uint64_t n, uint64_t first, uint64_t count, int threshold,
                            cudaStream_t st);
 int k_bitswap_decode_range(int w, const uint16_t* in, uint16_t* out, uint64_t n, uint64_t first, uint64_t count, cudaStream_t st);
 
-// bitshuffle.cu: the bitshuffle library's blocked bit transpose for uint16 (encoders/bitshuffle_scheme_impl.hpp:91-160).
-// block_size in elements, 0 = the library's default (4096); -81 (the library's own code) when it is not a multiple of 8
-int k_bitshuffle16_encode(const uint16_t* in, uint16_t* out, uint64_t n, uint32_t block_size, cudaStream_t st);
-int k_bitshuffle16_decode(const uint16_t* in, uint16_t* out, uint64_t n, uint32_t block_size, cudaStream_t st);
-int k_bitshuffle8_encode(const uint8_t* in, uint8_t* out, uint64_t n, uint32_t block_size, cudaStream_t st);   // uint8: default 8192
-int k_bitshuffle8_decode(const uint8_t* in, uint8_t* out, uint64_t n, uint32_t block_size, cudaStream_t st);
+// bitshuffle.cu: the bitshuffle library's blocked bit transpose (encoders/bitshuffle_scheme_impl.hpp:91-160).
+// block_size in elements, 0 = the library's default (4096 for uint16, 8192 for uint8); -81 (the library's own code) when it
+// is not a multiple of 8
+int k_bitshuffle_encode(int elem, const void* in, void* out, uint64_t n, uint32_t block_size, cudaStream_t st);
+int k_bitshuffle_decode(int elem, const void* in, void* out, uint64_t n, uint32_t block_size, cudaStream_t st);
 uint32_t bitshuffle_block_elems(uint32_t block_size, int elem_size);
 
-// diff.cu: diff3x3x1 (encoders/diff_scheme_impl.hpp:78-199), elem = bytes per voxel (1 or 2); in != out; 1 = shape refused
+// diff.cu: diff3x3x1 (encoders/diff_scheme_impl.hpp:78-199); in != out; 1 = shape refused
 bool diff_shape_supported(uint64_t Z, uint64_t Y, uint64_t X, int elem);
 int k_diff_encode(int elem, const void* in, void* out, uint64_t Z, uint64_t Y, uint64_t X, cudaStream_t st);
 int k_diff_decode(int elem, const void* in, void* out, uint64_t Z, uint64_t Y, uint64_t X, cudaStream_t st);
-
-// bitswap8.cu (uint8 volumes)
-int k_bitswap8_encode(int w, const uint8_t* in, uint8_t* out, uint64_t n, int threshold, cudaStream_t st);
-int k_bitswap8_decode(int w, const uint8_t* in, uint8_t* out, uint64_t n, cudaStream_t st);
-int k_remove_background8(const uint8_t* in, uint8_t* out, uint64_t n, int threshold, cudaStream_t st);
 
 // quantise.cu
 int k_histogram_u16(const uint16_t* in, uint64_t n, uint32_t* hist /* 65536 x u32, accumulated into */, cudaStream_t st);

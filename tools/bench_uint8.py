@@ -1,4 +1,4 @@
-"""uint8 path: device times of the bitswap8 / remove_background8 kernels (1 GiB) and of bitswap1->lz4 through sqyx_*_UI8."""
+"""uint8 path: device times of the uint8 bitswap / remove_background kernels (1 GiB) and of bitswap1->lz4 through sqyx_*_UI8."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch

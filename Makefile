@@ -8,7 +8,7 @@ CSRC      := sqeazy_b200/csrc
 OBJDIR    := build/obj
 LIB       := sqeazy_b200/libsqeazy.so
 
-CU_SRCS   := $(CSRC)/api.cu $(CSRC)/staging.cu $(CSRC)/device/bitswap.cu $(CSRC)/device/bitshuffle.cu $(CSRC)/device/diff.cu $(CSRC)/device/quantise.cu $(CSRC)/device/lz4_encode.cu $(CSRC)/device/lz4_decode.cu
+CU_SRCS   := $(CSRC)/api.cu $(CSRC)/staging.cu $(CSRC)/device/bitswap.cu $(CSRC)/device/bitshuffle.cu $(CSRC)/device/diff.cu $(CSRC)/device/quantise.cu $(CSRC)/device/lz4_encode.cu $(CSRC)/device/lz4_decode.cu $(CSRC)/device/roi.cu
 CPP_SRCS  := $(CSRC)/host/text.cpp $(CSRC)/host/numerics.cpp $(CSRC)/host/pipeline.cpp $(CSRC)/host/h5_filter.cpp
 CU_OBJS   := $(patsubst $(CSRC)/%.cu,$(OBJDIR)/%.o,$(CU_SRCS))
 CPP_OBJS  := $(patsubst $(CSRC)/%.cpp,$(OBJDIR)/%.o,$(CPP_SRCS))
@@ -33,7 +33,7 @@ $(LIB): $(CU_OBJS) $(CPP_OBJS)
 	$(NVCC) $(ARCH) -shared -o $@ $^ -cudart static -ldl
 
 # ---- sqy command line tool: a plain C++ client of the C ABI (no CUDA in this translation unit)
-$(SQY): $(CSRC)/cli/sqy.cpp $(CSRC)/cli/tiff_min.hpp include/sqeazy.h $(LIB)
+$(SQY): $(CSRC)/cli/sqy.cpp $(CSRC)/cli/tiff_min.hpp include/sqeazy.h include/sqeazy_b200.h $(LIB)
 	@mkdir -p $(dir $@)
 	$(CXX) -O2 -std=c++17 -Wall -o $@ $(CSRC)/cli/sqy.cpp -Lsqeazy_b200 -lsqeazy -Wl,-rpath,'$$ORIGIN/..'
 

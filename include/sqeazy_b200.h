@@ -32,6 +32,31 @@ int sqyx_encode_device_ex_UI16(const char* pipeline, const void* d_src, const lo
 /* d_blob: [header][payload] in device memory; d_dst: device buffer of dst_capacity bytes (>= raw bytes). */
 int sqyx_decode_device_UI16(const void* d_blob, long blob_bytes, void* d_dst, long dst_capacity, void* stream);
 
+/* ---- sub-volumes: a box of a stack, decoded from the LZ4 blocks that hold it ----
+ * box: 2*ndims longs {lo_0, hi_0, lo_1, hi_1, ...}, half-open, in the order SQY_Decompressed_Shape reports (C order: the last
+ * dimension is contiguous in the stack); ndims must equal the blob's. The box's voxels are written densely in C order:
+ * prod(hi_k - lo_k) * sizeof(voxel) bytes at dst, nothing past them. An empty box (some hi_k == lo_k) returns 0 and writes
+ * nothing. 3 = box malformed or outside the shape (lo_k > hi_k, hi_k > shape_k, ndims mismatch), 1 = dst_capacity too small or
+ * any other failure, 11 / 101 = a broken LZ4 block the box needs (the codes of the whole-stack decode).
+ * Routes: the whole stack is the ordinary decode. Blobs of `[filters ->] bitswapW -> lz4` (uint16) and `quantiser -> lz4` whose
+ * payload is one frame of this library in full 16 KiB blocks (N a multiple of 8192 * 16/W voxels, or of 16384) decode only the
+ * blocks that hold the box; every other blob is decoded whole and cropped. The calls run on the calling thread's device, also
+ * when a device set is configured (sqyx_set_devices). */
+int sqyx_decode_roi_device_UI16(const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst, long dst_capacity,
+                                void* stream);
+int sqyx_decode_roi_device_UI8(const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst, long dst_capacity,
+                               void* stream);
+/* host buffers (the blob and dst in host memory, pageable or pinned; nthreads as for SQY_Decode_UI16). Only the header, the index
+ * frame and the compressed bytes of the blocks the box needs go to the device when the blob takes the indexed route. */
+int sqyx_decode_roi_UI16(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads);
+int sqyx_decode_roi_UI8(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads);
+/* out4 = {route of the most recent ROI call on this thread's device (0 = box is the whole stack: the ordinary decode, 1 = indexed,
+ * 2 = decode whole + crop, -1 = an empty box: nothing decoded), LZ4 blocks decoded by the indexed route (0 on
+ * the others), bytes sent host->device (0 for device calls; the blob's payload on routes 0 and 2), voxels written}.
+ * Route 0 of a host call is SQY_Decode_UI16 / _UI8 itself: like them it may stream the stack slab by slab or shard it over a
+ * configured device set, and its byte count is then the payload the GPUs received together, not one device's share. */
+int sqyx_last_roi_info(long* out4);
+
 /* ---- batches of independent stacks: a time-lapse or a set of stacks (BASELINE cfg4, cfg5; the reference loops over files,
  * src/cpp/src/verbs/compress.hpp:204-338, one stack after the other). Up to 8 stacks are in flight on streams and scratch
  * of their own, so the block decoders / encoders of different stacks share the SMs (a single stack of few large LZ4

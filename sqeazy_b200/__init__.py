@@ -38,6 +38,7 @@ SQYX_SYMBOLS = [
     "sqyx_bitswap_decode_UI8", "sqyx_remove_background_UI8", "sqyx_decode_batch_device_UI16", "sqyx_encode_batch_device_UI16",
     "sqyx_bitshuffle_encode_UI16", "sqyx_bitshuffle_decode_UI16", "sqyx_bitshuffle_encode_UI8", "sqyx_bitshuffle_decode_UI8", "sqyx_set_lz4_defer_min",
     "sqyx_diff_device", "sqyx_diff_shape_supported", "sqyx_set_devices", "sqyx_last_shard_info", "sqyx_nccl_allreduces", "sqyx_lz4_encode_ex",
+    "sqyx_decode_roi_device_UI16", "sqyx_decode_roi_device_UI8", "sqyx_decode_roi_UI16", "sqyx_decode_roi_UI8", "sqyx_last_roi_info",
 ]
 
 # include/sqeazy_h5_filter.h: what HDF5 looks up in a filter plugin
@@ -209,6 +210,47 @@ def decode(blob: np.ndarray, nthreads: int = 1, out: np.ndarray | None = None) -
     return out.reshape(shape) if shape else out
 
 
+def _roi_box(box):
+    """box: (lo, hi) pairs, one per dimension of the stack -> (the C array of 2 * ndims longs, ndims, the box's shape). A box that
+    the library refuses (3) is passed on as it is."""
+    pairs = [(int(lo), int(hi)) for lo, hi in box]
+    arr = (c_long * max(2 * len(pairs), 1))(*[v for p in pairs for v in p])
+    return arr, len(pairs), tuple(max(hi - lo, 0) for lo, hi in pairs)
+
+
+def _decode_roi(fn, name, dtype, blob, box, nthreads, out):
+    blob = np.ascontiguousarray(blob, dtype=np.uint8)
+    arr, nd, shape = _roi_box(box)
+    nbytes = int(np.prod(shape)) * np.dtype(dtype).itemsize
+    if out is None:
+        out = np.empty(shape, dtype=dtype)
+    _check_out(out, dtype, nbytes, name)
+    rc = fn(_vp(blob), c_long(blob.size), arr, c_uint(nd), _vp(out), c_long(out.nbytes), c_int(nthreads))
+    if rc != 0:
+        raise SqeazyError(f"{name} returned {rc}")
+    return out
+
+
+def decode_roi(blob: np.ndarray, box, nthreads: int = 1, out: np.ndarray | None = None) -> np.ndarray:
+    """sqyx_decode_roi_UI16: the box [(lo, hi), ...] (half-open, one pair per dimension of the stack) of a uint16 blob, as an
+    array of the box's shape. Only the blocks that hold the box cross the bus when the blob allows it (last_roi_info)."""
+    return _decode_roi(lib().sqyx_decode_roi_UI16, "sqyx_decode_roi_UI16", np.uint16, blob, box, nthreads, out)
+
+
+def decode_roi_u8(blob: np.ndarray, box, nthreads: int = 1, out: np.ndarray | None = None) -> np.ndarray:
+    """sqyx_decode_roi_UI8: the same for uint8 stacks"""
+    return _decode_roi(lib().sqyx_decode_roi_UI8, "sqyx_decode_roi_UI8", np.uint8, blob, box, nthreads, out)
+
+
+def last_roi_info():
+    """the most recent sub-volume decode on this thread's device: route (0 = the whole stack, 1 = indexed, 2 = decoded whole and
+    cropped, -1 = empty box), LZ4 blocks the indexed route decoded, bytes sent host -> device, voxels written"""
+    o = (c_long * 4)()
+    if lib().sqyx_last_roi_info(o) != 0:
+        raise SqeazyError("sqyx_last_roi_info failed")
+    return {"route": int(o[0]), "blocks": int(o[1]), "h2d_bytes": int(o[2]), "voxels": int(o[3])}
+
+
 # ------------------------------------------------------------------------------------------------
 # sqyx_* : device buffers (torch CUDA tensors). torch is plumbing only: memory, streams, distributed.
 # ------------------------------------------------------------------------------------------------
@@ -279,6 +321,26 @@ def decode_device(blob, out, stream=None):
         raise SqeazyError(f"sqyx_decode_device_UI16 returned {rc}")
     return out
 
+
+def _decode_roi_device(fn, name, blob, box, out, stream):
+    import torch
+    assert blob.is_cuda and out.is_cuda and blob.is_contiguous() and out.is_contiguous()
+    arr, nd, _ = _roi_box(box)
+    with torch.cuda.device(blob.device):
+        rc = fn(_dp(blob), c_long(blob.numel()), arr, c_uint(nd), _dp(out), c_long(out.numel() * out.element_size()), _stream_handle(stream))
+    if rc != 0:
+        raise SqeazyError(f"{name} returned {rc}")
+    return out
+
+
+def decode_roi_device(blob, box, out, stream=None):
+    """sqyx_decode_roi_device_UI16. blob: uint8 CUDA tensor; box: (lo, hi) pairs; out: CUDA tensor with room for the box's
+    voxels, written densely in C order"""
+    return _decode_roi_device(lib().sqyx_decode_roi_device_UI16, "sqyx_decode_roi_device_UI16", blob, box, out, stream)
+
+
+def decode_roi_device_u8(blob, box, out, stream=None):
+    return _decode_roi_device(lib().sqyx_decode_roi_device_UI8, "sqyx_decode_roi_device_UI8", blob, box, out, stream)
 
 
 def decode_batch_device(blobs, outs):

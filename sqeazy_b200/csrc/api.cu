@@ -13,6 +13,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -56,7 +57,7 @@ constexpr int kVersionMajor = 0, kVersionMinor = 7, kVersionPatch = 2;
   } while (0)
 
 // ---- cached device scratch, one arena per device, guarded by one lock (calls are serialised) ----
-enum Slot { kSlotA = 0, kSlotB, kSlotIn, kSlotOut, kSlotWs, kSlotSmall, kSlotOrigins, kNumSlots };
+enum Slot { kSlotA = 0, kSlotB, kSlotIn, kSlotOut, kSlotWs, kSlotSmall, kSlotOrigins, kSlotRoi, kNumSlots };
 
 struct Arena {
   void* ptr[kNumSlots] = {nullptr};
@@ -100,6 +101,7 @@ struct Dev {
   cudaStream_t copy_stream = nullptr;
   Arena batch_arena[kBatchLanes];
   cudaStream_t batch_stream[kBatchLanes] = {};
+  long roi_info[4] = {-1, 0, 0, 0};   // the most recent sub-volume decode on this device (sqyx_last_roi_info)
 };
 Dev g_dev[kMaxDevices];
 std::mutex g_timer_mu;   // g_stage_ms
@@ -490,6 +492,11 @@ constexpr uint64_t kStreamSlabBytes = uint64_t(256) << 20;
 constexpr uint64_t kStreamMinBytes = uint64_t(512) << 20;
 constexpr uint64_t kStreamGrainVoxels = 131072;   // a 16 KiB block of a 1-bit plane covers 131072 voxels (8192 * P for wider atoms)
 
+// blocks [k0, k1) of an LZ4 stream
+struct BlockRun {
+  uint64_t k0, k1;
+};
+
 // The LZ4 stream of n voxels that the host entry points encode and decode slab by slab: `sets` streams of equal length one
 // after the other, in 16 KiB blocks. Voxels [first, first + count) make up blocks [block(first), block(first + count)) of every
 // set when first and count are multiples of the block's voxels in one set.
@@ -504,7 +511,45 @@ struct StreamGeom {
   uint64_t blocks() const { return bytes() / kLz4BlockBytes; }
   uint32_t block(uint64_t v) const { return (uint32_t)(voxel_bytes * v / sets / kLz4BlockBytes); }
   uint32_t set_blocks() const { return block(n); }   // blocks per set: the set stride
+  // the blocks of one set that hold the voxels of `runs` row runs, run(i) = [v0, v1) with v0 < v1, ascending and disjoint: sorted
+  // disjoint block runs, the same in every set (a sub-volume decode needs these blocks of every set and no others)
+  template <class Run>
+  std::vector<BlockRun> blocks_of(uint64_t runs, Run&& run) const {
+    std::vector<BlockRun> out;
+    for (uint64_t i = 0; i < runs; ++i) {
+      const std::pair<uint64_t, uint64_t> r = run(i);
+      const uint64_t k0 = block(r.first), k1 = (uint64_t)block(r.second - 1) + 1;
+      if (!out.empty() && k0 <= out.back().k1) out.back().k1 = std::max(out.back().k1, k1);
+      else out.push_back({k0, k1});
+    }
+    return out;
+  }
 };
+
+// The kinds of blob whose LZ4 blocks each hold a known piece of the stack, on uint16 (the decode of a piece of the stack needs
+// just its blocks):
+//   planes: `[filters ->] bitswapW -> lz4`, N a multiple of the 8192 * 16/W voxels that fill a 16 KiB block of every plane; the
+//           filters decode as identity, so any number of them may stand anywhere in the head;
+//   codes:  `quantiser -> lz4`, N a multiple of 16384.
+// *w = W for planes, 0 for codes. Whether the payload is one frame of this library is for the caller to find out.
+bool indexed_stream(const Pipeline& pl, uint64_t N, StreamGeom* geo, int* w) {
+  if (pl.elem != 2 || !pl.has_sink) return false;
+  if (pl.sink.kind == StageKind::Lz4 && !pl.has_tail) {
+    int nswaps = 0;
+    for (const Stage& s : pl.head) {
+      if (s.kind == StageKind::Bitswap) { *w = s.w; nswaps++; }
+      else if (s.kind == StageKind::Bitshuffle || s.kind == StageKind::Diff) return false;
+    }
+    if (nswaps != 1 || N % (8192ull * (16 / *w))) return false;
+    *geo = StreamGeom::planes(N, *w);
+    return true;
+  }
+  if (pl.sink.kind != StageKind::Quantiser || !pl.has_tail || !pl.head.empty() || !pl.sink.has_decode_lut || N % kLz4BlockBytes)
+    return false;
+  *w = 0;
+  *geo = StreamGeom::codes(N);
+  return true;
+}
 
 int copy_stream(cudaStream_t* cs) {   // of the current device; its lock is held
   int dev = 0;
@@ -681,19 +726,12 @@ int encode_planes_slabs(const StreamGeom& geo, int w, Threshold&& threshold, uin
 // when the blob is not of these kinds (the caller takes the general route), 0 on success, an error code otherwise.
 int decode_streamed(Arena& A, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes, uint16_t* d_dst, uint64_t N,
                     cudaStream_t st, HostSink* host, uint64_t slab_voxels = kStreamSlabBytes / 2, uint64_t min_bytes = kStreamMinBytes) {
-  if (pl.elem != 2 || !pl.has_sink || g_timing.load() || 2 * N < min_bytes) return -1;
-  const bool planes = pl.sink.kind == StageKind::Lz4 && !pl.has_tail;
-  int w = 0, nswaps = 0;
-  if (planes) {
-    for (const Stage& s : pl.head) {
-      if (s.kind == StageKind::Bitswap) { w = s.w; nswaps++; }
-      else if (s.kind == StageKind::Bitshuffle || s.kind == StageKind::Diff) return -1;
-    }
-    if (nswaps != 1 || N % kStreamGrainVoxels) return -1;
-  } else if (pl.sink.kind != StageKind::Quantiser || !pl.has_tail || !pl.head.empty() || !pl.sink.has_decode_lut || N % kLz4BlockBytes) {
-    return -1;
-  }
-  const StreamGeom geo = planes ? StreamGeom::planes(N, w) : StreamGeom::codes(N);
+  if (g_timing.load() || 2 * N < min_bytes) return -1;
+  StreamGeom geo{};
+  int w = 0;
+  if (!indexed_stream(pl, N, &geo, &w)) return -1;
+  const bool planes = w != 0;
+  if (planes && N % kStreamGrainVoxels) return -1;
   void *ws = nullptr, *dec_v = nullptr;
   if (A.get(kSlotWs, k_lz4_decode_workspace_bytes(geo.bytes()), &ws) || A.get(kSlotA, geo.bytes(), &dec_v)) return 1;
   uint8_t* dec = static_cast<uint8_t*>(dec_v);
@@ -911,6 +949,213 @@ int bitshuffle_device(bool encode, int elem, const void* d_src, void* d_dst, lon
 }
 
 #include "sharded.inl"
+
+// ---- sub-volume decode (sqyx_decode_roi_*) ----
+// A box of the stack: its row runs (kernels.h: RoiRuns), its voxels, whether it is the whole stack.
+struct Roi {
+  RoiRuns runs{};
+  uint64_t voxels = 0;
+  bool whole = true;
+};
+
+// box = {lo_0, hi_0, lo_1, hi_1, ...}, half-open, dimension 0 first. 3 when it is malformed or leaves the shape.
+int roi_of(const std::vector<uint64_t>& shape, const long* box, unsigned ndims, Roi* out) {
+  if (!box || ndims == 0 || ndims != shape.size()) return 3;
+  Roi roi;
+  roi.voxels = 1;
+  std::vector<uint64_t> stride(ndims, 1);
+  for (unsigned k = ndims; k-- > 0;) {
+    const long lo = box[2 * k], hi = box[2 * k + 1];
+    if (lo < 0 || lo > hi || (uint64_t)hi > shape[k]) return 3;
+    roi.voxels *= (uint64_t)(hi - lo);
+    roi.whole = roi.whole && lo == 0 && (uint64_t)hi == shape[k];
+    if (k + 1 < ndims) stride[k] = stride[k + 1] * shape[k + 1];
+  }
+  RoiRuns& R = roi.runs;
+  if (roi.voxels) {
+    // the trailing dimensions that the box spans whole go into the runs: one run per index tuple of the dimensions in front of j
+    unsigned j = ndims - 1;
+    while (j > 0 && box[2 * j] == 0 && (uint64_t)box[2 * j + 1] == shape[j]) --j;
+    R.len = (uint64_t)(box[2 * j + 1] - box[2 * j]) * stride[j];
+    R.base = (uint64_t)box[2 * j] * stride[j];
+    R.rows = 1;
+    for (unsigned k = 0; k < j; ++k) {
+      const uint64_t e = (uint64_t)(box[2 * k + 1] - box[2 * k]);
+      R.base += (uint64_t)box[2 * k] * stride[k];
+      if (e == 1) continue;
+      if (R.nlead == kRoiMaxLead) return 1;
+      R.extent[R.nlead] = e;
+      R.stride[R.nlead++] = stride[k];
+      R.rows *= e;
+    }
+  }
+  *out = roi;
+  return 0;
+}
+
+// The blocks of an indexed stream (indexed_stream) that a box needs: `runs` of every set, nsel blocks per set. They are decoded
+// into compact places, set after set: list[t] = the stream's block at compact place t, pos[k] = the place of block k within its
+// set (~0: not needed).
+struct RoiPlan {
+  std::vector<BlockRun> runs;
+  uint64_t nsel = 0;
+  std::vector<uint32_t> list, pos;
+};
+
+RoiPlan roi_plan(const StreamGeom& geo, const RoiRuns& R) {
+  RoiPlan P;
+  P.runs = geo.blocks_of(R.rows, [&](uint64_t r) {
+    const uint64_t v = R.start(r);
+    return std::make_pair(v, v + R.len);
+  });
+  P.pos.assign(geo.set_blocks(), ~0u);
+  for (const BlockRun& b : P.runs)
+    for (uint64_t k = b.k0; k < b.k1; ++k) P.pos[k] = (uint32_t)P.nsel++;
+  P.list.reserve(geo.sets * P.nsel);
+  for (uint32_t j = 0; j < geo.sets; ++j)
+    for (const BlockRun& b : P.runs)
+      for (uint64_t k = b.k0; k < b.k1; ++k) P.list.push_back((uint32_t)((uint64_t)j * geo.set_blocks() + k));
+  return P;
+}
+
+// P's tables on the device (the arena's kSlotRoi): pos, and the list when the caller decodes by list
+int roi_tables(Arena& A, const RoiPlan& P, bool with_list, uint32_t** d_pos, uint32_t** d_list, cudaStream_t st) {
+  void* p = nullptr;
+  if (A.get(kSlotRoi, 4 * (P.pos.size() + P.list.size()), &p)) return 1;
+  *d_pos = static_cast<uint32_t*>(p);
+  *d_list = *d_pos + P.pos.size();
+  CK(cudaMemcpyAsync(*d_pos, P.pos.data(), 4 * P.pos.size(), cudaMemcpyHostToDevice, st));
+  if (with_list) CK(cudaMemcpyAsync(*d_list, P.list.data(), 4 * P.list.size(), cudaMemcpyHostToDevice, st));
+  return 0;
+}
+
+// the gather behind the indexed route, from the compact blocks of P (`ws`: the block decode's workspace), then the block decode's
+// status: 11 (planes) / 101 (codes), what the whole-stack decode returns, when a block that the box needs did not decode
+int roi_finish(Arena& A, const Pipeline& pl, int w, const RoiPlan& P, const uint32_t* d_pos, const RoiRuns& R, const uint8_t* compact,
+               void* ws, uint16_t* d_dst, cudaStream_t st) {
+  if (w) {
+    CKK(k_roi_gather_planes(w, compact, d_pos, P.nsel, R, d_dst, st));
+  } else {
+    SmallSlot small;
+    if (small_slot(A, &small)) return 1;
+    CK(cudaMemcpyAsync(small.dec_lut, pl.sink.decode_lut, 512, cudaMemcpyHostToDevice, st));
+    CKK(k_roi_gather_codes(compact, d_pos, small.dec_lut, R, d_dst, st));
+  }
+  uint32_t err = 0, none = 0;
+  uint64_t total = 0;
+  if (k_lz4_decode_status(ws, &err, &total, &none, st)) return 1;   // (synchronises: P's host tables have been consumed)
+  if (err || total != (uint64_t)P.list.size() * kLz4BlockBytes) {
+    std::fprintf(stderr, "[sqeazy_b200] lz4 decode failed (code %u)\n", err ? err : 5u);
+    return w ? 11 : 101;
+  }
+  return 0;
+}
+
+// A box of a blob in device memory (not empty, not the whole stack) into d_dst. Indexed route (info[0] = 1): the block table of
+// the whole payload, one launch for the blocks the box needs, one gather. Every other blob (info[0] = 2): decoded whole into the
+// arena, then cropped.
+int roi_device(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes, const Roi& roi,
+               void* d_dst, cudaStream_t st, long* info) {
+  const uint64_t N = shape_product(hdr.shape);
+  StreamGeom geo{};
+  int w = 0;
+  if (indexed_stream(pl, N, &geo, &w)) {
+    void* ws = nullptr;
+    if (A.get(kSlotWs, k_lz4_decode_workspace_bytes(geo.bytes()), &ws)) return 1;
+    CKK(k_lz4_decode_tables(d_payload, payload_bytes, geo.bytes(), ws, 0, 0, st));
+    bool own = false;
+    if (k_lz4_decode_own_frame(ws, geo.bytes(), &own, st)) return 1;
+    if (own) {
+      const RoiPlan P = roi_plan(geo, roi.runs);
+      void* compact = nullptr;
+      uint32_t *d_pos = nullptr, *d_list = nullptr;
+      if (A.get(kSlotA, P.list.size() * kLz4BlockBytes, &compact) || roi_tables(A, P, true, &d_pos, &d_list, st)) return 1;
+      info[0] = 1;
+      CKK(k_lz4_decode_list(d_payload, payload_bytes, geo.bytes(), static_cast<uint8_t*>(compact), ws, d_list, (uint32_t)P.list.size(), st));
+      if (int rc = roi_finish(A, pl, w, P, d_pos, roi.runs, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_dst), st))
+        return rc;
+      info[1] = (long)P.list.size();
+      return 0;
+    }
+  }
+  info[0] = 2;
+  void* full = nullptr;
+  if (A.get(kSlotOut, pl.elem * N, &full)) return 1;
+  if (int rc = decode_device_impl(A, hdr, pl, d_payload, payload_bytes, full, pl.elem * N, st)) return rc;
+  CKK(k_roi_crop(pl.elem, full, N, roi.runs, d_dst, st));
+  CK(cudaStreamSynchronize(st));
+  return 0;
+}
+
+// The same for a blob in host memory, into the host buffer dst. Indexed route: the blocks the box needs are cut out of the blob
+// on the host into a frame of their own (index frame, their blocks, EndMark), which alone crosses the bus in one copy and is
+// decoded whole on the device: its blocks land at the compact places of the device route. Otherwise the payload goes to the
+// device as the whole-stack host decode sends it, is decoded whole and cropped. info[2] = the bytes sent to the device.
+int roi_host(Arena& A, const Header& hdr, const Pipeline& pl, const char* src, uint64_t srclength, const Roi& roi, char* dst,
+             int nthreads, long* info) {
+  const uint64_t N = shape_product(hdr.shape), box_bytes = pl.elem * roi.voxels;
+  const uint8_t* payload = reinterpret_cast<const uint8_t*>(src) + hdr.size;
+  const uint64_t payload_bytes = srclength - hdr.size;
+  cudaStream_t st = nullptr;
+  StreamGeom geo{};
+  int w = 0;
+  SqybIndexHeader index;
+  if (indexed_stream(pl, N, &geo, &w) && lz4_read_prefix(payload, payload_bytes, &index) &&
+      index.block_bytes == (uint32_t)kLz4BlockBytes && index.nblocks == geo.blocks() && index.raw_bytes == geo.bytes()) {
+    info[0] = 1;
+    const RoiPlan P = roi_plan(geo, roi.runs);
+    std::vector<BlockRun> runs;   // the needed blocks of every set, in stream order
+    for (uint32_t j = 0; j < geo.sets; ++j)
+      for (const BlockRun& b : P.runs) runs.push_back({(uint64_t)j * geo.set_blocks() + b.k0, (uint64_t)j * geo.set_blocks() + b.k1});
+    const uint8_t* words = payload + kSkippableHeaderBytes + sizeof(SqybIndexHeader);
+    std::vector<uint64_t> off;
+    if (piece_offsets(words, geo.blocks(), runs, off) || kLz4FrameHeaderBytes + off.back() + kLz4EndMarkBytes != index.frame_bytes)
+      return w ? 11 : 101;   // the sizes must add up to the frame
+    const uint64_t nlist = P.list.size(), sub_raw = nlist * kLz4BlockBytes;
+    uint64_t body = 0;
+    for (size_t i = 0; i < runs.size(); ++i) body += off[2 * i + 1] - off[2 * i];
+    const uint64_t prefix = lz4_prefix_bytes(nlist), sub_bytes = prefix + body + kLz4EndMarkBytes;
+    std::unique_ptr<uint8_t[]> sub(new uint8_t[sub_bytes]);   // every byte is written below
+    lz4_write_prefix(sub.get(), (uint32_t)nlist, sub_raw, kLz4FrameHeaderBytes + body + kLz4EndMarkBytes);
+    for (uint64_t t = 0; t < nlist; ++t)
+      std::memcpy(sub.get() + kSkippableHeaderBytes + sizeof(SqybIndexHeader) + 4 * t, words + 4ull * P.list[t], 4);
+    const uint8_t* blocks = payload + lz4_prefix_bytes(geo.blocks());
+    uint64_t q = prefix;
+    for (size_t i = 0; i < runs.size(); ++i) {
+      std::memcpy(sub.get() + q, blocks + off[2 * i], off[2 * i + 1] - off[2 * i]);
+      q += off[2 * i + 1] - off[2 * i];
+    }
+    lz4_put32(sub.get() + q, 0u);   // EndMark
+    void *d_sub = nullptr, *ws = nullptr, *compact = nullptr, *d_box = nullptr;
+    uint32_t *d_pos = nullptr, *d_list = nullptr;
+    if (A.get(kSlotIn, sub_bytes, &d_sub) || A.get(kSlotWs, k_lz4_decode_workspace_bytes(sub_raw), &ws) ||
+        A.get(kSlotA, sub_raw, &compact) || A.get(kSlotOut, box_bytes, &d_box) || roi_tables(A, P, false, &d_pos, &d_list, st))
+      return 1;
+    CK((cudaError_t)staged_h2d(d_sub, sub.get(), sub_bytes, nthreads, st));
+    info[2] = (long)sub_bytes;
+    const uint8_t* d_frame = static_cast<const uint8_t*>(d_sub);
+    CKK(k_lz4_decode_tables(d_frame, sub_bytes, sub_raw, ws, 0, 0, st));
+    CKK(k_lz4_decode_run(d_frame, sub_bytes, static_cast<uint8_t*>(compact), sub_raw, ws, 0, 0, 0, 0, 0, st));
+    if (int rc = roi_finish(A, pl, w, P, d_pos, roi.runs, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_box), st))
+      return rc;
+    info[1] = (long)nlist;
+    CK((cudaError_t)staged_d2h(dst, d_box, box_bytes, nthreads, st));
+    CK(cudaStreamSynchronize(st));
+    return 0;
+  }
+  info[0] = 2;
+  void *d_in = nullptr, *full = nullptr, *d_box = nullptr;
+  // the payload is staged at a 256-byte aligned device address, whatever the header length was
+  if (A.get(kSlotIn, payload_bytes + 256, &d_in) || A.get(kSlotOut, pl.elem * N, &full)) return 1;
+  CK((cudaError_t)staged_h2d(d_in, payload, payload_bytes, nthreads, st));
+  info[2] = (long)payload_bytes;
+  if (int rc = decode_device_impl(A, hdr, pl, static_cast<const uint8_t*>(d_in), payload_bytes, full, pl.elem * N, st)) return rc;
+  if (A.get(kSlotA, box_bytes, &d_box)) return 1;
+  CKK(k_roi_crop(pl.elem, full, N, roi.runs, d_box, st));
+  CK((cudaError_t)staged_d2h(dst, d_box, box_bytes, nthreads, st));
+  CK(cudaStreamSynchronize(st));
+  return 0;
+}
 
 }  // namespace
 
@@ -1536,6 +1781,93 @@ int SQY_PipelineEncode_UI8(const char* pipeline, const char* src, long* shape, u
 }
 int SQY_Decode_UI8(const char* src, long srclength, char* dst, int nthreads) {
   return host_decode(1, src, srclength, dst, nthreads);
+}
+
+// ---- sub-volume decode: the four entry points share the box checks and the whole-stack route ----
+static int decode_roi_device(int elem, const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst,
+                             long dst_capacity, void* stream) {
+  try {
+    if (!d_blob || blob_bytes <= 0 || dst_capacity < 0) return 1;
+    DevLock dl;
+    if (dl.acquire()) return 1;
+    Arena& A = dl.dev->arena;
+    long* info = dl.dev->roi_info;
+    info[0] = -1, info[1] = info[2] = info[3] = 0;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const uint8_t* blob = static_cast<const uint8_t*>(d_blob);
+    Header hdr;
+    if (parse_blob_header_device(blob, (uint64_t)blob_bytes, hdr, st) || sizeof_typename(hdr.raw_type) != (unsigned)elem) return 1;
+    Pipeline pl;
+    if (!(elem == 1 ? build_pipeline_u8(hdr.pipeline, pl) : build_pipeline_u16(hdr.pipeline, pl)) || pl.empty()) return 1;
+    Roi roi;
+    if (int rc = roi_of(hdr.shape, box, ndims, &roi)) return rc;
+    if ((uint64_t)dst_capacity < (uint64_t)elem * roi.voxels || (roi.voxels && !d_dst)) return 1;
+    if (roi.voxels == 0) return 0;
+    int rc = 0;
+    if (roi.whole) {
+      info[0] = 0;
+      rc = decode_device_blob(A, elem, d_blob, blob_bytes, d_dst, dst_capacity, st);
+    } else {
+      rc = roi_device(A, hdr, pl, blob + hdr.size, (uint64_t)blob_bytes - hdr.size, roi, d_dst, st, info);
+    }
+    if (rc == 0) info[3] = (long)roi.voxels;
+    return rc;
+  } catch (...) {
+    return 1;
+  }
+}
+
+static int decode_roi_host(int elem, const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity,
+                           int nthreads) {
+  NvtxRange range(elem == 1 ? "sqyx_decode_roi_UI8" : "sqyx_decode_roi_UI16");
+  try {
+    if (!src || srclength <= 0 || dst_capacity < 0) return 1;
+    const Header hdr = unpack_header(src, (size_t)srclength);
+    if (!hdr.valid || sizeof_typename(hdr.raw_type) != (unsigned)elem) return 1;
+    Pipeline pl;
+    if (!(elem == 1 ? build_pipeline_u8(hdr.pipeline, pl) : build_pipeline_u16(hdr.pipeline, pl)) || pl.empty()) return 1;
+    Roi roi;
+    if (int rc = roi_of(hdr.shape, box, ndims, &roi)) return rc;
+    if ((uint64_t)dst_capacity < (uint64_t)elem * roi.voxels || (roi.voxels && !dst)) return 1;
+    long info[4] = {-1, 0, 0, 0};
+    int rc = 0;
+    if (roi.voxels && roi.whole) {
+      info[0] = 0;
+      info[2] = srclength - (long)hdr.size;
+      rc = host_decode(elem, src, srclength, dst, nthreads);   // takes the device locks it needs itself
+    }
+    DevLock dl;
+    if (dl.acquire()) return 1;
+    if (roi.voxels && !roi.whole) rc = roi_host(dl.dev->arena, hdr, pl, src, (uint64_t)srclength, roi, dst, nthreads, info);
+    if (rc == 0) info[3] = (long)roi.voxels;
+    std::copy(info, info + 4, dl.dev->roi_info);
+    return rc;
+  } catch (...) {
+    return 1;
+  }
+}
+
+int sqyx_decode_roi_device_UI16(const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst, long dst_capacity,
+                                void* stream) {
+  return decode_roi_device(2, d_blob, blob_bytes, box, ndims, d_dst, dst_capacity, stream);
+}
+int sqyx_decode_roi_device_UI8(const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst, long dst_capacity,
+                               void* stream) {
+  return decode_roi_device(1, d_blob, blob_bytes, box, ndims, d_dst, dst_capacity, stream);
+}
+int sqyx_decode_roi_UI16(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads) {
+  return decode_roi_host(2, src, srclength, box, ndims, dst, dst_capacity, nthreads);
+}
+int sqyx_decode_roi_UI8(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads) {
+  return decode_roi_host(1, src, srclength, box, ndims, dst, dst_capacity, nthreads);
+}
+
+int sqyx_last_roi_info(long* out4) {
+  if (!out4) return 1;
+  DevLock dl;
+  if (dl.acquire()) return 1;
+  std::copy(dl.dev->roi_info, dl.dev->roi_info + 4, out4);
+  return 0;
 }
 
 int SQY_h5_query_sizeof(const char*, const char*, unsigned*) { return 1; }

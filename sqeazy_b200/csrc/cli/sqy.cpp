@@ -3,7 +3,7 @@
 // Mirrors the reference's `sqy` tool for the verbs of the volume-pipeline hot path (src/sqy.cpp:182-396,
 // verbs/compress.hpp:225-338, verbs/decompress.hpp:30-233, verbs/bench.hpp:60-131,383-526, verbs/compare.hpp):
 //   compress|enc|encode|comp   <tiff ..>   -p/--pipeline  -o/--output_name  -e/--output_suffix  -n/--nthreads  -v  -h
-//   decompress|dec|decode|rec  <sqy ..>    -o/--output_name  -e/--output_suffix (default .tif)
+//   decompress|dec|decode|rec  <sqy ..>    -o/--output_name  -e/--output_suffix (default .tif)  --roi lo:hi,lo:hi,.. (a box only)
 //   bench|ben                  <tiff ..>   + -c/--as-csv  --noheader  -r/--repetitions  --comment
 //   compare|cmp                <a.tif> <b.tif>     (exit 0 when both stacks hold the same voxels)
 // The reference CLI instantiates the C++ pipeline templates; this one only calls the exported SQY_* functions, i.e. it is
@@ -25,6 +25,7 @@
 #include <vector>
 
 #include "../../../include/sqeazy.h"
+#include "../../../include/sqeazy_b200.h"
 #include "tiff_min.hpp"
 
 namespace {
@@ -48,6 +49,9 @@ const OptSpec kCompress[] = {
     {"dataset_name", 'd', true, "name of the HDF5 dataset (ignored: no HDF5 in this build)"},
     {"output_name", 'o', true, "file location to write output to (if only 1 is given)"},
     {"output_suffix", 'e', true, "file extension to be used (must include period)"},
+};
+const OptSpec kDecompress[] = {
+    {"roi", 0, true, "decompress only the box lo:hi,lo:hi,.. (half-open, one range per dimension, in the order of the shape)"},
 };
 const OptSpec kBench[] = {
     {"as-csv", 'c', false, "print results as comma-separated table"},
@@ -235,8 +239,33 @@ int compress_files(const Options& o) {
   return value;
 }
 
+// "lo:hi,lo:hi,.." -> {lo_0, hi_0, lo_1, hi_1, ..}; false when it is not of that form or a range is empty (lo >= hi): a TIFF
+// has no page of zero extent
+bool parse_roi(const std::string& text, std::vector<long>& box) {
+  box.clear();
+  std::stringstream ss(text);
+  std::string range;
+  while (std::getline(ss, range, ',')) {
+    const size_t colon = range.find(':');
+    if (colon == std::string::npos) return false;
+    char* end = nullptr;
+    const long lo = std::strtol(range.c_str(), &end, 10);
+    if (end != range.c_str() + colon) return false;
+    const long hi = std::strtol(range.c_str() + colon + 1, &end, 10);
+    if (*end != '\0' || colon + 1 == range.size() || lo >= hi) return false;
+    box.push_back(lo);
+    box.push_back(hi);
+  }
+  return !box.empty();
+}
+
 int decompress_files(const Options& o) {
   int value = 1;
+  std::vector<long> box;
+  if (o.has("roi") && !parse_roi(o.get("roi", ""), box)) {
+    std::cerr << "[SQY]\t--roi expects lo:hi,lo:hi,.. (one non-empty range per dimension, lo < hi)\n";
+    return 1;
+  }
   const int nthreads = std::atoi(o.get("nthreads", "1").c_str());
   if (o.files.size() > 1) std::cout << "[SQY]\tmultiple input files detected, ignoring --output_name flag\n";
   std::vector<char> blob, raw;
@@ -256,9 +285,23 @@ int decompress_files(const Options& o) {
     std::vector<long> shape((size_t)nd, 0);
     shape[0] = (long)blob.size();
     if (SQY_Decompressed_Shape(blob.data(), shape.data())) { std::cerr << "[SQY]\t" << file << " has no usable sqy header\n"; continue; }
-    raw.resize((size_t)bytes);
-    const int rc = so == 2 ? SQY_Decode_UI16(blob.data(), (long)blob.size(), raw.data(), nthreads)
-                           : SQY_Decode_UI8(blob.data(), (long)blob.size(), raw.data(), nthreads);
+    int rc = 0;
+    if (o.has("roi")) {
+      // the box alone, in the dimension order of the shape
+      if (box.size() != 2 * shape.size()) { std::cerr << "[SQY]\t" << file << ": --roi needs " << shape.size() << " ranges\n"; continue; }
+      bytes = so;
+      for (size_t k = 0; k < shape.size(); ++k) {
+        shape[k] = std::max(box[2 * k + 1] - box[2 * k], 0l);
+        bytes *= shape[k];
+      }
+      raw.resize((size_t)bytes);
+      rc = so == 2 ? sqyx_decode_roi_UI16(blob.data(), (long)blob.size(), box.data(), (unsigned)shape.size(), raw.data(), bytes, nthreads)
+                   : sqyx_decode_roi_UI8(blob.data(), (long)blob.size(), box.data(), (unsigned)shape.size(), raw.data(), bytes, nthreads);
+    } else {
+      raw.resize((size_t)bytes);
+      rc = so == 2 ? SQY_Decode_UI16(blob.data(), (long)blob.size(), raw.data(), nthreads)
+                   : SQY_Decode_UI8(blob.data(), (long)blob.size(), raw.data(), nthreads);
+    }
     if (rc) { std::cerr << "[SQY]\tdecompressing " << file << " failed! Nothing to write to disk...\n"; continue; }
     const std::string out = target_name(file, o, ".tif");
     const std::string err = sqycli::tiff_write(out, std::vector<uint64_t>(shape.begin(), shape.end()), (int)so * 8, raw.data());
@@ -364,6 +407,7 @@ int main(int argc, char** argv) {
   }
   if (mode == Compress || mode == Bench || mode == Decompress) { tables.push_back(kCompress); sizes.push_back(sizeof(kCompress) / sizeof(OptSpec)); }
   if (mode == Bench) { tables.push_back(kBench); sizes.push_back(sizeof(kBench) / sizeof(OptSpec)); }
+  if (mode == Decompress) { tables.push_back(kDecompress); sizes.push_back(sizeof(kDecompress) / sizeof(OptSpec)); }
   Options o;
   if (!parse(argc, argv, 2, tables, sizes, o)) return 1;
   if (o.has("help")) {

@@ -169,12 +169,11 @@ __device__ __forceinline__ void load_planes(const uint16_t* __restrict__ in, uin
   }
 }
 
-// ... and those words back into the 32 voxels
+// ... and those words back into the 32 voxels, two to a word (voxel 2k in the low half of L[k]) ...
 template <int W>
-__device__ __forceinline__ void store_voxels(uint32_t (&reg)[16], uint16_t* __restrict__ out, uint64_t t) {
+__device__ __forceinline__ void voxels_of(uint32_t (&reg)[16], uint32_t (&L)[16]) {
   constexpr int P = Geo<W>::P;
   transpose_sets<W>(reg);  // the atom transpose is an involution
-  uint32_t L[16];
 #pragma unroll
   for (int k = 0; k < 16; ++k) {
     const int m0 = 2 * k;
@@ -182,6 +181,13 @@ __device__ __forceinline__ void store_voxels(uint32_t (&reg)[16], uint16_t* __re
     const uint32_t sel = (2 * h) | ((2 * h + 1) << 4) | ((4 + 2 * h) << 8) | ((5 + 2 * h) << 12);
     L[k] = __byte_perm(reg[s * P + (P - 1 - j0)], reg[s * P + (P - 2 - j0)], sel);
   }
+}
+
+// ... stored in place
+template <int W>
+__device__ __forceinline__ void store_voxels(uint32_t (&reg)[16], uint16_t* __restrict__ out, uint64_t t) {
+  uint32_t L[16];
+  voxels_of<W>(reg, L);
   st256(out + t * 32, L);
   st256(out + t * 32 + 16, L + 8);
 }

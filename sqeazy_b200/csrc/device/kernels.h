@@ -90,5 +90,38 @@ int k_lz4_decode_linked(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, ui
 // linked blocks from which a stream takes the deferred-reference path (default 8, 0 = never); returns the previous value
 long k_lz4_set_defer_min(long nblocks);
 int k_lz4_decode_status(void* workspace, uint32_t* error, uint64_t* total_decoded, uint32_t* deferred_blocks, cudaStream_t st);
+// the blocks a list names, d_list[0 .. nlist) (indices into the table k_lz4_decode_tables built for stream_bytes decoded bytes; a
+// stream that k_lz4_decode_own_frame found to be one frame of this library): block d_list[t] is decoded into compact + t * 16 KiB.
+// Afterwards the status holds the bytes of the listed blocks that decoded as total_decoded.
+int k_lz4_decode_list(const uint8_t* src, uint64_t src_bytes, uint64_t stream_bytes, uint8_t* compact, void* workspace,
+                      const uint32_t* d_list, uint32_t nlist, cudaStream_t st);
+
+// roi.cu: the voxels of a box of a stack, written densely in C order. The box is `rows` row runs of `len` voxels: run r holds
+// voxels [start(r), start(r) + len) of the stack and lands at dst + r * len; start(r) = base + sum_k i_k * stride[k], where
+// (i_0 .. i_{nlead-1}) is r in mixed radix over extent[] (the last one fastest). Trailing dimensions that the box spans whole
+// are folded into the runs, leading ones of extent 1 into base.
+constexpr int kRoiMaxLead = 8;
+struct RoiRuns {
+  uint64_t base, len, rows;
+  int nlead;
+  uint64_t extent[kRoiMaxLead], stride[kRoiMaxLead];
+  __host__ __device__ uint64_t start(uint64_t r) const {
+    uint64_t v = base;
+    for (int k = nlead - 1; k >= 0; --k) {
+      v += (r % extent[k]) * stride[k];
+      r /= extent[k];
+    }
+    return v;
+  }
+};
+// from the compact 16 KiB blocks of the P = 16/w bit planes of a uint16 bitswap`w` that hold the box: block k of plane segment j
+// (the stream's set j) is compact block j * nsel + pos[k] (pos[k] = ~0: not there, never read)
+int k_roi_gather_planes(int w, const uint8_t* compact, const uint32_t* pos, uint64_t nsel, const RoiRuns& R, uint16_t* dst,
+                        cudaStream_t st);
+// from the compact 16 KiB blocks of 8-bit quantiser codes (block k is compact block pos[k]) through the 256-entry decode LUT
+int k_roi_gather_codes(const uint8_t* compact, const uint32_t* pos, const uint16_t* lut_dev, const RoiRuns& R, uint16_t* dst,
+                       cudaStream_t st);
+// from a whole decoded stack of n voxels of elem bytes (the crop)
+int k_roi_crop(int elem, const void* vol, uint64_t n, const RoiRuns& R, void* dst, cudaStream_t st);
 
 }  // namespace sqyb

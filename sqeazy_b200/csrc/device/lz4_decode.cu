@@ -981,9 +981,10 @@ __global__ void __launch_bounds__(kDirThreads) lz4_offsets_kernel(DecCtl* ctl, D
   }
 }
 
-// fused transpose (lz4_decode_kernel, FW != 0): a range's voxels go back in pieces of kPieceChunks 32-voxel chunks (16384 voxels).
+// fused transpose (lz4_decode_kernel, FW > 0): a range's voxels go back in pieces of kPieceChunks 32-voxel chunks (16384 voxels).
 // The range counter holds the range's decoded blocks in its low half and the pieces claimed so far in its high half.
 constexpr uint32_t kPieceChunks = 512;
+constexpr int kListMode = -1;   // lz4_decode_kernel's FW for the blocks of a list (k_lz4_decode_list)
 
 // transposes the still unclaimed pieces of a complete range (its planes were written by other warps of this launch: fence, then
 // L2 loads). One chunk per lane at a time: a second one in flight costs the 48-register decoder spills.
@@ -1009,13 +1010,16 @@ __device__ __forceinline__ void transpose_range(const uint16_t* planes, uint16_t
 // CTAS = CTAs per SM the registers are budgeted for: 5 (48 registers, 40 warps per SM) for streams that fill the machine,
 // 4 (64 registers, no spills) for small ones, which are bound by the serial chain of their slowest blocks and not by the
 // number of warps in flight (512x512x256 stack: 1.00 -> 0.75 ms; 4 GiB: 5.80 -> 6.25 ms)
-// FW != 0: the stream is one frame of this library holding the 16 KiB blocks of the P = 16/FW bit planes of a uint16 bitswapFW
+// FW > 0: the stream is one frame of this library holding the 16 KiB blocks of the P = 16/FW bit planes of a uint16 bitswapFW
 // (plane-major, bpp blocks per plane), and the kernel also transposes the planes back into `vox`. A range = block r of every
 // plane = voxels [r * 8192P, (r+1) * 8192P). Tickets are dealt range by range; the warp that finishes the last block of a
 // range (per-range counter) transposes it while its planes are still in L2, so the transpose, which needs memory bandwidth,
 // runs beside the decode of other blocks, which needs issue slots, instead of as a launch of its own behind them. Warps that find
 // no block left help with the pieces of the last ranges dealt instead of leaving a range's transpose to one warp at the end.
 // Two instantiations chosen at launch cost nothing; the plain one has no trace of the fused code.
+// FW == kListMode: the blocks named by a list (a sub-volume's blocks, k_lz4_decode_list). Ticket t decodes block T.range[t] of
+// `count` listed ones into dst + t * 16 KiB instead of its place in the stream; far matches read back from that compact place
+// (WinOut::d), and every block adds its decoded bytes to ctl->total_decoded.
 template <int CTAS, int FW>
 __global__ void __launch_bounds__(kWinWarps * 32, CTAS) lz4_decode_kernel(const uint8_t* __restrict__ src, uint64_t src_bytes,
                                                                         uint8_t* __restrict__ dst, DecCtl* ctl, DecTables T,
@@ -1030,15 +1034,16 @@ __global__ void __launch_bounds__(kWinWarps * 32, CTAS) lz4_decode_kernel(const 
   const uint32_t nblocks = ctl->nblocks;
   // count != 0: only `nsets` sets of `count` consecutive blocks, set j starting at first + j * set_stride (the blocks of all
   // bit planes that make up one z-slab), with a work counter of their own
-  const uint32_t total = count ? count * nsets : nblocks;
-  uint32_t* ticket = count ? &ctl->set_ticket[slot & 31u] : &ctl->ticket_decode;
-  constexpr uint32_t P = FW ? 16 / FW : 1;
+  constexpr bool kList = FW == kListMode;
+  const uint32_t total = kList ? count : count ? count * nsets : nblocks;
+  uint32_t* ticket = count && !kList ? &ctl->set_ticket[slot & 31u] : &ctl->ticket_decode;
+  constexpr uint32_t P = FW > 0 ? 16 / FW : 1;
   const uint64_t S = (uint64_t)bpp * (kLz4BlockBytes / 2);   // (fused only) 16-bit words per plane
   while (true) {
     uint32_t b = 0;
     if (lane == 0) b = atomicAdd(ticket, 1u);
     b = __shfl_sync(0xffffffffu, b, 0);
-    if constexpr (FW != 0) {
+    if constexpr (FW > 0) {
       if (b >= total) {
         // every block is held by a running warp: wait for one of the last ranges dealt and take pieces of its transpose
         constexpr uint32_t kPieces = 8192u * P / 32u / kPieceChunks;
@@ -1055,8 +1060,12 @@ __global__ void __launch_bounds__(kWinWarps * 32, CTAS) lz4_decode_kernel(const 
     }
     if (b >= total) return;
     const uint32_t range = b / P;                      // (fused only)
-    if (FW) b = (b % P) * bpp + range;
-    if (count) {
+    if (FW > 0) b = (b % P) * bpp + range;
+    const uint32_t listed = b;                         // (list mode only) the block's compact place
+    if constexpr (kList) {
+      b = T.range[listed];
+      if (b >= nblocks) continue;
+    } else if (count) {
       const uint32_t j = b / count;
       b = first + j * set_stride + (b - j * count);
       if (b >= nblocks) continue;
@@ -1069,7 +1078,7 @@ __global__ void __launch_bounds__(kWinWarps * 32, CTAS) lz4_decode_kernel(const 
     if (link != kNoLink && ctl->deferred) continue;   // block-linked frames: lz4_decode_deferred_kernel + resolve passes
     if (link == kLinkHead) link = kNoLink;
     const uint8_t* s = src + T.src_off[b];
-    uint8_t* d = dst + doff;
+    uint8_t* d = dst + (kList ? (unsigned long long)listed * kLz4BlockBytes : doff);
     bool waited = false;
     uint32_t err = 0;
     // closed-form run block (what the encoder emits for an all-equal block): token 0x1F, byte, offset 1, length
@@ -1113,7 +1122,11 @@ __global__ void __launch_bounds__(kWinWarps * 32, CTAS) lz4_decode_kernel(const 
       if (!err && (O.overflow || got != dsize)) err = kErrSizeMismatch;
     }
     if (err && lane == 0) atomicMax(&ctl->error, err);
-    if constexpr (FW != 0) {
+    if constexpr (kList) {
+      if (!err && lane == 0) atomicAdd(&ctl->total_decoded, (unsigned long long)dsize);
+      continue;
+    }
+    if constexpr (FW > 0) {
       // the planes of a complete range go back to voxels (a broken block sets ctl->error; the range is transposed all the same,
       // inside `vox`, and the caller reports the error)
       __syncwarp();
@@ -1543,6 +1556,22 @@ int k_lz4_decode_run(const uint8_t* src, uint64_t src_bytes, uint8_t* dst, uint6
   else
     lz4_decode_kernel<5, 0><<<kNumSMs * 5, kWinWarps * 32, win_smem, st>>>(src, src_bytes, dst, ctl, T, first, count, nsets, set_stride,
                                                                            slot, nullptr, 0);
+  SQYB_COUNT_LAUNCH(1);
+  return (int)cudaGetLastError();
+}
+
+// the blocks d_list[0 .. nlist) of the table k_lz4_decode_tables left in `workspace` (built for stream_bytes decoded bytes), block
+// d_list[t] into compact + t * 16 KiB;
+// ctl->total_decoded restarts at 0 and counts the bytes of the blocks that decoded. The list rides in the table's `range`
+// array (the fused transpose's counters, unused here). Always the 48-register build: a list is as long as the box is large.
+int k_lz4_decode_list(const uint8_t* src, uint64_t src_bytes, uint64_t stream_bytes, uint8_t* compact, void* workspace,
+                      const uint32_t* d_list, uint32_t nlist, cudaStream_t st) {
+  DecCtl* ctl = reinterpret_cast<DecCtl*>(workspace);
+  DecTables T = dec_tables(workspace, stream_bytes, nullptr);
+  T.range = const_cast<uint32_t*>(d_list);
+  SQYB_CUDA_OK(cudaMemsetAsync(&ctl->total_decoded, 0, sizeof(ctl->total_decoded), st));
+  lz4_decode_kernel<5, kListMode><<<kNumSMs * 5, kWinWarps * 32, kWinWarps * kWinWarpSmem, st>>>(src, src_bytes, compact, ctl, T, 0,
+                                                                                                 nlist, 0, 0, 0, nullptr, 0);
   SQYB_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }

@@ -50,7 +50,20 @@ int sqyx_decode_roi_device_UI8(const void* d_blob, long blob_bytes, const long* 
  * frame and the compressed bytes of the blocks the box needs go to the device when the blob takes the indexed route. */
 int sqyx_decode_roi_UI16(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads);
 int sqyx_decode_roi_UI8(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads);
-/* out4 = {route of the most recent ROI call on this thread's device (0 = box is the whole stack: the ordinary decode, 1 = indexed,
+/* strided slices: slices holds 3*ndims longs {lo_0, hi_0, step_0, lo_1, hi_1, step_1, ...}, half-open, step_k >= 1, in the order
+ * SQY_Decompressed_Shape reports; the slice takes ceil((hi_k - lo_k) / step_k) voxels of dimension k (numpy's lo:hi:step) and
+ * writes them densely in C order, nothing past them. Return codes and routes as for the boxes above, with 3 also for a step < 1;
+ * the indexed route decodes only the blocks that hold a selected voxel. An all-steps-1 slice is the box; a slice of every voxel
+ * is the ordinary decode, a whole range with a step is not. */
+int sqyx_decode_slice_device_UI16(const void* d_blob, long blob_bytes, const long* slices, unsigned ndims, void* d_dst,
+                                  long dst_capacity, void* stream);
+int sqyx_decode_slice_device_UI8(const void* d_blob, long blob_bytes, const long* slices, unsigned ndims, void* d_dst,
+                                 long dst_capacity, void* stream);
+int sqyx_decode_slice_UI16(const char* src, long srclength, const long* slices, unsigned ndims, char* dst, long dst_capacity,
+                           int nthreads);
+int sqyx_decode_slice_UI8(const char* src, long srclength, const long* slices, unsigned ndims, char* dst, long dst_capacity,
+                          int nthreads);
+/* out4 = {route of the most recent ROI or slice call on this thread's device (0 = box is the whole stack: the ordinary decode, 1 = indexed,
  * 2 = decode whole + crop, -1 = an empty box: nothing decoded), LZ4 blocks decoded by the indexed route (0 on
  * the others), bytes sent host->device (0 for device calls; the blob's payload on routes 0 and 2), voxels written}.
  * Route 0 of a host call is SQY_Decode_UI16 / _UI8 itself: like them it may stream the stack slab by slab or shard it over a

@@ -39,6 +39,7 @@ SQYX_SYMBOLS = [
     "sqyx_bitshuffle_encode_UI16", "sqyx_bitshuffle_decode_UI16", "sqyx_bitshuffle_encode_UI8", "sqyx_bitshuffle_decode_UI8", "sqyx_set_lz4_defer_min",
     "sqyx_diff_device", "sqyx_diff_shape_supported", "sqyx_set_devices", "sqyx_last_shard_info", "sqyx_nccl_allreduces", "sqyx_lz4_encode_ex",
     "sqyx_decode_roi_device_UI16", "sqyx_decode_roi_device_UI8", "sqyx_decode_roi_UI16", "sqyx_decode_roi_UI8", "sqyx_last_roi_info",
+    "sqyx_decode_slice_device_UI16", "sqyx_decode_slice_device_UI8", "sqyx_decode_slice_UI16", "sqyx_decode_slice_UI8",
 ]
 
 # include/sqeazy_h5_filter.h: what HDF5 looks up in a filter plugin
@@ -211,16 +212,23 @@ def decode(blob: np.ndarray, nthreads: int = 1, out: np.ndarray | None = None) -
 
 
 def _roi_box(box):
-    """box: (lo, hi) pairs, one per dimension of the stack -> (the C array of 2 * ndims longs, ndims, the box's shape). A box that
-    the library refuses (3) is passed on as it is."""
-    pairs = [(int(lo), int(hi)) for lo, hi in box]
-    arr = (c_long * max(2 * len(pairs), 1))(*[v for p in pairs for v in p])
-    return arr, len(pairs), tuple(max(hi - lo, 0) for lo, hi in pairs)
+    """box: one (lo, hi) pair or (lo, hi, step) triple per dimension of the stack -> (the C array of 2 * ndims longs, or of
+    3 * ndims when any triple is given, ndims, the selection's shape: ceil((hi - lo) / step) per dimension, whether it is
+    strided). A selection that the library refuses (3) is passed on as it is."""
+    tuples = [tuple(int(v) for v in t) for t in box]
+    strided = any(len(t) == 3 for t in tuples)
+    if strided:
+        tuples = [t if len(t) == 3 else (*t, 1) for t in tuples]
+    arr = (c_long * max(sum(len(t) for t in tuples), 1))(*[v for t in tuples for v in t])
+    step = [t[2] if strided else 1 for t in tuples]
+    shape = tuple(max(-(-(t[1] - t[0]) // s), 0) if s > 0 else 0 for t, s in zip(tuples, step))
+    return arr, len(tuples), shape, strided
 
 
-def _decode_roi(fn, name, dtype, blob, box, nthreads, out):
+def _decode_roi(fns, names, dtype, blob, box, nthreads, out):
     blob = np.ascontiguousarray(blob, dtype=np.uint8)
-    arr, nd, shape = _roi_box(box)
+    arr, nd, shape, strided = _roi_box(box)
+    fn, name = fns[strided], names[strided]
     nbytes = int(np.prod(shape)) * np.dtype(dtype).itemsize
     if out is None:
         out = np.empty(shape, dtype=dtype)
@@ -233,13 +241,19 @@ def _decode_roi(fn, name, dtype, blob, box, nthreads, out):
 
 def decode_roi(blob: np.ndarray, box, nthreads: int = 1, out: np.ndarray | None = None) -> np.ndarray:
     """sqyx_decode_roi_UI16: the box [(lo, hi), ...] (half-open, one pair per dimension of the stack) of a uint16 blob, as an
-    array of the box's shape. Only the blocks that hold the box cross the bus when the blob allows it (last_roi_info)."""
-    return _decode_roi(lib().sqyx_decode_roi_UI16, "sqyx_decode_roi_UI16", np.uint16, blob, box, nthreads, out)
+    array of the box's shape. Only the blocks that hold the box cross the bus when the blob allows it (last_roi_info).
+    With any (lo, hi, step) triple among the pairs it is the strided slice lo:hi:step (sqyx_decode_slice_UI16; a pair is step 1),
+    as an array of the slice's shape, ceil((hi - lo) / step) per dimension."""
+    L = lib()
+    return _decode_roi((L.sqyx_decode_roi_UI16, L.sqyx_decode_slice_UI16), ("sqyx_decode_roi_UI16", "sqyx_decode_slice_UI16"),
+                       np.uint16, blob, box, nthreads, out)
 
 
 def decode_roi_u8(blob: np.ndarray, box, nthreads: int = 1, out: np.ndarray | None = None) -> np.ndarray:
-    """sqyx_decode_roi_UI8: the same for uint8 stacks"""
-    return _decode_roi(lib().sqyx_decode_roi_UI8, "sqyx_decode_roi_UI8", np.uint8, blob, box, nthreads, out)
+    """sqyx_decode_roi_UI8 / sqyx_decode_slice_UI8: the same for uint8 stacks"""
+    L = lib()
+    return _decode_roi((L.sqyx_decode_roi_UI8, L.sqyx_decode_slice_UI8), ("sqyx_decode_roi_UI8", "sqyx_decode_slice_UI8"),
+                       np.uint8, blob, box, nthreads, out)
 
 
 def last_roi_info():
@@ -322,10 +336,11 @@ def decode_device(blob, out, stream=None):
     return out
 
 
-def _decode_roi_device(fn, name, blob, box, out, stream):
+def _decode_roi_device(fns, names, blob, box, out, stream):
     import torch
     assert blob.is_cuda and out.is_cuda and blob.is_contiguous() and out.is_contiguous()
-    arr, nd, _ = _roi_box(box)
+    arr, nd, _, strided = _roi_box(box)
+    fn, name = fns[strided], names[strided]
     with torch.cuda.device(blob.device):
         rc = fn(_dp(blob), c_long(blob.numel()), arr, c_uint(nd), _dp(out), c_long(out.numel() * out.element_size()), _stream_handle(stream))
     if rc != 0:
@@ -335,12 +350,17 @@ def _decode_roi_device(fn, name, blob, box, out, stream):
 
 def decode_roi_device(blob, box, out, stream=None):
     """sqyx_decode_roi_device_UI16. blob: uint8 CUDA tensor; box: (lo, hi) pairs; out: CUDA tensor with room for the box's
-    voxels, written densely in C order"""
-    return _decode_roi_device(lib().sqyx_decode_roi_device_UI16, "sqyx_decode_roi_device_UI16", blob, box, out, stream)
+    voxels, written densely in C order. With any (lo, hi, step) triple among the pairs: sqyx_decode_slice_device_UI16, the
+    strided slice's voxels"""
+    L = lib()
+    return _decode_roi_device((L.sqyx_decode_roi_device_UI16, L.sqyx_decode_slice_device_UI16),
+                              ("sqyx_decode_roi_device_UI16", "sqyx_decode_slice_device_UI16"), blob, box, out, stream)
 
 
 def decode_roi_device_u8(blob, box, out, stream=None):
-    return _decode_roi_device(lib().sqyx_decode_roi_device_UI8, "sqyx_decode_roi_device_UI8", blob, box, out, stream)
+    L = lib()
+    return _decode_roi_device((L.sqyx_decode_roi_device_UI8, L.sqyx_decode_slice_device_UI8),
+                              ("sqyx_decode_roi_device_UI8", "sqyx_decode_slice_device_UI8"), blob, box, out, stream)
 
 
 def decode_batch_device(blobs, outs):

@@ -511,16 +511,27 @@ struct StreamGeom {
   uint64_t blocks() const { return bytes() / kLz4BlockBytes; }
   uint32_t block(uint64_t v) const { return (uint32_t)(voxel_bytes * v / sets / kLz4BlockBytes); }
   uint32_t set_blocks() const { return block(n); }   // blocks per set: the set stride
-  // the blocks of one set that hold the voxels of `runs` row runs, run(i) = [v0, v1) with v0 < v1, ascending and disjoint: sorted
-  // disjoint block runs, the same in every set (a sub-volume decode needs these blocks of every set and no others)
-  template <class Run>
-  std::vector<BlockRun> blocks_of(uint64_t runs, Run&& run) const {
+  // the blocks of one set that hold a voxel of the runs R (kernels.h): sorted disjoint block runs, the same in every set (a
+  // sub-volume decode needs these blocks of every set and no others). While a run's step is at most the voxels of one block of
+  // one set, every block from its first voxel's to its last voxel's holds one of its voxels; beyond that each voxel has a block
+  // of its own, and the blocks between them hold nothing the run selects.
+  std::vector<BlockRun> blocks_of(const RoiRuns& R) const {
     std::vector<BlockRun> out;
-    for (uint64_t i = 0; i < runs; ++i) {
-      const std::pair<uint64_t, uint64_t> r = run(i);
-      const uint64_t k0 = block(r.first), k1 = (uint64_t)block(r.second - 1) + 1;
+    const auto add = [&](uint64_t k0, uint64_t k1) {
       if (!out.empty() && k0 <= out.back().k1) out.back().k1 = std::max(out.back().k1, k1);
       else out.push_back({k0, k1});
+    };
+    const uint64_t block_voxels = (uint64_t)kLz4BlockBytes * sets / voxel_bytes;
+    for (uint64_t r = 0; r < R.rows; ++r) {
+      const uint64_t v0 = R.start(r);
+      if (R.step <= block_voxels) {
+        add(block(v0), (uint64_t)block(v0 + (R.len - 1) * R.step) + 1);
+        continue;
+      }
+      for (uint64_t j = 0; j < R.len; ++j) {
+        const uint64_t k = block(v0 + j * R.step);
+        add(k, k + 1);
+      }
     }
     return out;
   }
@@ -950,50 +961,57 @@ int bitshuffle_device(bool encode, int elem, const void* d_src, void* d_dst, lon
 
 #include "sharded.inl"
 
-// ---- sub-volume decode (sqyx_decode_roi_*) ----
-// A box of the stack: its row runs (kernels.h: RoiRuns), its voxels, whether it is the whole stack.
+// ---- sub-volume decode (sqyx_decode_roi_*, sqyx_decode_slice_*) ----
+// A strided slice of the stack (a box when every step is 1): its runs (kernels.h: RoiRuns), its voxels, whether it selects
+// every voxel of the stack.
 struct Roi {
   RoiRuns runs{};
   uint64_t voxels = 0;
   bool whole = true;
 };
 
-// box = {lo_0, hi_0, lo_1, hi_1, ...}, half-open, dimension 0 first. 3 when it is malformed or leaves the shape.
-int roi_of(const std::vector<uint64_t>& shape, const long* box, unsigned ndims, Roi* out) {
-  if (!box || ndims == 0 || ndims != shape.size()) return 3;
+// sel = ndims tuples of `width` longs, dimension 0 first: {lo, hi} (width 2: a box, step 1) or {lo, hi, step} (width 3), half-open,
+// step >= 1; the slice takes ceil((hi - lo) / step) voxels of dimension k. 3 when it is malformed or leaves the shape.
+int roi_of(const std::vector<uint64_t>& shape, const long* sel, unsigned width, unsigned ndims, Roi* out) {
+  if (!sel || ndims == 0 || ndims != shape.size()) return 3;
   Roi roi;
   roi.voxels = 1;
-  std::vector<uint64_t> stride(ndims, 1);
+  std::vector<uint64_t> stride(ndims, 1), lo(ndims), extent(ndims), step(ndims);
   for (unsigned k = ndims; k-- > 0;) {
-    const long lo = box[2 * k], hi = box[2 * k + 1];
-    if (lo < 0 || lo > hi || (uint64_t)hi > shape[k]) return 3;
-    roi.voxels *= (uint64_t)(hi - lo);
-    roi.whole = roi.whole && lo == 0 && (uint64_t)hi == shape[k];
+    const long l = sel[width * k], h = sel[width * k + 1], s = width == 3 ? sel[width * k + 2] : 1;
+    if (l < 0 || l > h || (uint64_t)h > shape[k] || s < 1) return 3;
+    lo[k] = (uint64_t)l, step[k] = (uint64_t)s, extent[k] = ((uint64_t)(h - l) + step[k] - 1) / step[k];
+    roi.voxels *= extent[k];
+    roi.whole = roi.whole && l == 0 && extent[k] == shape[k];
     if (k + 1 < ndims) stride[k] = stride[k + 1] * shape[k + 1];
   }
   RoiRuns& R = roi.runs;
   if (roi.voxels) {
-    // the trailing dimensions that the box spans whole go into the runs: one run per index tuple of the dimensions in front of j
+    // the trailing dimensions that the slice spans whole with step 1 go into the runs: one run per index tuple of the dimensions
+    // in front of j. A step in j is the runs' inner step when j is the last dimension; otherwise j leads too, with its step in
+    // its stride, and a run is the stride[j] voxels of the dimensions behind it.
     unsigned j = ndims - 1;
-    while (j > 0 && box[2 * j] == 0 && (uint64_t)box[2 * j + 1] == shape[j]) --j;
-    R.len = (uint64_t)(box[2 * j + 1] - box[2 * j]) * stride[j];
-    R.base = (uint64_t)box[2 * j] * stride[j];
+    while (j > 0 && lo[j] == 0 && extent[j] == shape[j]) --j;
+    const bool inner = step[j] > 1 && extent[j] > 1;
+    const bool lead_j = inner && j + 1 < ndims;
+    R.len = lead_j ? stride[j] : inner ? extent[j] : extent[j] * stride[j];
+    R.step = inner && !lead_j ? step[j] : 1;
+    R.base = lo[j] * stride[j];
     R.rows = 1;
-    for (unsigned k = 0; k < j; ++k) {
-      const uint64_t e = (uint64_t)(box[2 * k + 1] - box[2 * k]);
-      R.base += (uint64_t)box[2 * k] * stride[k];
-      if (e == 1) continue;
+    for (unsigned k = 0; k < j + (lead_j ? 1 : 0); ++k) {
+      R.base += k < j ? lo[k] * stride[k] : 0;
+      if (extent[k] == 1) continue;
       if (R.nlead == kRoiMaxLead) return 1;
-      R.extent[R.nlead] = e;
-      R.stride[R.nlead++] = stride[k];
-      R.rows *= e;
+      R.extent[R.nlead] = extent[k];
+      R.stride[R.nlead++] = stride[k] * step[k];
+      R.rows *= extent[k];
     }
   }
   *out = roi;
   return 0;
 }
 
-// The blocks of an indexed stream (indexed_stream) that a box needs: `runs` of every set, nsel blocks per set. They are decoded
+// The blocks of an indexed stream (indexed_stream) that hold a voxel of a slice: `runs` of every set, nsel blocks per set. They are decoded
 // into compact places, set after set: list[t] = the stream's block at compact place t, pos[k] = the place of block k within its
 // set (~0: not needed).
 struct RoiPlan {
@@ -1004,10 +1022,7 @@ struct RoiPlan {
 
 RoiPlan roi_plan(const StreamGeom& geo, const RoiRuns& R) {
   RoiPlan P;
-  P.runs = geo.blocks_of(R.rows, [&](uint64_t r) {
-    const uint64_t v = R.start(r);
-    return std::make_pair(v, v + R.len);
-  });
+  P.runs = geo.blocks_of(R);
   P.pos.assign(geo.set_blocks(), ~0u);
   for (const BlockRun& b : P.runs)
     for (uint64_t k = b.k0; k < b.k1; ++k) P.pos[k] = (uint32_t)P.nsel++;
@@ -1030,7 +1045,7 @@ int roi_tables(Arena& A, const RoiPlan& P, bool with_list, uint32_t** d_pos, uin
 }
 
 // the gather behind the indexed route, from the compact blocks of P (`ws`: the block decode's workspace), then the block decode's
-// status: 11 (planes) / 101 (codes), what the whole-stack decode returns, when a block that the box needs did not decode
+// status: 11 (planes) / 101 (codes), what the whole-stack decode returns, when a block that the slice needs did not decode
 int roi_finish(Arena& A, const Pipeline& pl, int w, const RoiPlan& P, const uint32_t* d_pos, const RoiRuns& R, const uint8_t* compact,
                void* ws, uint16_t* d_dst, cudaStream_t st) {
   if (w) {
@@ -1051,8 +1066,8 @@ int roi_finish(Arena& A, const Pipeline& pl, int w, const RoiPlan& P, const uint
   return 0;
 }
 
-// A box of a blob in device memory (not empty, not the whole stack) into d_dst. Indexed route (info[0] = 1): the block table of
-// the whole payload, one launch for the blocks the box needs, one gather. Every other blob (info[0] = 2): decoded whole into the
+// A slice of a blob in device memory (not empty, not the whole stack) into d_dst. Indexed route (info[0] = 1): the block table of
+// the whole payload, one launch for the blocks that hold a selected voxel, one gather. Every other blob (info[0] = 2): decoded whole into the
 // arena, then cropped.
 int roi_device(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes, const Roi& roi,
                void* d_dst, cudaStream_t st, long* info) {
@@ -1087,7 +1102,7 @@ int roi_device(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d
   return 0;
 }
 
-// The same for a blob in host memory, into the host buffer dst. Indexed route: the blocks the box needs are cut out of the blob
+// The same for a blob in host memory, into the host buffer dst. Indexed route: the blocks the slice needs are cut out of the blob
 // on the host into a frame of their own (index frame, their blocks, EndMark), which alone crosses the bus in one copy and is
 // decoded whole on the device: its blocks land at the compact places of the device route. Otherwise the payload goes to the
 // device as the whole-stack host decode sends it, is decoded whole and cropped. info[2] = the bytes sent to the device.
@@ -1783,9 +1798,10 @@ int SQY_Decode_UI8(const char* src, long srclength, char* dst, int nthreads) {
   return host_decode(1, src, srclength, dst, nthreads);
 }
 
-// ---- sub-volume decode: the four entry points share the box checks and the whole-stack route ----
-static int decode_roi_device(int elem, const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst,
-                             long dst_capacity, void* stream) {
+// ---- sub-volume decode: the eight entry points share the planner, the checks and the whole-stack route. sel: ndims tuples of
+// `width` longs, boxes (width 2) or strided slices (width 3); roi_of ----
+static int decode_roi_device(int elem, const void* d_blob, long blob_bytes, const long* sel, unsigned width, unsigned ndims,
+                             void* d_dst, long dst_capacity, void* stream) {
   try {
     if (!d_blob || blob_bytes <= 0 || dst_capacity < 0) return 1;
     DevLock dl;
@@ -1800,7 +1816,7 @@ static int decode_roi_device(int elem, const void* d_blob, long blob_bytes, cons
     Pipeline pl;
     if (!(elem == 1 ? build_pipeline_u8(hdr.pipeline, pl) : build_pipeline_u16(hdr.pipeline, pl)) || pl.empty()) return 1;
     Roi roi;
-    if (int rc = roi_of(hdr.shape, box, ndims, &roi)) return rc;
+    if (int rc = roi_of(hdr.shape, sel, width, ndims, &roi)) return rc;
     if ((uint64_t)dst_capacity < (uint64_t)elem * roi.voxels || (roi.voxels && !d_dst)) return 1;
     if (roi.voxels == 0) return 0;
     int rc = 0;
@@ -1817,9 +1833,10 @@ static int decode_roi_device(int elem, const void* d_blob, long blob_bytes, cons
   }
 }
 
-static int decode_roi_host(int elem, const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity,
-                           int nthreads) {
-  NvtxRange range(elem == 1 ? "sqyx_decode_roi_UI8" : "sqyx_decode_roi_UI16");
+static int decode_roi_host(int elem, const char* src, long srclength, const long* sel, unsigned width, unsigned ndims, char* dst,
+                           long dst_capacity, int nthreads) {
+  NvtxRange range(width == 3 ? (elem == 1 ? "sqyx_decode_slice_UI8" : "sqyx_decode_slice_UI16")
+                             : (elem == 1 ? "sqyx_decode_roi_UI8" : "sqyx_decode_roi_UI16"));
   try {
     if (!src || srclength <= 0 || dst_capacity < 0) return 1;
     const Header hdr = unpack_header(src, (size_t)srclength);
@@ -1827,7 +1844,7 @@ static int decode_roi_host(int elem, const char* src, long srclength, const long
     Pipeline pl;
     if (!(elem == 1 ? build_pipeline_u8(hdr.pipeline, pl) : build_pipeline_u16(hdr.pipeline, pl)) || pl.empty()) return 1;
     Roi roi;
-    if (int rc = roi_of(hdr.shape, box, ndims, &roi)) return rc;
+    if (int rc = roi_of(hdr.shape, sel, width, ndims, &roi)) return rc;
     if ((uint64_t)dst_capacity < (uint64_t)elem * roi.voxels || (roi.voxels && !dst)) return 1;
     long info[4] = {-1, 0, 0, 0};
     int rc = 0;
@@ -1849,17 +1866,33 @@ static int decode_roi_host(int elem, const char* src, long srclength, const long
 
 int sqyx_decode_roi_device_UI16(const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst, long dst_capacity,
                                 void* stream) {
-  return decode_roi_device(2, d_blob, blob_bytes, box, ndims, d_dst, dst_capacity, stream);
+  return decode_roi_device(2, d_blob, blob_bytes, box, 2, ndims, d_dst, dst_capacity, stream);
 }
 int sqyx_decode_roi_device_UI8(const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst, long dst_capacity,
                                void* stream) {
-  return decode_roi_device(1, d_blob, blob_bytes, box, ndims, d_dst, dst_capacity, stream);
+  return decode_roi_device(1, d_blob, blob_bytes, box, 2, ndims, d_dst, dst_capacity, stream);
 }
 int sqyx_decode_roi_UI16(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads) {
-  return decode_roi_host(2, src, srclength, box, ndims, dst, dst_capacity, nthreads);
+  return decode_roi_host(2, src, srclength, box, 2, ndims, dst, dst_capacity, nthreads);
 }
 int sqyx_decode_roi_UI8(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads) {
-  return decode_roi_host(1, src, srclength, box, ndims, dst, dst_capacity, nthreads);
+  return decode_roi_host(1, src, srclength, box, 2, ndims, dst, dst_capacity, nthreads);
+}
+int sqyx_decode_slice_device_UI16(const void* d_blob, long blob_bytes, const long* slices, unsigned ndims, void* d_dst,
+                                  long dst_capacity, void* stream) {
+  return decode_roi_device(2, d_blob, blob_bytes, slices, 3, ndims, d_dst, dst_capacity, stream);
+}
+int sqyx_decode_slice_device_UI8(const void* d_blob, long blob_bytes, const long* slices, unsigned ndims, void* d_dst,
+                                 long dst_capacity, void* stream) {
+  return decode_roi_device(1, d_blob, blob_bytes, slices, 3, ndims, d_dst, dst_capacity, stream);
+}
+int sqyx_decode_slice_UI16(const char* src, long srclength, const long* slices, unsigned ndims, char* dst, long dst_capacity,
+                           int nthreads) {
+  return decode_roi_host(2, src, srclength, slices, 3, ndims, dst, dst_capacity, nthreads);
+}
+int sqyx_decode_slice_UI8(const char* src, long srclength, const long* slices, unsigned ndims, char* dst, long dst_capacity,
+                          int nthreads) {
+  return decode_roi_host(1, src, srclength, slices, 3, ndims, dst, dst_capacity, nthreads);
 }
 
 int sqyx_last_roi_info(long* out4) {

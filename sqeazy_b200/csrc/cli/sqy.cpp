@@ -3,7 +3,7 @@
 // Mirrors the reference's `sqy` tool for the verbs of the volume-pipeline hot path (src/sqy.cpp:182-396,
 // verbs/compress.hpp:225-338, verbs/decompress.hpp:30-233, verbs/bench.hpp:60-131,383-526, verbs/compare.hpp):
 //   compress|enc|encode|comp   <tiff ..>   -p/--pipeline  -o/--output_name  -e/--output_suffix  -n/--nthreads  -v  -h
-//   decompress|dec|decode|rec  <sqy ..>    -o/--output_name  -e/--output_suffix (default .tif)  --roi lo:hi,lo:hi,.. (a box only)
+//   decompress|dec|decode|rec  <sqy ..>    -o/--output_name  -e/--output_suffix (default .tif)  --roi lo:hi[:step],.. (a box or strided slice only)
 //   bench|ben                  <tiff ..>   + -c/--as-csv  --noheader  -r/--repetitions  --comment
 //   compare|cmp                <a.tif> <b.tif>     (exit 0 when both stacks hold the same voxels)
 // The reference CLI instantiates the C++ pipeline templates; this one only calls the exported SQY_* functions, i.e. it is
@@ -51,7 +51,7 @@ const OptSpec kCompress[] = {
     {"output_suffix", 'e', true, "file extension to be used (must include period)"},
 };
 const OptSpec kDecompress[] = {
-    {"roi", 0, true, "decompress only the box lo:hi,lo:hi,.. (half-open, one range per dimension, in the order of the shape)"},
+    {"roi", 0, true, "decompress only the slice lo:hi[:step],lo:hi[:step],.. (half-open, step >= 1, one range per dimension, in the order of the shape)"},
 };
 const OptSpec kBench[] = {
     {"as-csv", 'c', false, "print results as comma-separated table"},
@@ -239,10 +239,10 @@ int compress_files(const Options& o) {
   return value;
 }
 
-// "lo:hi,lo:hi,.." -> {lo_0, hi_0, lo_1, hi_1, ..}; false when it is not of that form or a range is empty (lo >= hi): a TIFF
-// has no page of zero extent
-bool parse_roi(const std::string& text, std::vector<long>& box) {
-  box.clear();
+// "lo:hi[:step],.." -> {lo_0, hi_0, step_0, lo_1, ..} (step 1 when it is left out); false when it is not of that form, a range
+// is empty (lo >= hi: a TIFF has no page of zero extent) or a step is less than 1
+bool parse_roi(const std::string& text, std::vector<long>& slices) {
+  slices.clear();
   std::stringstream ss(text);
   std::string range;
   while (std::getline(ss, range, ',')) {
@@ -251,19 +251,26 @@ bool parse_roi(const std::string& text, std::vector<long>& box) {
     char* end = nullptr;
     const long lo = std::strtol(range.c_str(), &end, 10);
     if (end != range.c_str() + colon) return false;
-    const long hi = std::strtol(range.c_str() + colon + 1, &end, 10);
-    if (*end != '\0' || colon + 1 == range.size() || lo >= hi) return false;
-    box.push_back(lo);
-    box.push_back(hi);
+    const char* hi_text = range.c_str() + colon + 1;
+    const long hi = std::strtol(hi_text, &end, 10);
+    if (end == hi_text || lo >= hi) return false;
+    long step = 1;
+    if (*end == ':') {
+      const char* step_text = end + 1;
+      step = std::strtol(step_text, &end, 10);
+      if (end == step_text || step < 1) return false;
+    }
+    if (*end != '\0') return false;
+    slices.insert(slices.end(), {lo, hi, step});
   }
-  return !box.empty();
+  return !slices.empty();
 }
 
 int decompress_files(const Options& o) {
   int value = 1;
-  std::vector<long> box;
-  if (o.has("roi") && !parse_roi(o.get("roi", ""), box)) {
-    std::cerr << "[SQY]\t--roi expects lo:hi,lo:hi,.. (one non-empty range per dimension, lo < hi)\n";
+  std::vector<long> slices;
+  if (o.has("roi") && !parse_roi(o.get("roi", ""), slices)) {
+    std::cerr << "[SQY]\t--roi expects lo:hi[:step],.. (one non-empty range per dimension, lo < hi, step >= 1)\n";
     return 1;
   }
   const int nthreads = std::atoi(o.get("nthreads", "1").c_str());
@@ -287,16 +294,16 @@ int decompress_files(const Options& o) {
     if (SQY_Decompressed_Shape(blob.data(), shape.data())) { std::cerr << "[SQY]\t" << file << " has no usable sqy header\n"; continue; }
     int rc = 0;
     if (o.has("roi")) {
-      // the box alone, in the dimension order of the shape
-      if (box.size() != 2 * shape.size()) { std::cerr << "[SQY]\t" << file << ": --roi needs " << shape.size() << " ranges\n"; continue; }
+      // the slice alone, in the dimension order of the shape
+      if (slices.size() != 3 * shape.size()) { std::cerr << "[SQY]\t" << file << ": --roi needs " << shape.size() << " ranges\n"; continue; }
       bytes = so;
       for (size_t k = 0; k < shape.size(); ++k) {
-        shape[k] = std::max(box[2 * k + 1] - box[2 * k], 0l);
+        shape[k] = std::max((slices[3 * k + 1] - slices[3 * k] + slices[3 * k + 2] - 1) / slices[3 * k + 2], 0l);
         bytes *= shape[k];
       }
       raw.resize((size_t)bytes);
-      rc = so == 2 ? sqyx_decode_roi_UI16(blob.data(), (long)blob.size(), box.data(), (unsigned)shape.size(), raw.data(), bytes, nthreads)
-                   : sqyx_decode_roi_UI8(blob.data(), (long)blob.size(), box.data(), (unsigned)shape.size(), raw.data(), bytes, nthreads);
+      rc = so == 2 ? sqyx_decode_slice_UI16(blob.data(), (long)blob.size(), slices.data(), (unsigned)shape.size(), raw.data(), bytes, nthreads)
+                   : sqyx_decode_slice_UI8(blob.data(), (long)blob.size(), slices.data(), (unsigned)shape.size(), raw.data(), bytes, nthreads);
     } else {
       raw.resize((size_t)bytes);
       rc = so == 2 ? SQY_Decode_UI16(blob.data(), (long)blob.size(), raw.data(), nthreads)

@@ -96,13 +96,14 @@ int k_lz4_decode_status(void* workspace, uint32_t* error, uint64_t* total_decode
 int k_lz4_decode_list(const uint8_t* src, uint64_t src_bytes, uint64_t stream_bytes, uint8_t* compact, void* workspace,
                       const uint32_t* d_list, uint32_t nlist, cudaStream_t st);
 
-// roi.cu: the voxels of a box of a stack, written densely in C order. The box is `rows` row runs of `len` voxels: run r holds
-// voxels [start(r), start(r) + len) of the stack and lands at dst + r * len; start(r) = base + sum_k i_k * stride[k], where
-// (i_0 .. i_{nlead-1}) is r in mixed radix over extent[] (the last one fastest). Trailing dimensions that the box spans whole
-// are folded into the runs, leading ones of extent 1 into base.
+// roi.cu: the voxels of a strided slice of a stack (a box when every step is 1), written densely in C order. The slice is `rows`
+// runs of `len` voxels: run r holds voxels start(r) + j * step (0 <= j < len) of the stack and lands at dst + r * len;
+// start(r) = base + sum_k i_k * stride[k], where (i_0 .. i_{nlead-1}) is r in mixed radix over extent[] (the last one fastest).
+// Trailing dimensions that the slice spans whole with step 1 are folded into the runs, leading ones of extent 1 into base; a step
+// in a leading dimension is part of its stride.
 constexpr int kRoiMaxLead = 8;
 struct RoiRuns {
-  uint64_t base, len, rows;
+  uint64_t base, len, rows, step;
   int nlead;
   uint64_t extent[kRoiMaxLead], stride[kRoiMaxLead];
   __host__ __device__ uint64_t start(uint64_t r) const {

@@ -1,11 +1,16 @@
-// Sub-volume gather (api.cu: the sqyx_decode_roi_* entry points): the voxels of a box of a stack, densely in C order, out of
+// Sub-volume gather (api.cu: the sqyx_decode_roi_* and sqyx_decode_slice_* entry points): the voxels of a strided slice of a
+// stack (a box when every step is 1), densely in C order, out of
 //   planes: the compact 16 KiB blocks of the bit planes of a uint16 bitswapW that hold the box (k_lz4_decode_list, or a
 //           sub-frame decoded whole), transposed back by the thread program of bitswap_thread.h;
 //   codes:  the compact 16 KiB blocks of 8-bit quantiser codes that hold the box, through the 256-entry decode LUT;
 //   raw:    a whole decoded stack (the crop behind the decode-whole route).
-// One kernel, templated on the source. A thread takes one aligned group of G voxels of the stack (32, or 16 codes: one 16-byte
-// load) that meets a row run and writes the voxels of the group that lie in the run to their dense place in the box: whole
-// groups with 16-byte stores where the destination allows it, the groups at the ends of a run voxel by voxel.
+// One kernel, templated on the source and on one of three thread programs, chosen by the runs' inner step at launch:
+//   run   (step 1): a thread takes one aligned group of G voxels of the stack (32, or 16 codes: one 16-byte load) that meets a
+//                   run and writes the voxels of the group that lie in the run to their dense place: whole groups with 16-byte
+//                   stores where the destination allows it, the groups at the ends of a run voxel by voxel;
+//   group (1 < step < G/2): the same groups, of which a thread writes the selected voxels, at least three of each whole group;
+//   voxel (step >= G/2, when a group holds at most two selected voxels): a thread reads one selected voxel straight from its
+//                   source (its bits of the P planes, its code, or the voxel) and writes it; nothing is transposed.
 #include "bitswap_thread.h"
 #include "common.cuh"
 #include "kernels.h"
@@ -34,6 +39,22 @@ struct FromPlanes {
     bitswap_thread::load_planes<W, false>(block, (o % kLz4BlockBytes) / (4 * W), nsel * (kLz4BlockBytes / 2), reg);
     bitswap_thread::voxels_of<W>(reg, L);
   }
+  // voxel v alone: W bits of it from each of the P planes (the layout of bitswap_thread.h's encode_chunk: in the words of
+  // group v / 32, voxel m = v % 32 is atom P-1 - m % P of half (m / P) & 1 of word m / 2P; plane p is segment P-1-p)
+  __device__ T voxel(uint64_t v) const {
+    constexpr int P = 16 / W;
+    const uint64_t o = (v / G) * (4 * W);
+    const uint32_t* seg = reinterpret_cast<const uint32_t*>(compact + (uint64_t)__ldg(pos + o / kLz4BlockBytes) * kLz4BlockBytes +
+                                                            o % kLz4BlockBytes);
+    const uint32_t m = (uint32_t)(v % G);
+    const int shift = 16 * ((m / P) & 1) + W * (P - 1 - m % P);
+    const uint64_t S = nsel * (kLz4BlockBytes / 4);
+    seg += m / (2 * P);
+    uint32_t x = 0;
+#pragma unroll
+    for (int p = 0; p < P; ++p) x |= ((__ldg(seg + (uint64_t)(P - 1 - p) * S) >> shift) & ((1u << W) - 1u)) << (p * W);
+    return (T)x;
+  }
 };
 
 struct FromCodes {
@@ -59,6 +80,10 @@ struct FromCodes {
       L[2 * i] = roi_lut[w[i] & 0xff] | ((uint32_t)roi_lut[(w[i] >> 8) & 0xff] << 16);
       L[2 * i + 1] = roi_lut[(w[i] >> 16) & 0xff] | ((uint32_t)roi_lut[w[i] >> 24] << 16);
     }
+  }
+  __device__ T voxel(uint64_t v) const {
+    extern __shared__ uint16_t roi_lut[];
+    return roi_lut[__ldg(compact + (uint64_t)__ldg(pos + v / kLz4BlockBytes) * kLz4BlockBytes + v % kLz4BlockBytes)];
   }
 };
 
@@ -93,23 +118,50 @@ struct FromVolume {
       L[i] = w;
     }
   }
+  __device__ T voxel(uint64_t v) const { return __ldg(vol + v); }
 };
 
-// items = R.rows * groups: item (r, q) is the q-th group that meets run r (groups = the most a run of R.len voxels meets)
-template <class Src>
+enum RoiProgram { kRoiRun, kRoiGroup, kRoiVoxel };
+
+// run / group: items = R.rows * groups, item (r, q) is the q-th group that meets the span of run r (groups = the most a span
+// meets); voxel: items = R.rows * R.len, one per selected voxel
+template <class Src, int kProgram>
 __global__ void __launch_bounds__(kRoiThreads) roi_gather_kernel(Src src, RoiRuns R, uint64_t groups, typename Src::T* __restrict__ dst) {
   using T = typename Src::T;
   constexpr int G = Src::G;
   constexpr int kPer = 4 / sizeof(T);
   src.prologue();
+  if (kProgram == kRoiVoxel) {
+    const uint64_t items = R.rows * R.len;
+    for (uint64_t it = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; it < items; it += (uint64_t)gridDim.x * blockDim.x) {
+      const uint64_t r = it / R.len;
+      dst[it] = src.voxel(R.start(r) + (it - r * R.len) * R.step);
+    }
+    return;
+  }
   const uint64_t items = R.rows * groups;
   for (uint64_t it = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; it < items; it += (uint64_t)gridDim.x * blockDim.x) {
-    const uint64_t r = it / groups, v0 = R.start(r), v1 = v0 + R.len;
+    const uint64_t r = it / groups, v0 = R.start(r), v1 = v0 + (kProgram == kRoiRun ? R.len : (R.len - 1) * R.step + 1);
     const uint64_t g = v0 / G + (it - r * groups);
     if (g * G >= v1) continue;
     uint32_t L[Src::kWords];
     src.load(g, L);
-    T* out = dst + r * R.len;   // voxel v of the run lands at out[v - v0]
+    T* out = dst + r * R.len;   // run: voxel v of the run lands at out[v - v0]; group: at out[(v - v0) / step]
+    if (kProgram == kRoiGroup) {
+      // the group's first selected voxel, at offset `next` in the group (G or more: none)
+      const uint64_t j0 = g * G > v0 ? (g * G - v0 + R.step - 1) / R.step : 0;
+      uint32_t next = (uint32_t)(v0 + j0 * R.step - g * G);
+      const uint32_t step = (uint32_t)R.step;
+      T* o = out + j0;
+#pragma unroll
+      for (int k = 0; k < G; ++k) {
+        if (k == next && g * G + k < v1) {
+          *o++ = (T)(L[k / kPer] >> (8 * sizeof(T) * (k % kPer)));
+          next += step;
+        }
+      }
+      continue;
+    }
     if (g * G >= v0 && (g + 1) * G <= v1 && (((uintptr_t)(out + (g * G - v0))) & 15) == 0) {
       uint4* o = reinterpret_cast<uint4*>(out + (g * G - v0));
 #pragma unroll
@@ -124,11 +176,23 @@ __global__ void __launch_bounds__(kRoiThreads) roi_gather_kernel(Src src, RoiRun
   }
 }
 
+template <class Src, int kProgram>
+void launch_program(const Src& src, const RoiRuns& R, uint64_t items, uint64_t groups, typename Src::T* dst, size_t smem,
+                    cudaStream_t st) {
+  roi_gather_kernel<Src, kProgram><<<grid_for(items, kRoiThreads), kRoiThreads, smem, st>>>(src, R, groups, dst);
+}
+
+// one launch; the program by the runs' inner step
 template <class Src>
 int launch_gather(const Src& src, const RoiRuns& R, typename Src::T* dst, size_t smem, cudaStream_t st) {
   if (R.rows == 0 || R.len == 0) return 0;
-  const uint64_t groups = (R.len + Src::G - 1) / Src::G + 1;
-  roi_gather_kernel<Src><<<grid_for(R.rows * groups, kRoiThreads), kRoiThreads, smem, st>>>(src, R, groups, dst);
+  if (R.step >= (uint64_t)Src::G / 2) {
+    launch_program<Src, kRoiVoxel>(src, R, R.rows * R.len, 0, dst, smem, st);
+  } else {
+    const uint64_t span = (R.len - 1) * R.step + 1, groups = (span + Src::G - 1) / Src::G + 1;
+    if (R.step == 1) launch_program<Src, kRoiRun>(src, R, R.rows * groups, groups, dst, smem, st);
+    else launch_program<Src, kRoiGroup>(src, R, R.rows * groups, groups, dst, smem, st);
+  }
   SQYB_COUNT_LAUNCH(1);
   return (int)cudaGetLastError();
 }

@@ -1,10 +1,12 @@
-"""Sub-volume decode against the whole-stack decode of the same blob, in one process.
+"""Sub-volume and strided-slice decode against the whole-stack decode of the same blob, in one process.
 
 cfg2 (`rmestbkrd->bitswap1->lz4`) and cfg3 (`quantiser->lz4`) on a seeded synthetic 512x2048x2048 uint16 stack, each encoded once.
 Device: sqyx_decode_roi_device_UI16 for one z-plane, 16 z-planes, a 64-row band through all planes and a 256^3 box in the middle,
 and the full sqyx_decode_device_UI16 — CUDA events, after warm-up, median of --reps. Host: sqyx_decode_roi_UI16 for the same
 boxes against SQY_Decode_UI16 (pageable buffers, wall clock), with the bytes each sends to the device. A torch.profiler pass
-over the one-plane device call gives its per-kernel times. The card's name and power limit are read in the same run.
+over the one-plane device call gives its per-kernel times. Slices (sqyx_decode_slice_*): an overview [::8, ::4, ::4], every
+8th plane [::8, :, :] and every 4th column of one plane [Z/2, :, ::4], each with its call times, blocks decoded, bytes sent and
+the gather kernel's time (torch.profiler). The card's name and power limit are read in the same run.
 
 usage: python tools/bench_roi.py [--reps 20] [--out result.json]
 """
@@ -30,6 +32,9 @@ BOXES = {
     "16_planes": [(Z // 2, Z // 2 + 16), (0, Y), (0, X)],
     "64_row_band": [(0, Z), (Y // 2 - 32, Y // 2 + 32), (0, X)],
     "box_256": [(Z // 2 - 128, Z // 2 + 128), (Y // 2 - 128, Y // 2 + 128), (X // 2 - 128, X // 2 + 128)],
+    "overview": [(0, Z, 8), (0, Y, 4), (0, X, 4)],
+    "z_step_8": [(0, Z, 8), (0, Y), (0, X)],
+    "x_step_4_one_plane": [(Z // 2, Z // 2 + 1), (0, Y), (0, X, 4)],
 }
 
 
@@ -82,6 +87,22 @@ def kernel_breakdown(fn):
     return out
 
 
+def gather_ms(fn, reps=5):
+    """the gather kernel's device time per call"""
+    from torch.profiler import ProfilerActivity, profile
+    fn()
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            fn()
+        torch.cuda.synchronize()
+    return sum(e.self_device_time_total for e in prof.key_averages() if "roi_gather_kernel" in e.key) / 1e3 / reps
+
+
+def sel_of(box):
+    return tuple(slice(*t) for t in box)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=20)
@@ -101,13 +122,13 @@ def main():
         r["full_host_ms"] = host_ms(lambda: sq.decode(h_blob, nthreads=8, out=h_full), max(3, args.reps // 4))
         r["boxes"] = {}
         for name, box in BOXES.items():
-            n = int(np.prod([hi - lo for lo, hi in box]))
+            n = int(np.prod([len(range(*t)) for t in box]))
             out = torch.empty(n, dtype=torch.int16, device="cuda")
             d = {"voxels": n}
             d["device_ms"] = device_ms(lambda: sq.decode_roi_device(blob, box, out), args.reps)
-            d["device_route"] = sq.last_roi_info()["route"]
+            d["device_route"], d["device_blocks"] = sq.last_roi_info()["route"], sq.last_roi_info()["blocks"]
             d["device_share_of_full"] = d["device_ms"] / r["full_device_ms"]
-            want = full.view(SHAPE)[tuple(slice(lo, hi) for lo, hi in box)].reshape(-1)
+            want = full.view(SHAPE)[sel_of(box)].reshape(-1)
             assert torch.equal(out, want), (cfg, name, "device")
             h_out = np.empty(n, dtype=np.uint16)
             d["host_ms"] = host_ms(lambda: sq.decode_roi(h_blob, box, nthreads=8, out=h_out), max(3, args.reps // 4))
@@ -115,6 +136,7 @@ def main():
             d["host_route"], d["host_h2d_bytes"], d["blocks"] = info["route"], info["h2d_bytes"], info["blocks"]
             d["host_h2d_share_of_blob"] = info["h2d_bytes"] / r["blob_bytes"]
             assert np.array_equal(h_out, want.cpu().numpy().view(np.uint16)), (cfg, name, "host")
+            d["gather_ms"] = gather_ms(lambda: sq.decode_roi_device(blob, box, out))
             r["boxes"][name] = d
         one = BOXES["one_plane"]
         out = torch.empty(Y * X, dtype=torch.int16, device="cuda")

@@ -63,9 +63,27 @@ int sqyx_decode_slice_UI16(const char* src, long srclength, const long* slices, 
                            int nthreads);
 int sqyx_decode_slice_UI8(const char* src, long srclength, const long* slices, unsigned ndims, char* dst, long dst_capacity,
                           int nthreads);
-/* out4 = {route of the most recent ROI or slice call on this thread's device (0 = box is the whole stack: the ordinary decode, 1 = indexed,
- * 2 = decode whole + crop, -1 = an empty box: nothing decoded), LZ4 blocks decoded by the indexed route (0 on
- * the others), bytes sent host->device (0 for device calls; the blob's payload on routes 0 and 2), voxels written}.
+/* many strided slices of one stack in one call: slices holds nsel * ndims * 3 longs, selection i's {lo_0, hi_0, step_0, lo_1, ...}
+ * at slices + 3 * ndims * i (a box is step 1). The selections are written densely in C order, one after the other with no gaps:
+ * selection i starts sizeof(voxel) * (voxels of selections 0 .. i-1) bytes into dst. Nothing is written past the last one.
+ * Selections may overlap, repeat or be empty; an empty one writes nothing and takes no space. Return codes as for one slice, with
+ * 3 also for nsel == 0 or nsel > 65536; every selection is checked before anything is decoded, so a refused call writes nothing.
+ * The indexed route plans the union of the selections' blocks once: one block table, one decode of the union (each block once;
+ * the host calls send the union in one copy), one gather launch per thread program the selections take (7 launches for a batch
+ * of boxes, at most 9). Every other blob is decoded whole once and every selection cropped out of it. A batch never takes
+ * route 0; a batch of empty selections reports route -1. */
+int sqyx_decode_slice_batch_device_UI16(const void* d_blob, long blob_bytes, const long* slices, unsigned nsel, unsigned ndims,
+                                        void* d_dst, long dst_capacity, void* stream);
+int sqyx_decode_slice_batch_device_UI8(const void* d_blob, long blob_bytes, const long* slices, unsigned nsel, unsigned ndims,
+                                       void* d_dst, long dst_capacity, void* stream);
+int sqyx_decode_slice_batch_UI16(const char* src, long srclength, const long* slices, unsigned nsel, unsigned ndims, char* dst,
+                                 long dst_capacity, int nthreads);
+int sqyx_decode_slice_batch_UI8(const char* src, long srclength, const long* slices, unsigned nsel, unsigned ndims, char* dst,
+                                long dst_capacity, int nthreads);
+/* out4 = {route of the most recent ROI, slice or slice-batch call on this thread's device (0 = box is the whole stack: the ordinary
+ * decode, 1 = indexed, 2 = decode whole + crop, -1 = an empty box: nothing decoded), LZ4 blocks decoded by the indexed route (0 on
+ * the others; a batch counts each block of the union once), bytes sent host->device (0 for device calls; the blob's payload on
+ * routes 0 and 2), voxels written (a batch: summed over its selections)}.
  * Route 0 of a host call is SQY_Decode_UI16 / _UI8 itself: like them it may stream the stack slab by slab or shard it over a
  * configured device set, and its byte count is then the payload the GPUs received together, not one device's share. */
 int sqyx_last_roi_info(long* out4);

@@ -40,6 +40,8 @@ SQYX_SYMBOLS = [
     "sqyx_diff_device", "sqyx_diff_shape_supported", "sqyx_set_devices", "sqyx_last_shard_info", "sqyx_nccl_allreduces", "sqyx_lz4_encode_ex",
     "sqyx_decode_roi_device_UI16", "sqyx_decode_roi_device_UI8", "sqyx_decode_roi_UI16", "sqyx_decode_roi_UI8", "sqyx_last_roi_info",
     "sqyx_decode_slice_device_UI16", "sqyx_decode_slice_device_UI8", "sqyx_decode_slice_UI16", "sqyx_decode_slice_UI8",
+    "sqyx_decode_slice_batch_device_UI16", "sqyx_decode_slice_batch_device_UI8", "sqyx_decode_slice_batch_UI16",
+    "sqyx_decode_slice_batch_UI8",
 ]
 
 # include/sqeazy_h5_filter.h: what HDF5 looks up in a filter plugin
@@ -256,6 +258,54 @@ def decode_roi_u8(blob: np.ndarray, box, nthreads: int = 1, out: np.ndarray | No
                        np.uint8, blob, box, nthreads, out)
 
 
+def _roi_batch(sels):
+    """sels: selections in the form decode_roi takes -> (the C array of nsel * ndims * 3 longs, nsel, ndims, the selections'
+    shapes). Every selection must have as many dimensions as the first; the library checks that number against the stack."""
+    triples = [[(int(t[0]), int(t[1]), int(t[2]) if len(t) == 3 else 1) for t in sel] for sel in sels]
+    nd = len(triples[0]) if triples else 0
+    if any(len(sel) != nd for sel in triples):
+        raise SqeazyError("decode_roi_batch: the selections differ in their number of dimensions")
+    flat = [v for sel in triples for t in sel for v in t]
+    shapes = [_roi_box(sel)[2] for sel in triples]
+    return (c_long * max(len(flat), 1))(*flat), len(triples), nd, shapes
+
+
+def _views(flat, shapes):
+    """the selections' arrays (or tensors), one after the other in the packed buffer `flat`"""
+    out, at = [], 0
+    for shape in shapes:
+        n = int(np.prod(shape))
+        out.append(flat[at : at + n].reshape(shape))
+        at += n
+    return out
+
+
+def _decode_roi_batch(fn, name, dtype, blob, sels, nthreads, out):
+    blob = np.ascontiguousarray(blob, dtype=np.uint8)
+    arr, nsel, nd, shapes = _roi_batch(sels)
+    total = sum(int(np.prod(s)) for s in shapes)
+    if out is None:
+        out = np.empty(total, dtype=dtype)
+    _check_out(out, dtype, total * np.dtype(dtype).itemsize, name)
+    rc = fn(_vp(blob), c_long(blob.size), arr, c_uint(nsel), c_uint(nd), _vp(out), c_long(out.nbytes), c_int(nthreads))
+    if rc != 0:
+        raise SqeazyError(f"{name} returned {rc}")
+    return _views(out.reshape(-1), shapes)
+
+
+def decode_roi_batch(blob: np.ndarray, sels, nthreads: int = 1, out: np.ndarray | None = None) -> list:
+    """sqyx_decode_slice_batch_UI16: many selections of one uint16 blob in one call, each a list of (lo, hi) pairs or (lo, hi, step)
+    triples as decode_roi takes them (a pair is step 1). Every LZ4 block that they need is decoded once. Returns one array per
+    selection, in its own shape; all of them are views into one packed buffer (`out`, if given: room for the voxels of every
+    selection), the selections one after the other in C order."""
+    return _decode_roi_batch(lib().sqyx_decode_slice_batch_UI16, "sqyx_decode_slice_batch_UI16", np.uint16, blob, sels, nthreads, out)
+
+
+def decode_roi_batch_u8(blob: np.ndarray, sels, nthreads: int = 1, out: np.ndarray | None = None) -> list:
+    """sqyx_decode_slice_batch_UI8: the same for uint8 stacks"""
+    return _decode_roi_batch(lib().sqyx_decode_slice_batch_UI8, "sqyx_decode_slice_batch_UI8", np.uint8, blob, sels, nthreads, out)
+
+
 def last_roi_info():
     """the most recent sub-volume decode on this thread's device: route (0 = the whole stack, 1 = indexed, 2 = decoded whole and
     cropped, -1 = empty box), LZ4 blocks the indexed route decoded, bytes sent host -> device, voxels written"""
@@ -361,6 +411,31 @@ def decode_roi_device_u8(blob, box, out, stream=None):
     L = lib()
     return _decode_roi_device((L.sqyx_decode_roi_device_UI8, L.sqyx_decode_slice_device_UI8),
                               ("sqyx_decode_roi_device_UI8", "sqyx_decode_slice_device_UI8"), blob, box, out, stream)
+
+
+def _decode_roi_batch_device(fn, name, blob, sels, out, stream):
+    import torch
+    assert blob.is_cuda and out.is_cuda and blob.is_contiguous() and out.is_contiguous()
+    arr, nsel, nd, shapes = _roi_batch(sels)
+    with torch.cuda.device(blob.device):
+        rc = fn(_dp(blob), c_long(blob.numel()), arr, c_uint(nsel), c_uint(nd), _dp(out), c_long(out.numel() * out.element_size()),
+                _stream_handle(stream))
+    if rc != 0:
+        raise SqeazyError(f"{name} returned {rc}")
+    return _views(out.view(-1), shapes)
+
+
+def decode_roi_batch_device(blob, sels, out, stream=None):
+    """sqyx_decode_slice_batch_device_UI16. blob: uint8 CUDA tensor; sels: selections as decode_roi_batch takes them; out: CUDA
+    tensor with room for the voxels of every selection, written one after the other. Returns one view of `out` per selection, in
+    its shape. For K patches of one shape, out.view(K, *shape) is the batch."""
+    return _decode_roi_batch_device(lib().sqyx_decode_slice_batch_device_UI16, "sqyx_decode_slice_batch_device_UI16", blob, sels, out,
+                                    stream)
+
+
+def decode_roi_batch_device_u8(blob, sels, out, stream=None):
+    return _decode_roi_batch_device(lib().sqyx_decode_slice_batch_device_UI8, "sqyx_decode_slice_batch_device_UI8", blob, sels, out,
+                                    stream)
 
 
 def decode_batch_device(blobs, outs):

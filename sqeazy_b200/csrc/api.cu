@@ -80,12 +80,26 @@ struct Arena {
     *out = ptr[slot];
     return 0;
   }
+  // host memory: the sub-frame that the indexed host route of the ROI calls assembles (roi_host). It is kept across calls: a buffer
+  // of hundreds of MB (a batch of patches) would be mapped afresh by every allocation and have all its pages faulted in again
+  std::unique_ptr<uint8_t[]> frame;
+  size_t frame_cap = 0;
+  uint8_t* host_frame(size_t bytes) {
+    if (frame_cap < bytes) {
+      frame.reset();
+      frame.reset(new uint8_t[bytes]);   // uninitialised: the caller writes every byte it sends
+      frame_cap = bytes;
+    }
+    return frame.get();
+  }
   void release() {
     for (int i = 0; i < kNumSlots; ++i) {
       if (ptr[i]) cudaFree(ptr[i]);
       ptr[i] = nullptr;
       cap[i] = 0;
     }
+    frame.reset();
+    frame_cap = 0;
   }
 };
 
@@ -1011,18 +1025,43 @@ int roi_of(const std::vector<uint64_t>& shape, const long* sel, unsigned width, 
   return 0;
 }
 
-// The blocks of an indexed stream (indexed_stream) that hold a voxel of a slice: `runs` of every set, nsel blocks per set. They are decoded
-// into compact places, set after set: list[t] = the stream's block at compact place t, pos[k] = the place of block k within its
-// set (~0: not needed).
+// The selections of a call: nsel of them one after the other, ndims tuples of `width` longs each (roi_of), and their voxels in
+// all. 3 when any is malformed, or nsel is 0 or above kMaxSelections.
+constexpr unsigned kMaxSelections = 65536;
+int rois_of(const std::vector<uint64_t>& shape, const long* sels, unsigned width, unsigned ndims, unsigned nsel, std::vector<Roi>* out,
+            uint64_t* voxels) {
+  if (!sels || nsel == 0 || nsel > kMaxSelections) return 3;
+  out->assign(nsel, Roi{});
+  *voxels = 0;
+  for (unsigned i = 0; i < nsel; ++i) {
+    if (int rc = roi_of(shape, sels + (size_t)width * ndims * i, width, ndims, &(*out)[i])) return rc;
+    *voxels += (*out)[i].voxels;
+  }
+  return 0;
+}
+
+// The blocks of an indexed stream (indexed_stream) that hold a voxel of any of the selections: `runs` of every set (the union of
+// every selection's blocks, sorted and disjoint), nsel blocks per set. Each block is decoded once, into compact places, set after
+// set: list[t] = the stream's block at compact place t, pos[k] = the place of block k within its set (~0: not needed).
 struct RoiPlan {
   std::vector<BlockRun> runs;
   uint64_t nsel = 0;
   std::vector<uint32_t> list, pos;
 };
 
-RoiPlan roi_plan(const StreamGeom& geo, const RoiRuns& R) {
+RoiPlan roi_plan(const StreamGeom& geo, const std::vector<Roi>& rois) {
   RoiPlan P;
-  P.runs = geo.blocks_of(R);
+  std::vector<BlockRun> all;
+  for (const Roi& roi : rois) {
+    if (!roi.voxels) continue;
+    const std::vector<BlockRun> b = geo.blocks_of(roi.runs);
+    all.insert(all.end(), b.begin(), b.end());
+  }
+  std::sort(all.begin(), all.end(), [](const BlockRun& a, const BlockRun& b) { return a.k0 < b.k0; });
+  for (const BlockRun& b : all) {
+    if (!P.runs.empty() && b.k0 <= P.runs.back().k1) P.runs.back().k1 = std::max(P.runs.back().k1, b.k1);
+    else P.runs.push_back(b);
+  }
   P.pos.assign(geo.set_blocks(), ~0u);
   for (const BlockRun& b : P.runs)
     for (uint64_t k = b.k0; k < b.k1; ++k) P.pos[k] = (uint32_t)P.nsel++;
@@ -1033,32 +1072,56 @@ RoiPlan roi_plan(const StreamGeom& geo, const RoiRuns& R) {
   return P;
 }
 
-// P's tables on the device (the arena's kSlotRoi): pos, and the list when the caller decodes by list
-int roi_tables(Arena& A, const RoiPlan& P, bool with_list, uint32_t** d_pos, uint32_t** d_list, cudaStream_t st) {
+// The gather's tables on the device, in the arena's kSlotRoi: for a batch (the sqyx_decode_slice_batch_* calls) the descriptors of
+// its selections (kernels.h: roi_batch; `host` holds what that copy reads until the caller synchronises), then P's pos, then P's
+// list when the caller decodes by list, one copy each. P = nullptr: the descriptors alone. A single call takes no descriptor: its
+// runs go to roi_gather_kernel by value, which tools/ab_roi.py measured faster than a batch of one (profiles/README.md).
+struct RoiTables {
+  RoiBatch batch;
+  const RoiSel* d_sels;   // nullptr: a single call
+  const uint32_t *d_pos, *d_list;
+};
+
+int roi_tables(Arena& A, RoiSource source, const std::vector<Roi>& rois, bool batch, const RoiPlan* P, bool with_list,
+               std::vector<RoiSel>& host, RoiTables* T, cudaStream_t st) {
+  if (batch) {
+    std::vector<RoiRuns> runs;
+    runs.reserve(rois.size());
+    for (const Roi& roi : rois) runs.push_back(roi.runs);
+    host.resize(rois.size());
+    T->batch = roi_batch(source, runs.data(), runs.size(), host.data());
+  }
+  const size_t sel_bytes = batch ? sizeof(RoiSel) * rois.size() : 0, pos_bytes = P ? 4 * P->pos.size() : 0;
+  const size_t list_bytes = P && with_list ? 4 * P->list.size() : 0;
   void* p = nullptr;
-  if (A.get(kSlotRoi, 4 * (P.pos.size() + P.list.size()), &p)) return 1;
-  *d_pos = static_cast<uint32_t*>(p);
-  *d_list = *d_pos + P.pos.size();
-  CK(cudaMemcpyAsync(*d_pos, P.pos.data(), 4 * P.pos.size(), cudaMemcpyHostToDevice, st));
-  if (with_list) CK(cudaMemcpyAsync(*d_list, P.list.data(), 4 * P.list.size(), cudaMemcpyHostToDevice, st));
+  if (A.get(kSlotRoi, sel_bytes + pos_bytes + list_bytes, &p)) return 1;
+  uint8_t* d = static_cast<uint8_t*>(p);
+  T->d_sels = batch ? reinterpret_cast<const RoiSel*>(d) : nullptr;
+  T->d_pos = reinterpret_cast<const uint32_t*>(d + sel_bytes);
+  T->d_list = reinterpret_cast<const uint32_t*>(d + sel_bytes + pos_bytes);
+  if (sel_bytes) CK(cudaMemcpyAsync(d, host.data(), sel_bytes, cudaMemcpyHostToDevice, st));
+  if (pos_bytes) CK(cudaMemcpyAsync(d + sel_bytes, P->pos.data(), pos_bytes, cudaMemcpyHostToDevice, st));
+  if (list_bytes) CK(cudaMemcpyAsync(d + sel_bytes + pos_bytes, P->list.data(), list_bytes, cudaMemcpyHostToDevice, st));
   return 0;
 }
 
 // the gather behind the indexed route, from the compact blocks of P (`ws`: the block decode's workspace), then the block decode's
-// status: 11 (planes) / 101 (codes), what the whole-stack decode returns, when a block that the slice needs did not decode
-int roi_finish(Arena& A, const Pipeline& pl, int w, const RoiPlan& P, const uint32_t* d_pos, const RoiRuns& R, const uint8_t* compact,
-               void* ws, uint16_t* d_dst, cudaStream_t st) {
+// status: 11 (planes) / 101 (codes), what the whole-stack decode returns, when a block that a selection needs did not decode
+int roi_finish(Arena& A, const Pipeline& pl, int w, const RoiPlan& P, const std::vector<Roi>& rois, const RoiTables& T,
+               const uint8_t* compact, void* ws, uint16_t* d_dst, cudaStream_t st) {
   if (w) {
-    CKK(k_roi_gather_planes(w, compact, d_pos, P.nsel, R, d_dst, st));
+    if (T.d_sels) CKK(k_roi_gather_planes_batch(w, compact, T.d_pos, P.nsel, T.d_sels, T.batch, d_dst, st));
+    else CKK(k_roi_gather_planes(w, compact, T.d_pos, P.nsel, rois[0].runs, d_dst, st));
   } else {
     SmallSlot small;
     if (small_slot(A, &small)) return 1;
     CK(cudaMemcpyAsync(small.dec_lut, pl.sink.decode_lut, 512, cudaMemcpyHostToDevice, st));
-    CKK(k_roi_gather_codes(compact, d_pos, small.dec_lut, R, d_dst, st));
+    if (T.d_sels) CKK(k_roi_gather_codes_batch(compact, T.d_pos, small.dec_lut, T.d_sels, T.batch, d_dst, st));
+    else CKK(k_roi_gather_codes(compact, T.d_pos, small.dec_lut, rois[0].runs, d_dst, st));
   }
   uint32_t err = 0, none = 0;
   uint64_t total = 0;
-  if (k_lz4_decode_status(ws, &err, &total, &none, st)) return 1;   // (synchronises: P's host tables have been consumed)
+  if (k_lz4_decode_status(ws, &err, &total, &none, st)) return 1;   // (synchronises: the host tables have been consumed)
   if (err || total != (uint64_t)P.list.size() * kLz4BlockBytes) {
     std::fprintf(stderr, "[sqeazy_b200] lz4 decode failed (code %u)\n", err ? err : 5u);
     return w ? 11 : 101;
@@ -1066,14 +1129,29 @@ int roi_finish(Arena& A, const Pipeline& pl, int w, const RoiPlan& P, const uint
   return 0;
 }
 
-// A slice of a blob in device memory (not empty, not the whole stack) into d_dst. Indexed route (info[0] = 1): the block table of
-// the whole payload, one launch for the blocks that hold a selected voxel, one gather. Every other blob (info[0] = 2): decoded whole into the
-// arena, then cropped.
-int roi_device(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes, const Roi& roi,
-               void* d_dst, cudaStream_t st, long* info) {
+// the crop behind the decode-whole route: every selection out of the whole decoded stack `full` of N voxels
+int roi_crop(Arena& A, const Pipeline& pl, const void* full, uint64_t N, const std::vector<Roi>& rois, bool batch,
+             std::vector<RoiSel>& host, void* d_dst, cudaStream_t st) {
+  RoiTables T{};
+  if (!batch) {
+    CKK(k_roi_crop(pl.elem, full, N, rois[0].runs, d_dst, st));
+    return 0;
+  }
+  if (roi_tables(A, kRoiVolume, rois, true, nullptr, false, host, &T, st)) return 1;
+  CKK(k_roi_crop_batch(pl.elem, full, N, T.d_sels, T.batch, d_dst, st));
+  return 0;
+}
+
+// Selections of a blob in device memory (not all empty; not one selection of the whole stack) into d_dst, one after the other.
+// Indexed route (info[0] = 1): the block table of the whole payload, one launch for the blocks that hold a selected voxel of any
+// selection, each once, and the gather. Every other blob (info[0] = 2): decoded whole into the arena once, then cropped.
+int roi_device(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d_payload, uint64_t payload_bytes,
+               const std::vector<Roi>& rois, bool batch, void* d_dst, cudaStream_t st, long* info) {
   const uint64_t N = shape_product(hdr.shape);
   StreamGeom geo{};
   int w = 0;
+  std::vector<RoiSel> host;   // what the descriptor copy reads
+  RoiTables T{};
   if (indexed_stream(pl, N, &geo, &w)) {
     void* ws = nullptr;
     if (A.get(kSlotWs, k_lz4_decode_workspace_bytes(geo.bytes()), &ws)) return 1;
@@ -1081,13 +1159,14 @@ int roi_device(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d
     bool own = false;
     if (k_lz4_decode_own_frame(ws, geo.bytes(), &own, st)) return 1;
     if (own) {
-      const RoiPlan P = roi_plan(geo, roi.runs);
+      const RoiPlan P = roi_plan(geo, rois);
       void* compact = nullptr;
-      uint32_t *d_pos = nullptr, *d_list = nullptr;
-      if (A.get(kSlotA, P.list.size() * kLz4BlockBytes, &compact) || roi_tables(A, P, true, &d_pos, &d_list, st)) return 1;
+      if (A.get(kSlotA, P.list.size() * kLz4BlockBytes, &compact) ||
+          roi_tables(A, w ? kRoiPlanes : kRoiCodes, rois, batch, &P, true, host, &T, st))
+        return 1;
       info[0] = 1;
-      CKK(k_lz4_decode_list(d_payload, payload_bytes, geo.bytes(), static_cast<uint8_t*>(compact), ws, d_list, (uint32_t)P.list.size(), st));
-      if (int rc = roi_finish(A, pl, w, P, d_pos, roi.runs, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_dst), st))
+      CKK(k_lz4_decode_list(d_payload, payload_bytes, geo.bytes(), static_cast<uint8_t*>(compact), ws, T.d_list, (uint32_t)P.list.size(), st));
+      if (int rc = roi_finish(A, pl, w, P, rois, T, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_dst), st))
         return rc;
       info[1] = (long)P.list.size();
       return 0;
@@ -1097,28 +1176,31 @@ int roi_device(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d
   void* full = nullptr;
   if (A.get(kSlotOut, pl.elem * N, &full)) return 1;
   if (int rc = decode_device_impl(A, hdr, pl, d_payload, payload_bytes, full, pl.elem * N, st)) return rc;
-  CKK(k_roi_crop(pl.elem, full, N, roi.runs, d_dst, st));
+  if (int rc = roi_crop(A, pl, full, N, rois, batch, host, d_dst, st)) return rc;
   CK(cudaStreamSynchronize(st));
   return 0;
 }
 
-// The same for a blob in host memory, into the host buffer dst. Indexed route: the blocks the slice needs are cut out of the blob
-// on the host into a frame of their own (index frame, their blocks, EndMark), which alone crosses the bus in one copy and is
-// decoded whole on the device: its blocks land at the compact places of the device route. Otherwise the payload goes to the
-// device as the whole-stack host decode sends it, is decoded whole and cropped. info[2] = the bytes sent to the device.
-int roi_host(Arena& A, const Header& hdr, const Pipeline& pl, const char* src, uint64_t srclength, const Roi& roi, char* dst,
-             int nthreads, long* info) {
-  const uint64_t N = shape_product(hdr.shape), box_bytes = pl.elem * roi.voxels;
+// The same for a blob in host memory, into the host buffer dst (`voxels` in all). Indexed route: the blocks the selections need,
+// each once, are cut out of the blob on the host into a frame of their own (index frame, their blocks, EndMark), which alone crosses
+// the bus in one copy and is decoded whole on the device: its blocks land at the compact places of the device route. Otherwise the
+// payload goes to the device as the whole-stack host decode sends it, once, is decoded whole and cropped. info[2] = the bytes sent
+// to the device.
+int roi_host(Arena& A, const Header& hdr, const Pipeline& pl, const char* src, uint64_t srclength, const std::vector<Roi>& rois,
+             bool batch, uint64_t voxels, char* dst, int nthreads, long* info) {
+  const uint64_t N = shape_product(hdr.shape), box_bytes = pl.elem * voxels;
   const uint8_t* payload = reinterpret_cast<const uint8_t*>(src) + hdr.size;
   const uint64_t payload_bytes = srclength - hdr.size;
   cudaStream_t st = nullptr;
   StreamGeom geo{};
   int w = 0;
   SqybIndexHeader index;
+  std::vector<RoiSel> host;   // what the descriptor copy reads
+  RoiTables T{};
   if (indexed_stream(pl, N, &geo, &w) && lz4_read_prefix(payload, payload_bytes, &index) &&
       index.block_bytes == (uint32_t)kLz4BlockBytes && index.nblocks == geo.blocks() && index.raw_bytes == geo.bytes()) {
     info[0] = 1;
-    const RoiPlan P = roi_plan(geo, roi.runs);
+    const RoiPlan P = roi_plan(geo, rois);
     std::vector<BlockRun> runs;   // the needed blocks of every set, in stream order
     for (uint32_t j = 0; j < geo.sets; ++j)
       for (const BlockRun& b : P.runs) runs.push_back({(uint64_t)j * geo.set_blocks() + b.k0, (uint64_t)j * geo.set_blocks() + b.k1});
@@ -1130,28 +1212,28 @@ int roi_host(Arena& A, const Header& hdr, const Pipeline& pl, const char* src, u
     uint64_t body = 0;
     for (size_t i = 0; i < runs.size(); ++i) body += off[2 * i + 1] - off[2 * i];
     const uint64_t prefix = lz4_prefix_bytes(nlist), sub_bytes = prefix + body + kLz4EndMarkBytes;
-    std::unique_ptr<uint8_t[]> sub(new uint8_t[sub_bytes]);   // every byte is written below
-    lz4_write_prefix(sub.get(), (uint32_t)nlist, sub_raw, kLz4FrameHeaderBytes + body + kLz4EndMarkBytes);
+    uint8_t* const sub = A.host_frame(sub_bytes);   // every byte is written below
+    lz4_write_prefix(sub, (uint32_t)nlist, sub_raw, kLz4FrameHeaderBytes + body + kLz4EndMarkBytes);
     for (uint64_t t = 0; t < nlist; ++t)
-      std::memcpy(sub.get() + kSkippableHeaderBytes + sizeof(SqybIndexHeader) + 4 * t, words + 4ull * P.list[t], 4);
+      std::memcpy(sub + kSkippableHeaderBytes + sizeof(SqybIndexHeader) + 4 * t, words + 4ull * P.list[t], 4);
     const uint8_t* blocks = payload + lz4_prefix_bytes(geo.blocks());
     uint64_t q = prefix;
     for (size_t i = 0; i < runs.size(); ++i) {
-      std::memcpy(sub.get() + q, blocks + off[2 * i], off[2 * i + 1] - off[2 * i]);
+      std::memcpy(sub + q, blocks + off[2 * i], off[2 * i + 1] - off[2 * i]);
       q += off[2 * i + 1] - off[2 * i];
     }
-    lz4_put32(sub.get() + q, 0u);   // EndMark
+    lz4_put32(sub + q, 0u);   // EndMark
     void *d_sub = nullptr, *ws = nullptr, *compact = nullptr, *d_box = nullptr;
-    uint32_t *d_pos = nullptr, *d_list = nullptr;
     if (A.get(kSlotIn, sub_bytes, &d_sub) || A.get(kSlotWs, k_lz4_decode_workspace_bytes(sub_raw), &ws) ||
-        A.get(kSlotA, sub_raw, &compact) || A.get(kSlotOut, box_bytes, &d_box) || roi_tables(A, P, false, &d_pos, &d_list, st))
+        A.get(kSlotA, sub_raw, &compact) || A.get(kSlotOut, box_bytes, &d_box) ||
+        roi_tables(A, w ? kRoiPlanes : kRoiCodes, rois, batch, &P, false, host, &T, st))
       return 1;
-    CK((cudaError_t)staged_h2d(d_sub, sub.get(), sub_bytes, nthreads, st));
+    CK((cudaError_t)staged_h2d(d_sub, sub, sub_bytes, nthreads, st));
     info[2] = (long)sub_bytes;
     const uint8_t* d_frame = static_cast<const uint8_t*>(d_sub);
     CKK(k_lz4_decode_tables(d_frame, sub_bytes, sub_raw, ws, 0, 0, st));
     CKK(k_lz4_decode_run(d_frame, sub_bytes, static_cast<uint8_t*>(compact), sub_raw, ws, 0, 0, 0, 0, 0, st));
-    if (int rc = roi_finish(A, pl, w, P, d_pos, roi.runs, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_box), st))
+    if (int rc = roi_finish(A, pl, w, P, rois, T, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_box), st))
       return rc;
     info[1] = (long)nlist;
     CK((cudaError_t)staged_d2h(dst, d_box, box_bytes, nthreads, st));
@@ -1166,7 +1248,7 @@ int roi_host(Arena& A, const Header& hdr, const Pipeline& pl, const char* src, u
   info[2] = (long)payload_bytes;
   if (int rc = decode_device_impl(A, hdr, pl, static_cast<const uint8_t*>(d_in), payload_bytes, full, pl.elem * N, st)) return rc;
   if (A.get(kSlotA, box_bytes, &d_box)) return 1;
-  CKK(k_roi_crop(pl.elem, full, N, roi.runs, d_box, st));
+  if (int rc = roi_crop(A, pl, full, N, rois, batch, host, d_box, st)) return rc;
   CK((cudaError_t)staged_d2h(dst, d_box, box_bytes, nthreads, st));
   CK(cudaStreamSynchronize(st));
   return 0;
@@ -1798,10 +1880,12 @@ int SQY_Decode_UI8(const char* src, long srclength, char* dst, int nthreads) {
   return host_decode(1, src, srclength, dst, nthreads);
 }
 
-// ---- sub-volume decode: the eight entry points share the planner, the checks and the whole-stack route. sel: ndims tuples of
-// `width` longs, boxes (width 2) or strided slices (width 3); roi_of ----
+// ---- sub-volume decode: the twelve entry points share the planner, the checks and the whole-stack route. sel: nsel selections
+// one after the other, each ndims tuples of `width` longs, boxes (width 2) or strided slices (width 3); rois_of. The selections
+// are written one after the other. A batch (the sqyx_decode_slice_batch_* calls) never takes route 0: its union then holds every
+// block ----
 static int decode_roi_device(int elem, const void* d_blob, long blob_bytes, const long* sel, unsigned width, unsigned ndims,
-                             void* d_dst, long dst_capacity, void* stream) {
+                             unsigned nsel, bool batch, void* d_dst, long dst_capacity, void* stream) {
   try {
     if (!d_blob || blob_bytes <= 0 || dst_capacity < 0) return 1;
     DevLock dl;
@@ -1815,48 +1899,50 @@ static int decode_roi_device(int elem, const void* d_blob, long blob_bytes, cons
     if (parse_blob_header_device(blob, (uint64_t)blob_bytes, hdr, st) || sizeof_typename(hdr.raw_type) != (unsigned)elem) return 1;
     Pipeline pl;
     if (!(elem == 1 ? build_pipeline_u8(hdr.pipeline, pl) : build_pipeline_u16(hdr.pipeline, pl)) || pl.empty()) return 1;
-    Roi roi;
-    if (int rc = roi_of(hdr.shape, sel, width, ndims, &roi)) return rc;
-    if ((uint64_t)dst_capacity < (uint64_t)elem * roi.voxels || (roi.voxels && !d_dst)) return 1;
-    if (roi.voxels == 0) return 0;
+    std::vector<Roi> rois;
+    uint64_t voxels = 0;
+    if (int rc = rois_of(hdr.shape, sel, width, ndims, nsel, &rois, &voxels)) return rc;
+    if ((uint64_t)dst_capacity < (uint64_t)elem * voxels || (voxels && !d_dst)) return 1;
+    if (voxels == 0) return 0;
     int rc = 0;
-    if (roi.whole) {
+    if (!batch && rois[0].whole) {
       info[0] = 0;
       rc = decode_device_blob(A, elem, d_blob, blob_bytes, d_dst, dst_capacity, st);
     } else {
-      rc = roi_device(A, hdr, pl, blob + hdr.size, (uint64_t)blob_bytes - hdr.size, roi, d_dst, st, info);
+      rc = roi_device(A, hdr, pl, blob + hdr.size, (uint64_t)blob_bytes - hdr.size, rois, batch, d_dst, st, info);
     }
-    if (rc == 0) info[3] = (long)roi.voxels;
+    if (rc == 0) info[3] = (long)voxels;
     return rc;
   } catch (...) {
     return 1;
   }
 }
 
-static int decode_roi_host(int elem, const char* src, long srclength, const long* sel, unsigned width, unsigned ndims, char* dst,
-                           long dst_capacity, int nthreads) {
-  NvtxRange range(width == 3 ? (elem == 1 ? "sqyx_decode_slice_UI8" : "sqyx_decode_slice_UI16")
-                             : (elem == 1 ? "sqyx_decode_roi_UI8" : "sqyx_decode_roi_UI16"));
+static int decode_roi_host(const char* name, int elem, const char* src, long srclength, const long* sel, unsigned width, unsigned ndims,
+                           unsigned nsel, bool batch, char* dst, long dst_capacity, int nthreads) {
+  NvtxRange range(name);
   try {
     if (!src || srclength <= 0 || dst_capacity < 0) return 1;
     const Header hdr = unpack_header(src, (size_t)srclength);
     if (!hdr.valid || sizeof_typename(hdr.raw_type) != (unsigned)elem) return 1;
     Pipeline pl;
     if (!(elem == 1 ? build_pipeline_u8(hdr.pipeline, pl) : build_pipeline_u16(hdr.pipeline, pl)) || pl.empty()) return 1;
-    Roi roi;
-    if (int rc = roi_of(hdr.shape, sel, width, ndims, &roi)) return rc;
-    if ((uint64_t)dst_capacity < (uint64_t)elem * roi.voxels || (roi.voxels && !dst)) return 1;
+    std::vector<Roi> rois;
+    uint64_t voxels = 0;
+    if (int rc = rois_of(hdr.shape, sel, width, ndims, nsel, &rois, &voxels)) return rc;
+    if ((uint64_t)dst_capacity < (uint64_t)elem * voxels || (voxels && !dst)) return 1;
     long info[4] = {-1, 0, 0, 0};
     int rc = 0;
-    if (roi.voxels && roi.whole) {
+    const bool whole = !batch && rois[0].whole;
+    if (voxels && whole) {
       info[0] = 0;
       info[2] = srclength - (long)hdr.size;
       rc = host_decode(elem, src, srclength, dst, nthreads);   // takes the device locks it needs itself
     }
     DevLock dl;
     if (dl.acquire()) return 1;
-    if (roi.voxels && !roi.whole) rc = roi_host(dl.dev->arena, hdr, pl, src, (uint64_t)srclength, roi, dst, nthreads, info);
-    if (rc == 0) info[3] = (long)roi.voxels;
+    if (voxels && !whole) rc = roi_host(dl.dev->arena, hdr, pl, src, (uint64_t)srclength, rois, batch, voxels, dst, nthreads, info);
+    if (rc == 0) info[3] = (long)voxels;
     std::copy(info, info + 4, dl.dev->roi_info);
     return rc;
   } catch (...) {
@@ -1866,33 +1952,49 @@ static int decode_roi_host(int elem, const char* src, long srclength, const long
 
 int sqyx_decode_roi_device_UI16(const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst, long dst_capacity,
                                 void* stream) {
-  return decode_roi_device(2, d_blob, blob_bytes, box, 2, ndims, d_dst, dst_capacity, stream);
+  return decode_roi_device(2, d_blob, blob_bytes, box, 2, ndims, 1, false, d_dst, dst_capacity, stream);
 }
 int sqyx_decode_roi_device_UI8(const void* d_blob, long blob_bytes, const long* box, unsigned ndims, void* d_dst, long dst_capacity,
                                void* stream) {
-  return decode_roi_device(1, d_blob, blob_bytes, box, 2, ndims, d_dst, dst_capacity, stream);
+  return decode_roi_device(1, d_blob, blob_bytes, box, 2, ndims, 1, false, d_dst, dst_capacity, stream);
 }
 int sqyx_decode_roi_UI16(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads) {
-  return decode_roi_host(2, src, srclength, box, 2, ndims, dst, dst_capacity, nthreads);
+  return decode_roi_host("sqyx_decode_roi_UI16", 2, src, srclength, box, 2, ndims, 1, false, dst, dst_capacity, nthreads);
 }
 int sqyx_decode_roi_UI8(const char* src, long srclength, const long* box, unsigned ndims, char* dst, long dst_capacity, int nthreads) {
-  return decode_roi_host(1, src, srclength, box, 2, ndims, dst, dst_capacity, nthreads);
+  return decode_roi_host("sqyx_decode_roi_UI8", 1, src, srclength, box, 2, ndims, 1, false, dst, dst_capacity, nthreads);
 }
 int sqyx_decode_slice_device_UI16(const void* d_blob, long blob_bytes, const long* slices, unsigned ndims, void* d_dst,
                                   long dst_capacity, void* stream) {
-  return decode_roi_device(2, d_blob, blob_bytes, slices, 3, ndims, d_dst, dst_capacity, stream);
+  return decode_roi_device(2, d_blob, blob_bytes, slices, 3, ndims, 1, false, d_dst, dst_capacity, stream);
 }
 int sqyx_decode_slice_device_UI8(const void* d_blob, long blob_bytes, const long* slices, unsigned ndims, void* d_dst,
                                  long dst_capacity, void* stream) {
-  return decode_roi_device(1, d_blob, blob_bytes, slices, 3, ndims, d_dst, dst_capacity, stream);
+  return decode_roi_device(1, d_blob, blob_bytes, slices, 3, ndims, 1, false, d_dst, dst_capacity, stream);
 }
 int sqyx_decode_slice_UI16(const char* src, long srclength, const long* slices, unsigned ndims, char* dst, long dst_capacity,
                            int nthreads) {
-  return decode_roi_host(2, src, srclength, slices, 3, ndims, dst, dst_capacity, nthreads);
+  return decode_roi_host("sqyx_decode_slice_UI16", 2, src, srclength, slices, 3, ndims, 1, false, dst, dst_capacity, nthreads);
 }
 int sqyx_decode_slice_UI8(const char* src, long srclength, const long* slices, unsigned ndims, char* dst, long dst_capacity,
                           int nthreads) {
-  return decode_roi_host(1, src, srclength, slices, 3, ndims, dst, dst_capacity, nthreads);
+  return decode_roi_host("sqyx_decode_slice_UI8", 1, src, srclength, slices, 3, ndims, 1, false, dst, dst_capacity, nthreads);
+}
+int sqyx_decode_slice_batch_device_UI16(const void* d_blob, long blob_bytes, const long* slices, unsigned nsel, unsigned ndims,
+                                        void* d_dst, long dst_capacity, void* stream) {
+  return decode_roi_device(2, d_blob, blob_bytes, slices, 3, ndims, nsel, true, d_dst, dst_capacity, stream);
+}
+int sqyx_decode_slice_batch_device_UI8(const void* d_blob, long blob_bytes, const long* slices, unsigned nsel, unsigned ndims,
+                                       void* d_dst, long dst_capacity, void* stream) {
+  return decode_roi_device(1, d_blob, blob_bytes, slices, 3, ndims, nsel, true, d_dst, dst_capacity, stream);
+}
+int sqyx_decode_slice_batch_UI16(const char* src, long srclength, const long* slices, unsigned nsel, unsigned ndims, char* dst,
+                                 long dst_capacity, int nthreads) {
+  return decode_roi_host("sqyx_decode_slice_batch_UI16", 2, src, srclength, slices, 3, ndims, nsel, true, dst, dst_capacity, nthreads);
+}
+int sqyx_decode_slice_batch_UI8(const char* src, long srclength, const long* slices, unsigned nsel, unsigned ndims, char* dst,
+                                long dst_capacity, int nthreads) {
+  return decode_roi_host("sqyx_decode_slice_batch_UI8", 1, src, srclength, slices, 3, ndims, nsel, true, dst, dst_capacity, nthreads);
 }
 
 int sqyx_last_roi_info(long* out4) {

@@ -124,5 +124,27 @@ int k_roi_gather_codes(const uint8_t* compact, const uint32_t* pos, const uint16
                        cudaStream_t st);
 // from a whole decoded stack of n voxels of elem bytes (the crop)
 int k_roi_crop(int elem, const void* vol, uint64_t n, const RoiRuns& R, void* dst, cudaStream_t st);
+// The same gathers for a batch of selections, written densely one after the other, one launch per thread program that one of them
+// takes. RoiSel describes a non-empty selection in device memory: its runs, its first voxel in the packed destination, and the
+// work items of the selections in front of it in its program's launch.
+enum RoiProgram { kRoiRun, kRoiGroup, kRoiVoxel };
+struct RoiSel {
+  RoiRuns runs;
+  uint64_t first, before;
+};
+// the launches: program p takes descriptors [begin[p], begin[p] + count[p]) and items[p] work items
+struct RoiBatch {
+  uint32_t begin[3], count[3];
+  uint64_t items[3];
+};
+enum RoiSource { kRoiPlanes, kRoiCodes, kRoiVolume };
+// host: the descriptors of selections R[0 .. n) in the order the launches take them, into sels (room for n; an empty selection
+// takes no descriptor and no room in the destination), for a gather from `source`
+RoiBatch roi_batch(RoiSource source, const RoiRuns* R, size_t n, RoiSel* sels);
+int k_roi_gather_planes_batch(int w, const uint8_t* compact, const uint32_t* pos, uint64_t nsel, const RoiSel* d_sels, const RoiBatch& B,
+                              uint16_t* dst, cudaStream_t st);
+int k_roi_gather_codes_batch(const uint8_t* compact, const uint32_t* pos, const uint16_t* lut_dev, const RoiSel* d_sels, const RoiBatch& B,
+                             uint16_t* dst, cudaStream_t st);
+int k_roi_crop_batch(int elem, const void* vol, uint64_t n, const RoiSel* d_sels, const RoiBatch& B, void* dst, cudaStream_t st);
 
 }  // namespace sqyb

@@ -4,7 +4,9 @@
 //           sub-frame decoded whole), transposed back by the thread program of bitswap_thread.h;
 //   codes:  the compact 16 KiB blocks of 8-bit quantiser codes that hold the box, through the 256-entry decode LUT;
 //   raw:    a whole decoded stack (the crop behind the decode-whole route).
-// One kernel, templated on the source and on one of three thread programs, chosen by the runs' inner step at launch:
+// One kernel, templated on the source and on one of three thread programs, chosen by the runs' inner step at launch (the single
+// calls: one selection, its runs by value), and its batch form (roi_gather_batch_kernel: many selections, written one after the
+// other, one launch per program that any of them takes):
 //   run   (step 1): a thread takes one aligned group of G voxels of the stack (32, or 16 codes: one 16-byte load) that meets a
 //                   run and writes the voxels of the group that lie in the run to their dense place: whole groups with 16-byte
 //                   stores where the destination allows it, the groups at the ends of a run voxel by voxel;
@@ -121,8 +123,6 @@ struct FromVolume {
   __device__ T voxel(uint64_t v) const { return __ldg(vol + v); }
 };
 
-enum RoiProgram { kRoiRun, kRoiGroup, kRoiVoxel };
-
 // run / group: items = R.rows * groups, item (r, q) is the q-th group that meets the span of run r (groups = the most a span
 // meets); voxel: items = R.rows * R.len, one per selected voxel
 template <class Src, int kProgram>
@@ -197,6 +197,97 @@ int launch_gather(const Src& src, const RoiRuns& R, typename Src::T* dst, size_t
   return (int)cudaGetLastError();
 }
 
+// R.start(r) with its loop kept rolled: unrolled, the chain of 64-bit divisions makes the batch gather spill
+__device__ __forceinline__ uint64_t run_start(const RoiRuns& R, uint64_t r) {
+  uint64_t v = R.base;
+#pragma unroll 1
+  for (int k = R.nlead - 1; k >= 0; --k) {
+    v += (r % R.extent[k]) * R.stride[k];
+    r /= R.extent[k];
+  }
+  return v;
+}
+
+__host__ __device__ inline uint64_t roi_groups(const RoiRuns& R, int G) { return ((R.len - 1) * R.step + 1 + G - 1) / G + 1; }
+
+// The batch: one launch per thread program serves every selection of the call that takes it. sels[0 .. nsel) hold the prefix sums
+// of their items (`before`); a thread finds the selection of its item by a binary search over them and runs the program of
+// roi_gather_kernel for it, into dst + sels[s].first.
+template <class Src, int kProgram>
+__global__ void __launch_bounds__(kRoiThreads) roi_gather_batch_kernel(Src src, const RoiSel* __restrict__ sels, uint32_t nsel,
+                                                                       uint64_t items, typename Src::T* __restrict__ dst) {
+  using T = typename Src::T;
+  constexpr int G = Src::G;
+  constexpr int kPer = 4 / sizeof(T);
+  src.prologue();
+  for (uint64_t it = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; it < items; it += (uint64_t)gridDim.x * blockDim.x) {
+    uint32_t s = 0, hi = nsel;   // sels[s].before <= it < sels[hi].before (hi = nsel: items)
+    while (hi - s > 1) {
+      const uint32_t mid = (s + hi) / 2;
+      if (__ldg(&sels[mid].before) <= it) s = mid;
+      else hi = mid;
+    }
+    const RoiRuns& R = sels[s].runs;
+    const uint64_t local = it - __ldg(&sels[s].before);
+    T* const base = dst + __ldg(&sels[s].first);
+    if (kProgram == kRoiVoxel) {
+      const uint64_t r = local / R.len;
+      base[local] = src.voxel(run_start(R, r) + (local - r * R.len) * R.step);
+      continue;
+    }
+    const uint64_t groups = roi_groups(R, G);
+    const uint64_t r = local / groups, v0 = run_start(R, r), v1 = v0 + (kProgram == kRoiRun ? R.len : (R.len - 1) * R.step + 1);
+    const uint64_t g = v0 / G + (local - r * groups);
+    if (g * G >= v1) continue;
+    uint32_t L[Src::kWords];
+    src.load(g, L);
+    T* out = base + r * R.len;
+    if (kProgram == kRoiGroup) {
+      const uint64_t j0 = g * G > v0 ? (g * G - v0 + R.step - 1) / R.step : 0;
+      uint32_t next = (uint32_t)(v0 + j0 * R.step - g * G);
+      const uint32_t step = (uint32_t)R.step;
+      T* o = out + j0;
+#pragma unroll
+      for (int k = 0; k < G; ++k) {
+        if (k == next && g * G + k < v1) {
+          *o++ = (T)(L[k / kPer] >> (8 * sizeof(T) * (k % kPer)));
+          next += step;
+        }
+      }
+      continue;
+    }
+    // packed selections start anywhere: whole groups take 16-byte stores only where the destination is aligned
+    if (g * G >= v0 && (g + 1) * G <= v1 && (((uintptr_t)(out + (g * G - v0))) & 15) == 0) {
+      uint4* o = reinterpret_cast<uint4*>(out + (g * G - v0));
+#pragma unroll
+      for (uint32_t i = 0; i < Src::kWords / 4; ++i) o[i] = make_uint4(L[4 * i], L[4 * i + 1], L[4 * i + 2], L[4 * i + 3]);
+      continue;
+    }
+#pragma unroll
+    for (int k = 0; k < G; ++k) {
+      const uint64_t v = g * G + k;
+      if (v >= v0 && v < v1) out[v - v0] = (T)(L[k / kPer] >> (8 * sizeof(T) * (k % kPer)));
+    }
+  }
+}
+
+template <class Src, int kProgram>
+void launch_batch_program(const Src& src, const RoiSel* d_sels, const RoiBatch& B, typename Src::T* dst, size_t smem, cudaStream_t st) {
+  if (!B.count[kProgram]) return;
+  roi_gather_batch_kernel<Src, kProgram><<<grid_for(B.items[kProgram], kRoiThreads), kRoiThreads, smem, st>>>(
+      src, d_sels + B.begin[kProgram], B.count[kProgram], B.items[kProgram], dst);
+  SQYB_COUNT_LAUNCH(1);
+}
+
+// one launch per thread program that a selection takes
+template <class Src>
+int launch_batch(const Src& src, const RoiSel* d_sels, const RoiBatch& B, typename Src::T* dst, size_t smem, cudaStream_t st) {
+  launch_batch_program<Src, kRoiRun>(src, d_sels, B, dst, smem, st);
+  launch_batch_program<Src, kRoiGroup>(src, d_sels, B, dst, smem, st);
+  launch_batch_program<Src, kRoiVoxel>(src, d_sels, B, dst, smem, st);
+  return (int)cudaGetLastError();
+}
+
 }  // namespace
 
 int k_roi_gather_planes(int w, const uint8_t* compact, const uint32_t* pos, uint64_t nsel, const RoiRuns& R, uint16_t* dst,
@@ -223,6 +314,58 @@ int k_roi_crop(int elem, const void* vol, uint64_t n, const RoiRuns& R, void* ds
     return launch_gather(FromVolume<uint16_t>{static_cast<const uint16_t*>(vol), n}, R, static_cast<uint16_t*>(dst), 0, st);
   if (elem == 1)
     return launch_gather(FromVolume<uint8_t>{static_cast<const uint8_t*>(vol), n}, R, static_cast<uint8_t*>(dst), 0, st);
+  return -1;
+}
+
+RoiBatch roi_batch(RoiSource source, const RoiRuns* R, size_t n, RoiSel* sels) {
+  static_assert(FromPlanes<1>::G == FromVolume<uint16_t>::G && FromPlanes<1>::G == FromVolume<uint8_t>::G, "one group size");
+  const int G = source == kRoiCodes ? FromCodes::G : FromPlanes<1>::G;
+  const auto program = [&](const RoiRuns& r) {   // launch_gather's rule
+    return r.step >= (uint64_t)G / 2 ? kRoiVoxel : r.step == 1 ? kRoiRun : kRoiGroup;
+  };
+  RoiBatch B{};
+  for (size_t i = 0; i < n; ++i)
+    if (R[i].rows && R[i].len) B.count[program(R[i])]++;
+  B.begin[kRoiGroup] = B.count[kRoiRun];
+  B.begin[kRoiVoxel] = B.begin[kRoiGroup] + B.count[kRoiGroup];
+  uint32_t at[3] = {B.begin[0], B.begin[1], B.begin[2]};
+  uint64_t first = 0;
+  for (size_t i = 0; i < n; ++i) {
+    const uint64_t voxels = R[i].rows * R[i].len;
+    if (voxels) {
+      const int p = program(R[i]);
+      sels[at[p]++] = RoiSel{R[i], first, B.items[p]};
+      B.items[p] += R[i].rows * (p == kRoiVoxel ? R[i].len : roi_groups(R[i], G));
+    }
+    first += voxels;
+  }
+  return B;
+}
+
+int k_roi_gather_planes_batch(int w, const uint8_t* compact, const uint32_t* pos, uint64_t nsel, const RoiSel* d_sels, const RoiBatch& B,
+                              uint16_t* dst, cudaStream_t st) {
+  if ((((uintptr_t)compact) & 31) != 0) return -3;
+  switch (w) {
+    case 1: return launch_batch(FromPlanes<1>{compact, pos, nsel}, d_sels, B, dst, 0, st);
+    case 2: return launch_batch(FromPlanes<2>{compact, pos, nsel}, d_sels, B, dst, 0, st);
+    case 4: return launch_batch(FromPlanes<4>{compact, pos, nsel}, d_sels, B, dst, 0, st);
+    case 8: return launch_batch(FromPlanes<8>{compact, pos, nsel}, d_sels, B, dst, 0, st);
+  }
+  return -1;
+}
+
+int k_roi_gather_codes_batch(const uint8_t* compact, const uint32_t* pos, const uint16_t* lut_dev, const RoiSel* d_sels, const RoiBatch& B,
+                             uint16_t* dst, cudaStream_t st) {
+  if ((((uintptr_t)compact) & 15) != 0) return -3;
+  return launch_batch(FromCodes{compact, pos, lut_dev}, d_sels, B, dst, 256 * sizeof(uint16_t), st);
+}
+
+int k_roi_crop_batch(int elem, const void* vol, uint64_t n, const RoiSel* d_sels, const RoiBatch& B, void* dst, cudaStream_t st) {
+  if ((((uintptr_t)vol) & 15) != 0) return -3;
+  if (elem == 2)
+    return launch_batch(FromVolume<uint16_t>{static_cast<const uint16_t*>(vol), n}, d_sels, B, static_cast<uint16_t*>(dst), 0, st);
+  if (elem == 1)
+    return launch_batch(FromVolume<uint8_t>{static_cast<const uint8_t*>(vol), n}, d_sels, B, static_cast<uint8_t*>(dst), 0, st);
   return -1;
 }
 

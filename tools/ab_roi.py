@@ -1,9 +1,11 @@
-"""A/B of the box calls (sqyx_decode_roi_device_UI16, sqyx_decode_roi_UI16) between library builds on the same GPU in the same
-process (development tool): the one-plane and the 256^3 tile box of cfg2 (`rmestbkrd->bitswap1->lz4`) and cfg3 (`quantiser->lz4`)
-on a seeded synthetic 512x2048x2048 uint16 stack, each encoded once by the first build. The builds take turns inside every
-round: device calls timed with CUDA events, host calls (pageable buffers, nthreads = 8) with a wall clock, median over rounds.
-One torch.profiler pass per build and box gives the gather kernel's time. Round 0 checks that every build writes the same
-voxels and reports the same last_roi_info().
+"""A/B of the box and slice calls (sqyx_decode_roi_device_UI16 / sqyx_decode_roi_UI16, sqyx_decode_slice_*_UI16 for the strided
+cases) between library builds on the same GPU in the same process (development tool): the boxes and slices of bench_roi.py on
+cfg2 (`rmestbkrd->bitswap1->lz4`) and cfg3 (`quantiser->lz4`) on a seeded synthetic 512x2048x2048 uint16 stack, each encoded once
+by the first build. A build that has the batch calls is also timed with each selection as a batch of one
+(sqyx_decode_slice_batch_*_UI16, nsel = 1): the batch gather kernel against the single calls' by-value one. The variants take
+turns inside every round: device calls timed with CUDA events, host calls (pageable buffers, nthreads = 8) with a wall clock,
+median over rounds. One torch.profiler pass per variant and box gives the gather kernel's time. Round 0 checks that every
+variant writes the same voxels and reports the same last_roi_info().
 usage: ab_roi.py libA.so libB.so ...   (env AB_ROUNDS: rounds, default 7; AB_CALLS: calls per timing, default 5)"""
 import ctypes
 import os
@@ -18,6 +20,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 import sqeazy_b200 as sq  # noqa: E402
+from bench_roi import BOXES  # noqa: E402
 from sqeazy_b200.synth import torch_volume  # noqa: E402
 
 rounds = int(os.environ.get("AB_ROUNDS", "7"))
@@ -26,10 +29,6 @@ libs = [(p, ctypes.CDLL(os.path.abspath(p))) for p in sys.argv[1:]]
 SHAPE = (512, 2048, 2048)
 Z, Y, X = SHAPE
 CONFIGS = {"cfg2": "rmestbkrd->bitswap1->lz4", "cfg3": "quantiser->lz4"}
-BOXES = {
-    "one_plane": [(Z // 2, Z // 2 + 1), (0, Y), (0, X)],
-    "box_256": [(Z // 2 - 128, Z // 2 + 128), (Y // 2 - 128, Y // 2 + 128), (X // 2 - 128, X // 2 + 128)],
-}
 try:
     card = subprocess.run(["nvidia-smi", "--id=0", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True,
                           text=True, timeout=30).stdout.strip()
@@ -39,18 +38,35 @@ print(f"device: {card}", flush=True)
 
 
 def box_arr(box):
-    return (c_long * 6)(*[v for p in box for v in p])
+    """(the C array, whether it holds triples: the slice calls)"""
+    strided = any(len(t) == 3 for t in box)
+    vals = [v for t in box for v in ((t if len(t) == 3 else (*t, 1)) if strided else t)]
+    return (c_long * len(vals))(*vals), strided
 
 
-def roi_device(L, blob, box, out):
-    rc = L.sqyx_decode_roi_device_UI16(c_void_p(blob.data_ptr()), c_long(blob.numel()), box_arr(box), c_uint(3),
-                                       c_void_p(out.data_ptr()), c_long(2 * out.numel()), c_void_p(torch.cuda.current_stream().cuda_stream))
+def triples(box):
+    return (c_long * (3 * len(box)))(*[v for t in box for v in (t if len(t) == 3 else (*t, 1))])
+
+
+def roi_device(L, batch, blob, box, out):
+    args = (c_void_p(out.data_ptr()), c_long(2 * out.numel()), c_void_p(torch.cuda.current_stream().cuda_stream))
+    if batch:
+        rc = L.sqyx_decode_slice_batch_device_UI16(c_void_p(blob.data_ptr()), c_long(blob.numel()), triples(box), c_uint(1), c_uint(3), *args)
+    else:
+        arr, strided = box_arr(box)
+        fn = L.sqyx_decode_slice_device_UI16 if strided else L.sqyx_decode_roi_device_UI16
+        rc = fn(c_void_p(blob.data_ptr()), c_long(blob.numel()), arr, c_uint(3), *args)
     assert rc == 0, rc
 
 
-def roi_host(L, h_blob, box, h_out):
-    rc = L.sqyx_decode_roi_UI16(c_void_p(h_blob.ctypes.data), c_long(h_blob.size), box_arr(box), c_uint(3), c_void_p(h_out.ctypes.data),
-                                c_long(h_out.nbytes), c_int(8))
+def roi_host(L, batch, h_blob, box, h_out):
+    args = (c_void_p(h_out.ctypes.data), c_long(h_out.nbytes), c_int(8))
+    if batch:
+        rc = L.sqyx_decode_slice_batch_UI16(c_void_p(h_blob.ctypes.data), c_long(h_blob.size), triples(box), c_uint(1), c_uint(3), *args)
+    else:
+        arr, strided = box_arr(box)
+        fn = L.sqyx_decode_slice_UI16 if strided else L.sqyx_decode_roi_UI16
+        rc = fn(c_void_p(h_blob.ctypes.data), c_long(h_blob.size), arr, c_uint(3), *args)
     assert rc == 0, rc
 
 
@@ -84,12 +100,15 @@ def gather_ms(fn):
         for _ in range(calls):
             fn()
         torch.cuda.synchronize()
-    return sum(e.self_device_time_total for e in prof.key_averages() if "roi_gather_kernel" in e.key) / 1e3 / calls
+    return sum(e.self_device_time_total for e in prof.key_averages() if "roi_gather" in e.key) / 1e3 / calls
 
 
 torch.cuda.set_device(0)
 for _, L in libs:
     assert L.sqyx_set_device(c_int(0)) == 0
+# (label, library, as a batch of one)
+variants = [(os.path.basename(os.path.dirname(os.path.abspath(p))) + "/" + os.path.basename(p) + kind, L, batch) for p, L in libs
+            for kind, batch in (("", False), (" batch of 1", True)) if not batch or hasattr(L, "sqyx_decode_slice_batch_UI16")]
 sq.set_device(0)
 vol = torch_volume(SHAPE, "scmos", index=0)
 for cfg, pipeline in CONFIGS.items():
@@ -97,19 +116,19 @@ for cfg, pipeline in CONFIGS.items():
     blob = sq.encode_device(pipeline, vol).clone()
     h_blob = blob.cpu().numpy()
     for bname, box in BOXES.items():
-        n = int(np.prod([hi - lo for lo, hi in box]))
+        n = int(np.prod([len(range(*t)) for t in box]))
         out = torch.empty(n, dtype=torch.int16, device="cuda")
         h_out = np.empty(n, dtype=np.uint16)
-        ms = {name: {"device": [], "host": []} for name, _ in libs}
+        ms = {name: {"device": [], "host": []} for name, _, _ in variants}
         ref = None
         for rnd in range(rounds + 1):
-            for name, L in libs:
+            for name, L, batch in variants:
                 if rnd == 0:   # warm up and check
                     out.zero_()
-                    roi_device(L, blob, box, out)
+                    roi_device(L, batch, blob, box, out)
                     torch.cuda.synchronize()
                     got = (out.cpu().numpy().copy(), info(L))
-                    roi_host(L, h_blob, box, h_out)
+                    roi_host(L, batch, h_blob, box, h_out)
                     got_h = (h_out.copy(), info(L))
                     if ref is None:
                         ref = (got, got_h)
@@ -117,13 +136,13 @@ for cfg, pipeline in CONFIGS.items():
                         assert np.array_equal(got[0], ref[0][0]) and got[1] == ref[0][1], (cfg, bname, name, "device")
                         assert np.array_equal(got_h[0], ref[1][0]) and got_h[1] == ref[1][1], (cfg, bname, name, "host")
                     continue
-                ms[name]["device"].append(device_ms(lambda: roi_device(L, blob, box, out)))
-                ms[name]["host"].append(host_ms(lambda: roi_host(L, h_blob, box, h_out)))
-        for name, L in libs:
-            g = gather_ms(lambda: roi_device(L, blob, box, out))
-            print(f"{cfg} {bname:10s} {os.path.basename(os.path.dirname(os.path.abspath(name))) + '/' + os.path.basename(name):36s} "
+                ms[name]["device"].append(device_ms(lambda: roi_device(L, batch, blob, box, out)))
+                ms[name]["host"].append(host_ms(lambda: roi_host(L, batch, h_blob, box, h_out)))
+        for name, L, batch in variants:
+            g = gather_ms(lambda: roi_device(L, batch, blob, box, out))
+            print(f"{cfg} {bname:18s} {name:48s} "
                   + "  ".join(f"{k} {statistics.median(v):8.3f} ms [{min(v):.3f}..{max(v):.3f}]" for k, v in ms[name].items())
                   + f"  gather {g:.4f} ms", flush=True)
     del blob
     torch.cuda.empty_cache()
-print("identical voxels and last_roi_info() across builds", flush=True)
+print("identical voxels and last_roi_info() across variants", flush=True)

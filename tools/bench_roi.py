@@ -88,7 +88,7 @@ def kernel_breakdown(fn):
 
 
 def gather_ms(fn, reps=5):
-    """the gather kernel's device time per call"""
+    """the gather kernel's device time per call (roi_gather_kernel, or roi_gather_batch_kernel for the batch calls)"""
     from torch.profiler import ProfilerActivity, profile
     fn()
     torch.cuda.synchronize()
@@ -96,7 +96,7 @@ def gather_ms(fn, reps=5):
         for _ in range(reps):
             fn()
         torch.cuda.synchronize()
-    return sum(e.self_device_time_total for e in prof.key_averages() if "roi_gather_kernel" in e.key) / 1e3 / reps
+    return sum(e.self_device_time_total for e in prof.key_averages() if "roi_gather" in e.key) / 1e3 / reps
 
 
 def sel_of(box):

@@ -1072,31 +1072,33 @@ RoiPlan roi_plan(const StreamGeom& geo, const std::vector<Roi>& rois) {
   return P;
 }
 
-// The gather's tables on the device, in the arena's kSlotRoi: for a batch (the sqyx_decode_slice_batch_* calls) the descriptors of
-// its selections (kernels.h: roi_batch; `host` holds what that copy reads until the caller synchronises), then P's pos, then P's
-// list when the caller decodes by list, one copy each. P = nullptr: the descriptors alone. A single call takes no descriptor: its
-// runs go to roi_gather_kernel by value, which tools/ab_roi.py measured faster than a batch of one (profiles/README.md).
+// The gather's selections (kernels.h: RoiSelections) and its tables on the device, in the arena's kSlotRoi: for a batch (the
+// sqyx_decode_slice_batch_* calls) the descriptors of its selections (kernels.h: roi_batch; `host` holds what that copy reads until
+// the caller synchronises), then P's pos, then P's list when the caller decodes by list, one copy each. A single call takes no
+// descriptor: its runs go to roi_gather_kernel by value, which tools/ab_roi.py measured faster than a batch of one
+// (profiles/README.md). So a single crop (P = nullptr) copies nothing and takes no slot.
 struct RoiTables {
-  RoiBatch batch;
-  const RoiSel* d_sels;   // nullptr: a single call
+  RoiSelections sels;
   const uint32_t *d_pos, *d_list;
 };
 
 int roi_tables(Arena& A, RoiSource source, const std::vector<Roi>& rois, bool batch, const RoiPlan* P, bool with_list,
                std::vector<RoiSel>& host, RoiTables* T, cudaStream_t st) {
+  T->sels = RoiSelections{rois[0].runs, nullptr, {}};
   if (batch) {
     std::vector<RoiRuns> runs;
     runs.reserve(rois.size());
     for (const Roi& roi : rois) runs.push_back(roi.runs);
     host.resize(rois.size());
-    T->batch = roi_batch(source, runs.data(), runs.size(), host.data());
+    T->sels.batch = roi_batch(source, runs.data(), runs.size(), host.data());
   }
   const size_t sel_bytes = batch ? sizeof(RoiSel) * rois.size() : 0, pos_bytes = P ? 4 * P->pos.size() : 0;
   const size_t list_bytes = P && with_list ? 4 * P->list.size() : 0;
+  if (sel_bytes + pos_bytes + list_bytes == 0) return 0;
   void* p = nullptr;
   if (A.get(kSlotRoi, sel_bytes + pos_bytes + list_bytes, &p)) return 1;
   uint8_t* d = static_cast<uint8_t*>(p);
-  T->d_sels = batch ? reinterpret_cast<const RoiSel*>(d) : nullptr;
+  if (batch) T->sels.d_sels = reinterpret_cast<const RoiSel*>(d);
   T->d_pos = reinterpret_cast<const uint32_t*>(d + sel_bytes);
   T->d_list = reinterpret_cast<const uint32_t*>(d + sel_bytes + pos_bytes);
   if (sel_bytes) CK(cudaMemcpyAsync(d, host.data(), sel_bytes, cudaMemcpyHostToDevice, st));
@@ -1107,17 +1109,15 @@ int roi_tables(Arena& A, RoiSource source, const std::vector<Roi>& rois, bool ba
 
 // the gather behind the indexed route, from the compact blocks of P (`ws`: the block decode's workspace), then the block decode's
 // status: 11 (planes) / 101 (codes), what the whole-stack decode returns, when a block that a selection needs did not decode
-int roi_finish(Arena& A, const Pipeline& pl, int w, const RoiPlan& P, const std::vector<Roi>& rois, const RoiTables& T,
-               const uint8_t* compact, void* ws, uint16_t* d_dst, cudaStream_t st) {
+int roi_finish(Arena& A, const Pipeline& pl, int w, const RoiPlan& P, const RoiTables& T, const uint8_t* compact, void* ws,
+               uint16_t* d_dst, cudaStream_t st) {
   if (w) {
-    if (T.d_sels) CKK(k_roi_gather_planes_batch(w, compact, T.d_pos, P.nsel, T.d_sels, T.batch, d_dst, st));
-    else CKK(k_roi_gather_planes(w, compact, T.d_pos, P.nsel, rois[0].runs, d_dst, st));
+    CKK(k_roi_gather_planes(w, compact, T.d_pos, P.nsel, T.sels, d_dst, st));
   } else {
     SmallSlot small;
     if (small_slot(A, &small)) return 1;
     CK(cudaMemcpyAsync(small.dec_lut, pl.sink.decode_lut, 512, cudaMemcpyHostToDevice, st));
-    if (T.d_sels) CKK(k_roi_gather_codes_batch(compact, T.d_pos, small.dec_lut, T.d_sels, T.batch, d_dst, st));
-    else CKK(k_roi_gather_codes(compact, T.d_pos, small.dec_lut, rois[0].runs, d_dst, st));
+    CKK(k_roi_gather_codes(compact, T.d_pos, small.dec_lut, T.sels, d_dst, st));
   }
   uint32_t err = 0, none = 0;
   uint64_t total = 0;
@@ -1133,12 +1133,8 @@ int roi_finish(Arena& A, const Pipeline& pl, int w, const RoiPlan& P, const std:
 int roi_crop(Arena& A, const Pipeline& pl, const void* full, uint64_t N, const std::vector<Roi>& rois, bool batch,
              std::vector<RoiSel>& host, void* d_dst, cudaStream_t st) {
   RoiTables T{};
-  if (!batch) {
-    CKK(k_roi_crop(pl.elem, full, N, rois[0].runs, d_dst, st));
-    return 0;
-  }
-  if (roi_tables(A, kRoiVolume, rois, true, nullptr, false, host, &T, st)) return 1;
-  CKK(k_roi_crop_batch(pl.elem, full, N, T.d_sels, T.batch, d_dst, st));
+  if (roi_tables(A, kRoiVolume, rois, batch, nullptr, false, host, &T, st)) return 1;
+  CKK(k_roi_crop(pl.elem, full, N, T.sels, d_dst, st));
   return 0;
 }
 
@@ -1166,7 +1162,7 @@ int roi_device(Arena& A, const Header& hdr, const Pipeline& pl, const uint8_t* d
         return 1;
       info[0] = 1;
       CKK(k_lz4_decode_list(d_payload, payload_bytes, geo.bytes(), static_cast<uint8_t*>(compact), ws, T.d_list, (uint32_t)P.list.size(), st));
-      if (int rc = roi_finish(A, pl, w, P, rois, T, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_dst), st))
+      if (int rc = roi_finish(A, pl, w, P, T, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_dst), st))
         return rc;
       info[1] = (long)P.list.size();
       return 0;
@@ -1233,7 +1229,7 @@ int roi_host(Arena& A, const Header& hdr, const Pipeline& pl, const char* src, u
     const uint8_t* d_frame = static_cast<const uint8_t*>(d_sub);
     CKK(k_lz4_decode_tables(d_frame, sub_bytes, sub_raw, ws, 0, 0, st));
     CKK(k_lz4_decode_run(d_frame, sub_bytes, static_cast<uint8_t*>(compact), sub_raw, ws, 0, 0, 0, 0, 0, st));
-    if (int rc = roi_finish(A, pl, w, P, rois, T, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_box), st))
+    if (int rc = roi_finish(A, pl, w, P, T, static_cast<const uint8_t*>(compact), ws, static_cast<uint16_t*>(d_box), st))
       return rc;
     info[1] = (long)nlist;
     CK((cudaError_t)staged_d2h(dst, d_box, box_bytes, nthreads, st));

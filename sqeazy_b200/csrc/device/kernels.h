@@ -115,18 +115,9 @@ struct RoiRuns {
     return v;
   }
 };
-// from the compact 16 KiB blocks of the P = 16/w bit planes of a uint16 bitswap`w` that hold the box: block k of plane segment j
-// (the stream's set j) is compact block j * nsel + pos[k] (pos[k] = ~0: not there, never read)
-int k_roi_gather_planes(int w, const uint8_t* compact, const uint32_t* pos, uint64_t nsel, const RoiRuns& R, uint16_t* dst,
-                        cudaStream_t st);
-// from the compact 16 KiB blocks of 8-bit quantiser codes (block k is compact block pos[k]) through the 256-entry decode LUT
-int k_roi_gather_codes(const uint8_t* compact, const uint32_t* pos, const uint16_t* lut_dev, const RoiRuns& R, uint16_t* dst,
-                       cudaStream_t st);
-// from a whole decoded stack of n voxels of elem bytes (the crop)
-int k_roi_crop(int elem, const void* vol, uint64_t n, const RoiRuns& R, void* dst, cudaStream_t st);
-// The same gathers for a batch of selections, written densely one after the other, one launch per thread program that one of them
-// takes. RoiSel describes a non-empty selection in device memory: its runs, its first voxel in the packed destination, and the
-// work items of the selections in front of it in its program's launch.
+// The gathers write one selection, or a batch of them densely one after the other. Each takes one launch per thread program that
+// a selection takes (roi.cu). RoiSel describes a non-empty selection of a batch in device memory: its runs, its first voxel in the
+// packed destination, and the work items of the selections in front of it in its program's launch.
 enum RoiProgram { kRoiRun, kRoiGroup, kRoiVoxel };
 struct RoiSel {
   RoiRuns runs;
@@ -137,14 +128,25 @@ struct RoiBatch {
   uint32_t begin[3], count[3];
   uint64_t items[3];
 };
+// the selections of a gather: one selection's runs, passed to the kernel by value (d_sels = nullptr), or a batch's descriptors in
+// device memory and their launches (roi_batch)
+struct RoiSelections {
+  RoiRuns runs;
+  const RoiSel* d_sels;
+  RoiBatch batch;
+};
 enum RoiSource { kRoiPlanes, kRoiCodes, kRoiVolume };
 // host: the descriptors of selections R[0 .. n) in the order the launches take them, into sels (room for n; an empty selection
 // takes no descriptor and no room in the destination), for a gather from `source`
 RoiBatch roi_batch(RoiSource source, const RoiRuns* R, size_t n, RoiSel* sels);
-int k_roi_gather_planes_batch(int w, const uint8_t* compact, const uint32_t* pos, uint64_t nsel, const RoiSel* d_sels, const RoiBatch& B,
-                              uint16_t* dst, cudaStream_t st);
-int k_roi_gather_codes_batch(const uint8_t* compact, const uint32_t* pos, const uint16_t* lut_dev, const RoiSel* d_sels, const RoiBatch& B,
-                             uint16_t* dst, cudaStream_t st);
-int k_roi_crop_batch(int elem, const void* vol, uint64_t n, const RoiSel* d_sels, const RoiBatch& B, void* dst, cudaStream_t st);
+// from the compact 16 KiB blocks of the P = 16/w bit planes of a uint16 bitswap`w` that hold the selections: block k of plane
+// segment j (the stream's set j) is compact block j * nsel + pos[k] (pos[k] = ~0: not there, never read)
+int k_roi_gather_planes(int w, const uint8_t* compact, const uint32_t* pos, uint64_t nsel, const RoiSelections& S, uint16_t* dst,
+                        cudaStream_t st);
+// from the compact 16 KiB blocks of 8-bit quantiser codes (block k is compact block pos[k]) through the 256-entry decode LUT
+int k_roi_gather_codes(const uint8_t* compact, const uint32_t* pos, const uint16_t* lut_dev, const RoiSelections& S, uint16_t* dst,
+                       cudaStream_t st);
+// from a whole decoded stack of n voxels of elem bytes (the crop)
+int k_roi_crop(int elem, const void* vol, uint64_t n, const RoiSelections& S, void* dst, cudaStream_t st);
 
 }  // namespace sqyb
